@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the U-Net hot path (BASELINE.json metric: UNet train img/s @512^2 bf16).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 --config (default train512 = the headline, BASELINE.json configs[1]; the others give the remaining named shapes a line):
   train512       UNet(3,2) training step, 16 x 3x512x512 per GPU, dice_bce_mc + SGD; N > 1 = data parallel + SyncBN (weak)
@@ -18,6 +18,13 @@ ours      : `value`   images/s with the batch already resident in HBM, CUDA-even
 reference : the UNMODIFIED reference modules (oracle/_ref/Model.py + loss.py, staged by oracle/build_ref.py) running the
             same step on the host CPU with all host threads; each step is a bounded sample (fewer images) of the same
             workload. Falls back to the oracle port (kind "port") only if the staged copy is missing.
+
+--dump-outputs DIR (ours): after the timed steps, the arrays the last timed step handed its caller are written as
+DIR/<name>.npy (float32; float64 where the tensor is fp64 or integer): `loss`, `output` (the network output the loss saw),
+`grad.<parameter>` and `state.<state_dict key>` (after the optimizer step) for training, `mask` for inference. Inputs and
+initial weights are seeded, so two builds run with the same arguments can be compared array for array. An array of more
+than 2^18 elements is cut to a fixed seeded sample of 2^18 of them (the same elements for the same size), which keeps
+the whole dump within 64 MB.
 """
 from __future__ import annotations
 
@@ -76,6 +83,34 @@ def conv_traffic():
             return json.load(f)["dram_bytes_per_launch"]
     except Exception:
         return None
+
+
+DUMP_BYTES = 64_000_000   # --dump-outputs: the whole dump, .npy headers included
+DUMP_ELEMS = 1 << 18       # --dump-outputs: elements kept of any one array
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: tensor} as out_dir/<name>.npy. An array of more than DUMP_ELEMS elements is replaced by a fixed seeded
+    sample of DUMP_ELEMS of its flattened elements, in index order. The sample depends on nothing but the array's own size,
+    so the dumps of two builds line up element for element even where their sets of arrays differ.
+    Returns (bytes of data, sampled names)."""
+    import numpy as np
+
+    wide = {k: t.dtype in (torch.float64, torch.int64, torch.int32) for k, t in arrays.items()}  # exact in float64 only
+    nbytes = sum(min(t.numel(), DUMP_ELEMS) * (8 if wide[k] else 4) + 256 for k, t in arrays.items())
+    if nbytes > DUMP_BYTES:
+        raise RuntimeError(f"--dump-outputs: {len(arrays)} arrays need {nbytes} bytes, more than {DUMP_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    sampled = []
+    for k, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+            sampled.append(k)
+        a = t.to(torch.float64 if wide[k] else torch.float32).cpu().numpy()
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    return nbytes, sampled
 
 
 def batch_per_gpu(wl, n_gpus):
@@ -310,6 +345,7 @@ def run_ours(args):
         y_host = y_host.pin_memory()
         y_dev = y_host.to(dev)
 
+    # step() returns (what the timing reads back every step, the network output)
     if train:
         def step(x, y):
             out = net(x)
@@ -319,11 +355,12 @@ def run_ours(args):
             opt.zero_grad(set_to_none=True)
             loss.backward()
             opt.step()
-            return loss
+            return loss, out
     else:
         def step(x, y):
             with torch.no_grad():
-                return net.predict(x)  # OutConv + softmax + argmax + uint8 fused (test_mc3serousv5.py:878-887)
+                mask = net.predict(x)  # OutConv + softmax + argmax + uint8 fused (test_mc3serousv5.py:878-887)
+            return mask, mask
 
     def barrier():
         if dist_on:
@@ -407,7 +444,7 @@ def run_ours(args):
         if i + 1 < args.steps:
             fetch(i + 1)  # issued BEFORE this step's kernels, so it overlaps them; every step's inputs cross PCIe in the region
         cur.wait_event(ready[b])
-        res = step(xbuf[b], ybuf[b])
+        res, out = step(xbuf[b], ybuf[b])
         done[b].record(cur)
         res_host[b].copy_(res.detach(), non_blocking=True)  # device -> host read of the step's result, every step
         res_ready[b].record(cur)
@@ -420,6 +457,16 @@ def run_ours(args):
     barrier()
     ms_e2e = max_over_ranks(e0.elapsed_time(e1))
     e2e_value = B * world * args.steps / (ms_e2e / 1e3)
+    if args.dump_outputs and rank == 0:
+        if train:
+            arrays = {"loss": res, "output": out}
+            arrays.update({"grad." + k: p.grad for k, p in net.named_parameters() if p.grad is not None})
+            arrays.update({"state." + k: v for k, v in net.state_dict().items()})
+        else:
+            arrays = {"mask": res}
+        nbytes, sampled = dump_outputs(args.dump_outputs, arrays)
+        print(f"bench.py: {len(arrays)} arrays of the last timed step -> {args.dump_outputs} ({nbytes / 1e6:.1f} MB; "
+              f"{len(sampled)} sampled)", file=sys.stderr)
 
     # ---- roofline of the dominant kernel class (tcgen05 conv3x3 implicit GEMM), CUDA events around each launch
     net.enable_cuda_graphs(False)  # per-launch CUDA events need the eager launch path
@@ -522,7 +569,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--torch-optim", action="store_true", help="step with stock torch.optim.SGD instead of FusedSGD")
     ap.add_argument("--no-graphs", action="store_true", help="launch every kernel eagerly (no CUDA-graph replay)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     try:

@@ -249,3 +249,36 @@ def test_gate_checker_accepts_the_reference_and_flags_a_missing_term():
         assert check_gate(rec, tol_map=1e-9, tol_sum=1e-9, tol_grad=1e-9) == [], frozen
     rec["grads"]["W_q"] = rec["grads"]["W_q"] - torch.outer(rec["grads"]["b_q"], p["b_up"]).view(ch, cq, 1, 1)
     assert [b[0] for b in check_gate(rec, tol_map=1e-9, tol_sum=1e-9, tol_grad=1e-9)] == ["dW_q"]
+
+
+def test_bench_dump_outputs_samples_each_array_by_its_own_size_within_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: an array longer than the per-array cap is cut to a fixed seeded sample that depends only on
+    its own size (identical from run to run, and when other arrays come or go, so two builds compare element for
+    element); shorter arrays are written whole; fp64 / integer data stay exact; a dump over the byte budget is refused."""
+    import os
+
+    import numpy as np
+
+    import bench
+
+    monkeypatch.setattr(bench, "DUMP_ELEMS", 5000)
+    g = torch.Generator().manual_seed(0)
+    arrays = {"loss": torch.tensor(0.25), "output": torch.randn(4, 2, 64, 64, generator=g).bfloat16(),
+              "grad.w": torch.randn(64, 32, 3, 3, generator=g), "state.b": torch.randn(7, generator=g).double(),
+              "state.n": torch.tensor(12345678901, dtype=torch.int64)}
+    dumps = []
+    for run, names in (("a", list(arrays)), ("b", list(arrays)), ("c", ["grad.w"])):
+        nbytes, sampled = bench.dump_outputs(str(tmp_path / run), {k: arrays[k] for k in names})
+        files = sorted(os.listdir(tmp_path / run))
+        assert files == sorted(k + ".npy" for k in names) and sorted(sampled) == [k for k in ("grad.w", "output") if k in names]
+        assert sum(os.path.getsize(tmp_path / run / f) for f in files) <= nbytes <= bench.DUMP_BYTES
+        dumps.append({k: np.load(tmp_path / run / (k + ".npy")) for k in names})
+    a, b, c = dumps
+    assert all(np.array_equal(a[k], b[k]) for k in arrays) and np.array_equal(a["grad.w"], c["grad.w"])
+    assert a["output"].dtype == np.float32 and a["state.b"].dtype == np.float64 and int(a["state.n"]) == 12345678901
+    assert np.array_equal(a["state.b"], arrays["state.b"].numpy()) and float(a["loss"]) == 0.25
+    w = arrays["grad.w"].flatten().numpy()
+    assert a["grad.w"].size == a["output"].size == 5000 and np.isin(a["grad.w"], w).all()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 30_000)
+    with pytest.raises(RuntimeError, match="dump-outputs"):
+        bench.dump_outputs(str(tmp_path / "d"), arrays)

@@ -1,11 +1,12 @@
 """CPU: the oracle (oracle/unet_oracle.py) against the golden vectors produced by the UNMODIFIED reference
-(oracle/make_golden.py), and - when /root/reference is mounted - against the live reference."""
+(oracle/make_golden.py), and - when the reference modules are staged (oracle/build_ref.py) - against the live reference."""
 import os
 import sys
 
 import pytest
 import torch
 
+from oracle import ref_loader
 from oracle import unet_oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -84,14 +85,9 @@ def test_mse_losses(golden):
     assert abs(float(l) - float(g["loss"])) < 1e-6 and rel(gr, g["grad"]) < 1e-6
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/Model.py"), reason="reference not mounted")
+@pytest.mark.skipif(not ref_loader.available(), reason="reference modules not staged (python oracle/build_ref.py)")
 def test_live_reference_agrees():
-    sys.dont_write_bytecode = True
-    import importlib.util
-
-    spec = importlib.util.spec_from_file_location("_ref_model", "/root/reference/Model.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    ref, _ = ref_loader.load()
     torch.manual_seed(3)
     net = ref.UNet(2, 3, 4).double()
     x = torch.randn(2, 2, 32, 32, dtype=torch.float64)
@@ -108,19 +104,14 @@ def test_live_reference_agrees():
     assert rel(got, want) < 1e-10
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/Model.py"), reason="reference not mounted")
+@pytest.mark.skipif(not ref_loader.available(), reason="reference modules not staged (python oracle/build_ref.py)")
 @pytest.mark.parametrize("h,w,dropout", [(37, 45, False), (32, 32, True), (50, 35, True)])
 def test_live_reference_odd_sizes_and_dropout(h, w, dropout):
     """Pins the oracle's floor-mode pooling, the F.pad branch (Model.py:69-73) and the dropout placement
     (Model.py:34-39, 81-82) to the unmodified reference: same seed -> same masks (CPU generator, same draw order)."""
-    sys.dont_write_bytecode = True
-    import importlib.util
-
     import torch.nn.functional as F
 
-    spec = importlib.util.spec_from_file_location("_ref_model2", "/root/reference/Model.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
+    ref, _ = ref_loader.load()
     torch.manual_seed(4)
     net = ref.UNet(3, 2, 4, dropout=dropout, dropout_p=0.3).double()
     x = torch.randn(2, 3, h, w, dtype=torch.float64)
@@ -241,22 +232,16 @@ def test_bf16_storage_emulation_reproduces_the_references_own_bf16_error(golden)
 
 
 def test_staged_reference_copy_is_the_reference_byte_for_byte():
-    """oracle/_ref (git-ignored, travels to the GPU box) must be the unmodified reference files: the manifest hashes match the
-    staged files, and - where /root/reference is mounted - the mounted files too."""
+    """oracle/_ref (git-ignored) must be the unmodified reference files: the staged files still have the hashes that
+    oracle/build_ref.py recorded (and checked against the source) when it copied them."""
     import hashlib
     import json
 
-    from oracle import ref_loader
-
     d = os.path.join(ROOT, "oracle", "_ref")
     if not os.path.exists(os.path.join(d, "MANIFEST.json")):
-        pytest.skip("oracle/_ref not staged (run python oracle/build_ref.py where /root/reference exists)")
-    man = json.load(open(os.path.join(d, "MANIFEST.json")))["files"]
-    for name, digest in man.items():
+        pytest.skip("oracle/_ref not staged (python oracle/build_ref.py)")
+    for name, digest in json.load(open(os.path.join(d, "MANIFEST.json")))["files"].items():
         assert hashlib.sha256(open(os.path.join(d, name), "rb").read()).hexdigest() == digest, name
-        src = os.path.join("/root/reference", name)
-        if os.path.exists(src):
-            assert hashlib.sha256(open(src, "rb").read()).hexdigest() == digest, name
     RefModel, ref_loss = ref_loader.load()
     assert RefModel.UNet(1, 2, 4).state_dict().keys() and callable(ref_loss.calc_loss)
 
