@@ -32,7 +32,7 @@ CONV_SHAPES = [
     (2, 40, 72, 64, 128),     # BN = 128, ragged rows
     (3, 64, 64, 128, 64),     # two K blocks per tile
     (2, 48, 64, 128, 256),    # four channel slices share each pixel tile
-    # deep-layer shapes (streaming kernels; CTA pairs with B200UNET_PAIR=1): odd tile count, BN = 256 and 128
+    # deep-layer shapes (streaming CTA-pair kernel; B200UNET_PAIR=0 selects igemm): odd tile count, BN = 256 and 128
     (3, 16, 24, 256, 256),
     (1, 32, 40, 512, 128),
     (2, 16, 16, 256, 512),
@@ -121,7 +121,7 @@ def test_conv3x3_eval_bn_relu_folded_epilogue(ops, n, h, w, cin, cout, choice):
 
 
 @pytest.mark.parametrize("cin,cout,hw", [(64, 64, 512), (128, 64, 512), (128, 128, 256), (256, 256, 128), (512, 512, 64),
-                                         (1024, 512, 64), (1024, 1024, 32), (256, 128, 256)])
+                                         (1024, 512, 64), (1024, 1024, 32), (256, 128, 256), (64, 128, 256)])
 def test_full_size_layers_all_kernel_choices_agree(ops, cin, cout, hw):
     """BASELINE config-2 layer shapes (batch 16): the oracle is too slow here, so the property is that every kernel
     able to run the layer (one-tile-per-CTA igemm, resident, resident pairs, streaming pairs) produces the same

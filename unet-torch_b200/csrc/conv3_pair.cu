@@ -1,15 +1,29 @@
-// CTA-pair (tcgen05 cta_group::2) STREAMING 3x3 implicit GEMM for the deep levels (Cin >= 256; nn.Conv2d fprop and
-// dgrad, reference Model.py:15-16,19-20: down2.conv2 ... up3.conv1), where a channel slice of the weights no longer
-// fits in shared memory. Same skeleton as conv3_res2.cu (persistent pairs, M = 256 = two adjacent 16x8 pixel tiles, one
-// 18x10 halo tile per 64-channel block with the 9 taps as descriptor offsets, double-buffered TMEM, epilogue with
-// BatchNorm statistics), but the weights stream through a second TMA ring at tap granularity: per K block and CTA
-// 23 KB of activations + 9 x (BN/2 rows x 128 B) of weights. With BN = 256 that is 170 KB of L2->SM traffic per
-// 36 MMAs of 128 cycles (37 B/clk/SM; igemm.cu: 90 B/clk) and 64 B/clk of shared-memory operand reads (igemm.cu: 128).
+// CTA-pair (tcgen05 cta_group::2) persistent 3x3 implicit GEMMs (nn.Conv2d fprop and dgrad, reference
+// Model.py:15-16,19-20). Two kernels on one skeleton that differ only in how the weights reach shared memory:
+//  * conv3_res2_kernel<BN, KB, NA, OB>: weights RESIDENT, for the layers of conv3_res.cu's resident-weight kernel
+//    (Cin = 64 / 128). All 9 x KB weight tiles of the CTA's BN/2 rows are loaded once, behind one barrier.
+//  * conv3_pair_kernel<BN, NA, NB, OB>: weights STREAMED, for the deep levels (Cin >= 256: down2.conv2 ... up3.conv1),
+//    where a channel slice of the weights no longer fits in shared memory. They pass through a second TMA ring at tap
+//    granularity: per K block and CTA 23 KB of activations + 9 x (BN/2 rows x 128 B) of weights. With BN = 256 that is
+//    170 KB of L2->SM traffic per 36 MMAs of 128 cycles (37 B/clk/SM; igemm.cu: 90 B/clk) and 64 B/clk of
+//    shared-memory operand reads (igemm.cu: 128).
+//
+// Why pairs: with one CTA per MMA an N = 64 tile reads 6 KB of shared-memory operands per 32-cycle MMA (192 B/clk, over
+// the 128 B/clk an SM can deliver) and Cin = 128 layers cannot keep more than a 64-column weight slice resident. A pair
+// issues ONE M = 256 MMA for two adjacent 16x8 pixel tiles: each CTA supplies its own 128 activation rows and only HALF
+// of the weight rows (BN/2), so the resident slice per CTA halves (N = 128 fits for Cin = 128) and shared-memory reads
+// per MMA cycle drop to 96-160 B/clk. The MMA instruction count per FLOP halves as well.
+//
+// Persistent pairs walk a static tile-pair schedule; per 64-channel block one 18x10 halo tile is loaded and the 9 taps
+// are descriptor offsets into it; two TMEM accumulator buffers. Roles per CTA (192 threads): warp 0 TMA producer (its
+// own activation halo tiles, its half of the weights; completion bytes are credited to the LEADER's barriers), warp 1
+// MMA issuer (leader CTA only), warps 2-5 epilogue (each CTA drains its own 128 TMEM lanes: bf16 -> swizzled staging ->
+// TMA store, BatchNorm statistics in registers).
+// Barriers: B_full (weights) / A_full[NA] / T_empty[2] live in the leader (remote TMA complete_tx / remote arrives);
+// B_empty (streamed weights) / A_empty[NA] / T_full[2] exist in both CTAs and are signalled by multicast tcgen05.commit.
 #include "../../include/b200unet.h"
 #include "host_common.h"
 #include "tc_common.cuh"
-
-#include <stdlib.h>
 
 namespace {
 
@@ -28,31 +42,49 @@ struct PairArgs {
   int ncols;     // Cout
   int ntiles_n;  // Cout / BN
   int workers;   // CTA pairs per channel slice (grid = 2 * workers * ntiles_n)
-  int kblocks;   // Cin / 64
-  int ktap;      // Cin (K extent of one tap in the weight operand)
+  int kblocks;   // Cin / 64 (streamed weights; the resident kernel has it as a template parameter)
+  int ktap;      // Cin (K extent of one tap in the weight operand; streamed weights)
   float* stats;  // [2 * workers][2][ncols] or null
   const float* scale;  // eval-mode BatchNorm + ReLU folded into the epilogue: [ncols] each, or null
   const float* shift;
 };
 
-template <int BN, int NA, int NB, int OB>
-struct PairPlan {
-  static constexpr int BH = BN / 2;          // weight rows this CTA supplies
-  static constexpr int B_STAGE = BH * 128;   // one tap, one 64-channel block
+// Shared-memory plans: byte offsets from the 1024-aligned base, barriers in 8-byte slots from BAR_OFF. A_full[NA] and
+// A_empty[NA] start at slot A_BAR, T_full[2], T_empty[2] and the TMEM address at slot T_BAR, the weight barriers at B_BAR.
+template <int BN_, int KB_, int NA_, int OB_>
+struct Res2Plan {  // resident: 9 x KB weight tiles at B_OFF, one barrier B_full(0)
+  static constexpr bool RESIDENT = true;
+  static constexpr int BN = BN_, KB = KB_, NA = NA_, NB = 0, OB = OB_;
+  static constexpr int B_STAGE = (BN / 2) * 128;  // one weight tile: BN/2 rows x 64 channels
+  static constexpr int B_BYTES = 9 * KB * B_STAGE;
+  static constexpr int B_OFF = 0;
+  static constexpr int A_OFF = B_BYTES;
+  static constexpr int OUT_OFF = A_OFF + NA * A_STAGE;
+  static constexpr int BAR_OFF = OUT_OFF + OB * (BN / 64) * OUT_CHUNK;
+  static constexpr int TOTAL = BAR_OFF + 256 + 1024;
+  static constexpr int B_BAR = 0, A_BAR = 1, T_BAR = 1 + 2 * NA;
+  static_assert(B_BYTES % 1024 == 0, "weight tiles must stay 1024-byte aligned");
+};
+
+template <int BN_, int NA_, int NB_, int OB_>
+struct PairPlan {  // streamed: an NB-stage ring of (one tap, one 64-channel block) weight tiles, B_full[NB] / B_empty[NB]
+  static constexpr bool RESIDENT = false;
+  static constexpr int BN = BN_, KB = 0, NA = NA_, NB = NB_, OB = OB_;
+  static constexpr int B_STAGE = (BN / 2) * 128;  // one weight tile: BN/2 rows x 64 channels
   static constexpr int A_OFF = 0;
   static constexpr int B_OFF = NA * A_STAGE;
   static constexpr int OUT_OFF = B_OFF + NB * B_STAGE;
-  static constexpr int OUT_BYTES = OB * (BN / 64) * OUT_CHUNK;
-  static constexpr int BAR_OFF = OUT_OFF + OUT_BYTES;
+  static constexpr int BAR_OFF = OUT_OFF + OB * (BN / 64) * OUT_CHUNK;
   static constexpr int TOTAL = BAR_OFF + 512 + 1024;
-  static_assert(TOTAL <= 227 * 1024, "shared memory plan exceeds 227 KiB");
-  static_assert(4 * 2 * BN * 4 <= OUT_BYTES, "final statistics reduction aliases the staging buffer");
+  static constexpr int A_BAR = 0, B_BAR = 2 * NA, T_BAR = 2 * NA + 2 * NB;
 };
 
-template <int BN, int NA, int NB, int OB>
-__global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constant__ PairArgs args) {
-  using P = PairPlan<BN, NA, NB, OB>;
-  constexpr int BH = P::BH, B_STAGE = P::B_STAGE;
+template <class P>
+__device__ __forceinline__ void conv3_pair_body(const PairArgs& args) {
+  constexpr int BN = P::BN, NA = P::NA, NB = P::NB, OB = P::OB;
+  constexpr int BH = BN / 2;  // weight rows this CTA supplies
+  static_assert(P::TOTAL <= 227 * 1024, "shared memory plan exceeds 227 KiB");
+  static_assert(4 * 2 * BN * 4 <= OB * (BN / 64) * OUT_CHUNK, "final statistics reduction aliases the staging buffer");
   extern __shared__ uint8_t smem_raw[];
   // both CTAs must use IDENTICAL smem offsets (operand descriptors and barrier offsets are shared by the pair)
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -61,16 +93,15 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
   const uint32_t sB = smem_base + P::B_OFF;
   const uint32_t sO = smem_base + P::OUT_OFF;
   const uint32_t bars = smem_base + P::BAR_OFF;
-  auto A_full = [&](int i) { return bars + 8u * i; };
-  auto A_empty = [&](int i) { return bars + 8u * (NA + i); };
-  auto B_full = [&](int i) { return bars + 8u * (2 * NA + i); };
-  auto B_empty = [&](int i) { return bars + 8u * (2 * NA + NB + i); };
-  auto T_full = [&](int i) { return bars + 8u * (2 * NA + 2 * NB + i); };
-  auto T_empty = [&](int i) { return bars + 8u * (2 * NA + 2 * NB + 2 + i); };
-  const uint32_t tmem_slot = bars + 8u * (2 * NA + 2 * NB + 4);
-  volatile uint32_t* tmem_slot_gen =
-      reinterpret_cast<volatile uint32_t*>(smem_gen + P::BAR_OFF + 8 * (2 * NA + 2 * NB + 4));
-  const int KB = args.kblocks;
+  auto A_full = [&](int i) { return bars + 8u * (P::A_BAR + i); };
+  auto A_empty = [&](int i) { return bars + 8u * (P::A_BAR + NA + i); };
+  auto B_full = [&](int i) { return bars + 8u * (P::B_BAR + i); };
+  auto B_empty = [&](int i) { return bars + 8u * (P::B_BAR + NB + i); };
+  auto T_full = [&](int i) { return bars + 8u * (P::T_BAR + i); };
+  auto T_empty = [&](int i) { return bars + 8u * (P::T_BAR + 2 + i); };
+  const uint32_t tmem_slot = bars + 8u * (P::T_BAR + 4);
+  volatile uint32_t* tmem_slot_gen = reinterpret_cast<volatile uint32_t*>(smem_gen + P::BAR_OFF + 8 * (P::T_BAR + 4));
+  const int KB = P::RESIDENT ? P::KB : args.kblocks;
 
   const int warp = warp_idx_uniform();
   const int lane = threadIdx.x & 31;
@@ -86,13 +117,16 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
     prefetch_tmap(&args.tmA);
     prefetch_tmap(&args.tmW);
     prefetch_tmap(&args.tmO);
+    if constexpr (P::RESIDENT) mbar_init(B_full(0), 1);
     for (int i = 0; i < NA; ++i) {
       mbar_init(A_full(i), 1);   // the leader's arrive.expect_tx; bytes arrive from both CTAs
       mbar_init(A_empty(i), 1);  // multicast commit
     }
-    for (int i = 0; i < NB; ++i) {
-      mbar_init(B_full(i), 1);
-      mbar_init(B_empty(i), 1);
+    if constexpr (!P::RESIDENT) {
+      for (int i = 0; i < NB; ++i) {
+        mbar_init(B_full(i), 1);
+        mbar_init(B_empty(i), 1);
+      }
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(T_full(i), 1);   // multicast commit
@@ -119,6 +153,16 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
   if (warp == 0) {
     // ================================================================= TMA producer (both CTAs)
     if (elect_one_sync()) {
+      if constexpr (P::RESIDENT) {
+        const uint32_t B_full_l = mapa_cluster(B_full(0), 0);
+        if (crank == 0) mbar_arrive_expect_tx(B_full(0), 2 * P::B_BYTES);
+#pragma unroll 1
+        for (int tap = 0; tap < 9; ++tap)
+#pragma unroll
+          for (int cb = 0; cb < KB; ++cb)
+            tma_load_2d_2cta(sB + (tap * KB + cb) * P::B_STAGE, &args.tmW, B_full_l, (tap * KB + cb) * 64,
+                             n0 + static_cast<int>(crank) * BH);
+      }
       int sa = 0, pa = 0, sb = 0, pb = 0;
 #pragma unroll 1
       for (int j = 0; j < npairs_mine; ++j) {
@@ -130,13 +174,15 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
           if (crank == 0) mbar_arrive_expect_tx(A_full(sa), 2 * A_BOX_BYTES);
           tma_load_4d_2cta(sA + sa * A_STAGE, &args.tmA, mapa_cluster(A_full(sa), 0), cb * 64, w0 - 1, h0 - 1, img);
           if (++sa == NA) { sa = 0; pa ^= 1; }
+          if constexpr (!P::RESIDENT) {
 #pragma unroll 1
-          for (int tap = 0; tap < 9; ++tap) {
-            mbar_wait(B_empty(sb), pb ^ 1);
-            if (crank == 0) mbar_arrive_expect_tx(B_full(sb), 2 * B_STAGE);
-            tma_load_2d_2cta(sB + sb * B_STAGE, &args.tmW, mapa_cluster(B_full(sb), 0), tap * args.ktap + cb * 64,
-                             n0 + static_cast<int>(crank) * BH);
-            if (++sb == NB) { sb = 0; pb ^= 1; }
+            for (int tap = 0; tap < 9; ++tap) {
+              mbar_wait(B_empty(sb), pb ^ 1);
+              if (crank == 0) mbar_arrive_expect_tx(B_full(sb), 2 * P::B_STAGE);
+              tma_load_2d_2cta(sB + sb * P::B_STAGE, &args.tmW, mapa_cluster(B_full(sb), 0), tap * args.ktap + cb * 64,
+                               n0 + static_cast<int>(crank) * BH);
+              if (++sb == NB) { sb = 0; pb ^= 1; }
+            }
           }
         }
       }
@@ -147,6 +193,11 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
     if (crank == 0 && elect_one_sync()) {
       constexpr uint32_t idesc = umma_idesc_bf16(256, BN, 0, 0);
       constexpr uint32_t a_hi = umma_desc_hi_sw128(IN_W * 128), b_hi = umma_desc_hi_sw128(1024);
+      const uint32_t w_lo = umma_desc_lo(sB, 16);  // resident weights: tile (tap, cb) at w_lo + (tap * KB + cb) * (BH * 8)
+      if constexpr (P::RESIDENT) {
+        mbar_wait(B_full(0), 0);
+        tc_fence_after();
+      }
       int sa = 0, pa = 0, sb = 0, pb = 0;
 #pragma unroll 1
       for (int j = 0; j < npairs_mine; ++j) {
@@ -155,26 +206,30 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + buf * BN;
         uint32_t acc = 0;
-#pragma unroll 1
+#pragma unroll(P::RESIDENT && P::KB <= 2 ? P::KB : 1)
         for (int cb = 0; cb < KB; ++cb) {
           mbar_wait(A_full(sa), pa);
           tc_fence_after();
           const uint32_t a_lo = umma_desc_lo(sA + sa * A_STAGE, 16);
 #pragma unroll
           for (int tap = 0; tap < 9; ++tap) {
-            mbar_wait(B_full(sb), pb);
-            tc_fence_after();
+            if constexpr (!P::RESIDENT) {
+              mbar_wait(B_full(sb), pb);
+              tc_fence_after();
+            }
             const uint32_t a_tap = a_lo + ((tap / 3) * IN_W + (tap % 3)) * 8;
-            const uint32_t b_lo = umma_desc_lo(sB + sb * B_STAGE, 16);
+            const uint32_t b_tap = P::RESIDENT ? w_lo + (tap * KB + cb) * (BH * 8) : umma_desc_lo(sB + sb * P::B_STAGE, 16);
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-              umma_bf16_lh_2cta(d_tmem, a_tap + 2 * k, a_hi, b_lo + 2 * k, b_hi, idesc, acc);
+              umma_bf16_lh_2cta(d_tmem, a_tap + 2 * k, a_hi, b_tap + 2 * k, b_hi, idesc, acc);
               acc = 1;
             }
-            umma_commit_2cta(B_empty(sb));  // frees the weight stage in BOTH CTAs
-            if (++sb == NB) { sb = 0; pb ^= 1; }
+            if constexpr (!P::RESIDENT) {
+              umma_commit_2cta(B_empty(sb));  // frees the weight stage in BOTH CTAs
+              if (++sb == NB) { sb = 0; pb ^= 1; }
+            }
           }
-          umma_commit_2cta(A_empty(sa));
+          umma_commit_2cta(A_empty(sa));  // frees the activation stage in BOTH CTAs
           if (++sa == NA) { sa = 0; pa ^= 1; }
         }
         umma_commit_2cta(T_full(buf));  // accumulator ready: both CTAs' epilogues
@@ -287,15 +342,27 @@ __global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constan
   if (warp == 1) tmem_dealloc_2cta(tmem_base, 2 * BN);
 }
 
+template <int BN, int KB, int NA, int OB>
+__global__ void __launch_bounds__(192, 1) conv3_res2_kernel(const __grid_constant__ PairArgs args) {
+  conv3_pair_body<Res2Plan<BN, KB, NA, OB>>(args);
+}
+
 template <int BN, int NA, int NB, int OB>
-int launch_pair(const PairArgs& a, cudaStream_t st) {
-  using P = PairPlan<BN, NA, NB, OB>;
+__global__ void __launch_bounds__(192, 1) conv3_pair_kernel(const __grid_constant__ PairArgs args) {
+  conv3_pair_body<PairPlan<BN, NA, NB, OB>>(args);
+}
+
+using PairKernel = void (*)(PairArgs);
+
+// kern must be the kernel instantiation of plan P (P::TOTAL bytes of dynamic shared memory)
+template <class P>
+int launch_pair(PairKernel kern, const PairArgs& a, cudaStream_t st) {
+  const char* name = P::RESIDENT ? "conv3_res2" : "conv3_pair";
   static unsigned long long configured = 0;  // one bit per CUDA device
-  auto kern = conv3_pair_kernel<BN, NA, NB, OB>;
   if (b2h::first_use_on_device(configured)) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
     if (e != cudaSuccess) {
-      b2h::set_error("conv3_pair: cudaFuncSetAttribute(smem=%d): %s", P::TOTAL, cudaGetErrorString(e));
+      b2h::set_error("%s: cudaFuncSetAttribute(smem=%d): %s", name, P::TOTAL, cudaGetErrorString(e));
       return 2;
     }
   }
@@ -313,19 +380,18 @@ int launch_pair(const PairArgs& a, cudaStream_t st) {
   cfg.numAttrs = 1;
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a);
   if (e != cudaSuccess) {
-    b2h::set_error("conv3_pair launch: %s", cudaGetErrorString(e));
+    b2h::set_error("%s launch: %s", name, cudaGetErrorString(e));
     return 2;
   }
-  return b2h::check_launch("conv3_pair");
+  return b2h::check_launch(name);
 }
 
 // Number of CTA pairs that can be resident at once (one CTA per SM, both CTAs of a pair in one TPC): the persistent
-// schedule is static, so the grid must not exceed it. Queried once with the largest shared-memory variant.
-int max_pairs() {
+// schedule is static, so the grid must not exceed it. Queried once per kernel, with its largest shared-memory variant.
+template <class P>
+int max_pairs(PairKernel kern) {
   static int n = 0;
   if (n == 0) {
-    auto kern = conv3_pair_kernel<256, 2, 6, 1>;
-    using P = PairPlan<256, 2, 6, 1>;
     int got = 0;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * 74);
@@ -344,61 +410,91 @@ int max_pairs() {
     else
       n = 64;  // conservative
     cudaGetLastError();
-    const char* e = getenv("B200UNET_RESERVE_SMS");  // see conv3_res.cu num_sms()
-    const int r = e ? atoi(e) : 0;
-    if (r > 0 && r / 2 < n / 2) n -= (r + 1) / 2;
   }
   return n;
 }
+
+int res2_max_pairs() { return max_pairs<Res2Plan<128, 2, 2, 1>>(conv3_res2_kernel<128, 2, 2, 1>); }
+int pair_max_pairs() { return max_pairs<PairPlan<256, 2, 6, 1>>(conv3_pair_kernel<256, 2, 6, 1>); }
 
 }  // namespace
 
 namespace b2h {
 
-bool conv3_pair_applicable(int Cin, int Cout) { return Cin >= 256 && Cin % 64 == 0 && Cout % 128 == 0; }
-
+static int res2_bn(int Cout) { return (Cout % 128 == 0) ? 128 : 64; }
 static int pair_bn(int Cout) { return (Cout % 256 == 0) ? 256 : 128; }
 
-static void pair_geometry(int N, int H, int W, int Cout, int* bn, int* ntn, int* workers, int* tiles) {
-  *bn = pair_bn(Cout);
-  *ntn = Cout / *bn;
+// max_pairs: CTA pairs resident at once for the kernel that will run
+static void pair_geometry(int N, int H, int W, int Cout, int bn, int max_pairs, int* ntn, int* workers, int* tiles) {
+  *ntn = Cout / bn;
   *tiles = N * ceil_div(H, RTH) * ceil_div(W, RTW);
   const int pairs = (*tiles + 1) / 2;
-  int w = max_pairs() / *ntn;
+  int w = max_pairs / *ntn;
   if (w < 1) w = 1;
   if (w > pairs) w = pairs;
   *workers = w;
 }
 
+static int pair_stat_rows(int N, int H, int W, int Cout, int bn, int max_pairs) {
+  int ntn, workers, tiles;
+  pair_geometry(N, H, W, Cout, bn, max_pairs, &ntn, &workers, &tiles);
+  return 2 * workers;
+}
+
+// Arguments of either kernel; tensor-map encoding failures return their error code.
+static int pair_args(PairArgs* a, const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N,
+                     int H, int W, int Cin, int Cout, int bn, int max_pairs, const float* scale, const float* shift) {
+  pair_geometry(N, H, W, Cout, bn, max_pairs, &a->ntiles_n, &a->workers, &a->tiles_total);
+  a->tiles_w = ceil_div(W, RTW);
+  a->tiles_h = ceil_div(H, RTH);
+  a->H = H;
+  a->W = W;
+  a->ncols = Cout;
+  a->kblocks = Cin / 64;
+  a->ktap = Cin;
+  a->stats = stats_partial;
+  a->scale = scale;
+  a->shift = shift;
+  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
+  if (int e = make_tmap_4d(&a->tmA, x, Cin, W, H, N, xs, xs * W, xs * W * H, IN_W, IN_H)) return e;
+  if (int e = make_tmap_2d(&a->tmW, w, static_cast<uint64_t>(9) * Cin, Cout, bn / 2)) return e;
+  return make_tmap_4d(&a->tmO, y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH);
+}
+
+int conv3_res2_stat_rows(int N, int H, int W, int Cin, int Cout) {
+  (void)Cin;
+  return pair_stat_rows(N, H, W, Cout, res2_bn(Cout), res2_max_pairs());
+}
+
+int conv3_res2_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,
+                      int W, int Cin, int Cout, cudaStream_t st, const float* scale,
+                     const float* shift) {
+  const int bn = res2_bn(Cout);
+  PairArgs a;
+  if (int e = pair_args(&a, x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, bn, res2_max_pairs(), scale, shift))
+    return e;
+  if (Cin == 64 && bn == 64) return launch_pair<Res2Plan<64, 1, 4, 2>>(conv3_res2_kernel<64, 1, 4, 2>, a, st);
+  if (Cin == 64 && bn == 128) return launch_pair<Res2Plan<128, 1, 3, 2>>(conv3_res2_kernel<128, 1, 3, 2>, a, st);
+  if (Cin == 128 && bn == 64) return launch_pair<Res2Plan<64, 2, 4, 2>>(conv3_res2_kernel<64, 2, 4, 2>, a, st);
+  return launch_pair<Res2Plan<128, 2, 2, 1>>(conv3_res2_kernel<128, 2, 2, 1>, a, st);
+}
+
+bool conv3_pair_applicable(int Cin, int Cout) { return Cin >= 256 && Cin % 64 == 0 && Cout % 128 == 0; }
+
 int conv3_pair_stat_rows(int N, int H, int W, int Cin, int Cout) {
   (void)Cin;
-  int bn, ntn, workers, tiles;
-  pair_geometry(N, H, W, Cout, &bn, &ntn, &workers, &tiles);
-  return 2 * workers;
+  return pair_stat_rows(N, H, W, Cout, pair_bn(Cout), pair_max_pairs());
 }
 
 int conv3_pair_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,
                       int W, int Cin, int Cout, cudaStream_t st, const float* scale,
                      const float* shift) {
+  const int bn = pair_bn(Cout);
   PairArgs a;
-  int bn;
-  pair_geometry(N, H, W, Cout, &bn, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cout;
-  a.kblocks = Cin / 64;
-  a.ktap = Cin;
-  a.stats = stats_partial;
-  a.scale = scale;
-  a.shift = shift;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  if (int e = make_tmap_4d(&a.tmA, x, Cin, W, H, N, xs, xs * W, xs * W * H, IN_W, IN_H)) return e;
-  if (int e = make_tmap_2d(&a.tmW, w, static_cast<uint64_t>(9) * Cin, Cout, bn / 2)) return e;
-  if (int e = make_tmap_4d(&a.tmO, y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH)) return e;
-  if (bn == 256) return launch_pair<256, 2, 6, 1>(a, st);
-  return launch_pair<128, 3, 8, 2>(a, st);
+  if (int e = pair_args(&a, x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, bn, pair_max_pairs(), scale, shift))
+    return e;
+  if (bn == 256) return launch_pair<PairPlan<256, 2, 6, 1>>(conv3_pair_kernel<256, 2, 6, 1>, a, st);
+  return launch_pair<PairPlan<128, 3, 8, 2>>(conv3_pair_kernel<128, 3, 8, 2>, a, st);
 }
 
 }  // namespace b2h

@@ -19,8 +19,6 @@
 #include "first_tile.cuh"
 #include "tc_common.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 using namespace b2;
@@ -441,18 +439,13 @@ int launch_res(const ResArgs& a, cudaStream_t st) {
   return b2h::check_launch("conv3_res");
 }
 
-// SMs the persistent grids may fill. B200UNET_RESERVE_SMS (set by the data-parallel bring-up) leaves a few SMs to the
-// concurrently running NCCL all-reduce kernels: the tile schedule is static, so a CTA that cannot become resident
-// because a communication CTA holds its SM would serialise behind the first wave.
+// SMs the persistent grids fill
 int num_sms() {
   static int n = 0;
   if (n == 0) {
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0)
       n = 148;
-    const char* e = getenv("B200UNET_RESERVE_SMS");
-    const int r = e ? atoi(e) : 0;
-    if (r > 0 && r < n / 2) n -= r;
   }
   return n;
 }

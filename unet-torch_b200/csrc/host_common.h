@@ -52,12 +52,12 @@ bool conv3_res_bnred_applicable(int Cin, int Cout);
 int conv3_res_bnred_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, const void* bn_y, int bn_y_cs,
                            const float* scale, const float* shift, const float* mean, const float* rstd, float* partial, int N,
                            int H, int W, int Cin, int Cout, cudaStream_t st);
-// conv3_res2.cu: the same as CTA pairs (tcgen05 cta_group::2, M = 256)
+// conv3_pair.cu: two CTA-pair kernels (tcgen05 cta_group::2, M = 256) on one skeleton. conv3_res2: the same layers as
+// conv3_res with the weights resident; conv3_pair: weights streamed, for Cin >= 256
 int conv3_res2_stat_rows(int N, int H, int W, int Cin, int Cout);
 int conv3_res2_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,
                       int W, int Cin, int Cout, cudaStream_t st, const float* scale = nullptr,
                      const float* shift = nullptr);
-// conv3_pair.cu: streaming CTA-pair kernel for Cin >= 256
 bool conv3_pair_applicable(int Cin, int Cout);
 int conv3_pair_stat_rows(int N, int H, int W, int Cin, int Cout);
 int conv3_pair_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,

@@ -335,7 +335,7 @@ bool use_resident(int Cin, int Cout) {
   return g_opt_res != 0 && b2h::conv3_res_applicable(Cin, Cout);
 }
 
-// CTA pairs (conv3_res2.cu) for the resident-weight layers. Measured on B200 (profiles/): pairs win 25-35 % when a
+// CTA pairs (conv3_res2_kernel, conv3_pair.cu) for the resident-weight layers. Measured on B200 (profiles/): pairs win 25-35 % when a
 // tile carries two K blocks (Cin = 128: 128->128, 128->256 and 128->64 up to 256^2), and lose when the per-tile MMA
 // burst is short (Cin = 64) or for 128->64 at 512^2 and above, where the cluster-wide barrier round trip per tile is
 // exposed. B200UNET_RES2=0 / 1 forces the choice off / on for every resident-weight layer.

@@ -308,7 +308,8 @@ def init_from_env(sync_bn=True, bucket_mb=25.0, graphs=None):
         torch.cuda.set_device(local)
         backend = "nccl"
         # Measured on 2 x B200 (scripts/gpu_scale.sh): NCCL's default CTA count next to full-width persistent grids is
-        # fastest (23.99 ms/step vs 24.28-24.43 with NCCL_MAX_CTAS=4/8 and B200UNET_RESERVE_SMS=4/8), so neither is set.
+        # fastest (23.99 ms/step vs 24.28-24.43 with NCCL_MAX_CTAS=4/8 or with 4/8 SMs kept free of the persistent
+        # conv grids), so neither is done.
     else:
         backend = "gloo"
     if not dist.is_initialized():
