@@ -251,6 +251,150 @@ def test_gate_checker_accepts_the_reference_and_flags_a_missing_term():
     assert [b[0] for b in check_gate(rec, tol_map=1e-9, tol_sum=1e-9, tol_grad=1e-9)] == ["dW_q"]
 
 
+def test_conv_check_references_agree_with_torch():
+    """tests/conv_check.py: the fp64 references of the exact convolution tests against F.conv2d / conv_transpose2d / autograd /
+    torch.nn.grad.conv2d_weight on random fp64 data."""
+    import torch.nn.functional as F
+
+    import conv_check as C
+
+    g = torch.Generator().manual_seed(3)
+    r = lambda *s: torch.randn(*s, generator=g, dtype=torch.float64)  # noqa: E731
+    x, w, dy = r(2, 5, 7, 6), r(4, 5, 3, 3), r(2, 4, 7, 6)
+    xv = x.clone().requires_grad_(True)
+    (F.conv2d(xv, w, padding=1) * dy).sum().backward()
+    assert torch.allclose(C.conv3x3(x, w), F.conv2d(x, w, padding=1), rtol=1e-12, atol=1e-12)
+    assert torch.allclose(C.conv3x3_dgrad(dy, w), xv.grad, rtol=1e-12, atol=1e-12)
+    assert torch.allclose(C.conv3x3_wgrad(x, dy), torch.nn.grad.conv2d_weight(x, w.shape, dy, padding=1), rtol=1e-12, atol=1e-12)
+    wt, b, du = r(5, 3, 2, 2), r(3), r(2, 3, 14, 12)
+    xv = x.clone().requires_grad_(True)
+    wv = wt.clone().requires_grad_(True)
+    (F.conv_transpose2d(xv, wv, b, stride=2) * du).sum().backward()
+    assert torch.allclose(C.convt2x2(x, wt, b), F.conv_transpose2d(x, wt, b, stride=2), rtol=1e-12, atol=1e-12)
+    assert torch.allclose(C.convt2x2_dgrad(du, wt), xv.grad, rtol=1e-12, atol=1e-12)
+    assert torch.allclose(C.convt2x2_wgrad(x, du), wv.grad, rtol=1e-12, atol=1e-12)
+    w1, b1 = r(4, 5), r(4)
+    assert torch.allclose(C.conv1x1(x, w1, b1), F.conv2d(x, w1[:, :, None, None], b1), rtol=1e-12, atol=1e-12)
+    assert torch.allclose(C.conv1x1_wgrad(x, dy), torch.nn.grad.conv2d_weight(x, (4, 5, 1, 1), dy)[:, :, 0, 0], rtol=1e-12,
+                          atol=1e-12)
+    # eval BatchNorm + ReLU and the fused backward reduction, against autograd of the same module in fp64
+    y, sc, sh, mean, rstd = r(2, 4, 7, 6), r(4), r(4), r(4), r(4).abs()
+    assert torch.equal(C.bn_relu_eval(y, sc, sh), torch.relu(y * sc.view(1, -1, 1, 1) + sh.view(1, -1, 1, 1)))
+    beta = r(4)
+    bv = beta.clone().requires_grad_(True)
+    gv = torch.ones(4, dtype=torch.float64, requires_grad=True)
+    xhat = (y - mean.view(1, -1, 1, 1)) * rstd.view(1, -1, 1, 1)
+    (torch.relu(gv.view(1, -1, 1, 1) * xhat + bv.view(1, -1, 1, 1)) * dy).sum().backward()
+    s1, s2 = C.bn_backward_sums(dy, y, rstd, beta - mean * rstd, mean, rstd)
+    assert torch.allclose(s1, bv.grad, rtol=1e-10, atol=1e-10) and torch.allclose(s2, gv.grad, rtol=1e-10, atol=1e-10)
+
+
+def _emulate_fp32_conv(x, w, orders, gen):
+    """An fp32 conv3x3 that accumulates its K = 9 * Cin products one at a time, in a shuffled order and split into K blocks whose
+    fp32 partials are added at the end (like a split-K kernel), then rounds to bf16 nearest-even."""
+    import torch.nn.functional as F
+
+    import conv_check as C
+
+    n, c, h, wd = x.shape
+    cols = F.unfold(x.float(), 3, padding=1).view(n, c * 9, h * wd)              # [n, K, P]
+    prods = cols[:, :, None, :] * w.float().view(w.shape[0], -1).t()[None, :, :, None]  # [n, K, Cout, P], exact
+    outs = []
+    for nsplit in orders:
+        perm = torch.randperm(c * 9, generator=gen)
+        parts = []
+        for chunk in perm.chunk(nsplit):
+            acc = torch.zeros(n, w.shape[0], h * wd)
+            for k in chunk.tolist():
+                acc = acc + prods[:, k]
+            parts.append(acc)
+        tot = parts[0]
+        for p in parts[1:]:
+            tot = tot + p
+        outs.append(C.bf16_rne(tot.view(n, -1, h, wd)).double())
+    return outs
+
+
+@pytest.mark.parametrize("regime", ["sparse", "dense"])
+def test_conv_check_exactness_holds_under_any_summation_order(regime):
+    """The argument behind the exact GPU tests: under each regime's invariant, an fp32 accumulation in any order and any K split
+    rounds to bf16_rne(exact fp64) bit for bit."""
+    import conv_check as C
+
+    g = torch.Generator().manual_seed(7 if regime == "sparse" else 8)
+    x = C.operand((2, 64, 10, 12), regime, 9 * 64, g)
+    w = C.operand((64, 64, 3, 3), regime, 9 * 64, g, sparse_input=False)
+    y = C.conv3x3(x, w)
+    C.check_regime(regime, y, C.conv3x3(x.abs(), w.abs()))
+    for got in _emulate_fp32_conv(x, w, (1, 3, 8), g):
+        C.assert_exact(C.nhwc(got), C.nhwc(C.bf16_rne(y)))
+
+
+def test_conv_check_flags_the_defects_rel_l2_accepts():
+    """Dense case N = 4, 160 x 160, 64 -> 64 (m = 12). A dropped tap on one edge pixel, one pixel written with its neighbour's
+    values and round-toward-zero instead of nearest-even all pass the old `rel_l2 < 1e-2` comparison and all fail
+    assert_exact; so do a statistics row left unwritten and an element written into the guard image."""
+    import torch.nn.functional as F
+
+    import conv_check as C
+
+    g = torch.Generator().manual_seed(9)
+    n, c, h, w = 4, 64, 160, 160
+    assert C.dense_m(9 * c) == 12
+    x = C.operand((n, c, h, w), C.DENSE, 9 * c, g)
+    wt = C.operand((c, c, 3, 3), C.DENSE, 9 * c, g, sparse_input=False)
+    y = C.conv3x3(x, wt)
+    C.check_regime(C.DENSE, y, C.conv3x3(x.abs(), wt.abs()))
+    want = C.nhwc(C.bf16_rne(y))
+    C.assert_exact(want, want)
+    # one tap (r = s = 0) missing on the bottom-right pixel of image 0, all channels
+    dropped = y.clone()
+    tap = (x[0, :, h - 2, w - 2][None, :] * wt[:, :, 0, 0]).sum(1)
+    dropped[0, :, h - 1, w - 1] -= tap
+    # pixel (5, 3) of image 1 holds pixel (5, 4)'s channels
+    moved = C.bf16_rne(y)
+    moved[1, :, 5, 3] = moved[1, :, 5, 4]
+    defects = {"dropped tap": C.nhwc(C.bf16_rne(dropped)), "neighbour pixel": C.nhwc(moved), "round toward zero":
+               C.nhwc(C.bf16_rz(y))}
+    for what, got in defects.items():
+        err = C.rel_l2(got, want)
+        assert err < 1e-2, (what, err)                     # the old metric accepts it ...
+        with pytest.raises(AssertionError, match="elements differ"):
+            C.assert_exact(got, want, what)                # ... the exact comparison does not
+    with pytest.raises(AssertionError, match=r"differ\n  \(n=0, h=159, w=159, c=\d+\).*image 0, 16x8 tile 199, 8x16 tile 199"):
+        C.assert_exact(defects["dropped tap"], want)
+    # statistics: one row left as its NaN sentinel
+    rows = 7
+    st = C.stats_buffer(rows, c, device="cpu")
+    st.view(rows + 1, 2 * c)[:rows] = 1.0
+    C.assert_stats_rows(st, rows, c)
+    st.view(rows + 1, 2 * c)[3] = C.stats_buffer(0, c, device="cpu").view(1, 2 * c)
+    with pytest.raises(AssertionError, match=r"rows \[3\]"):
+        C.assert_stats_rows(st, rows, c)
+    # output canvas: one element written into the guard image after the last one
+    canvas, target = C.bf16_canvas(2, 3, 5, c, device="cpu")
+    target.copy_(torch.zeros(2, 3, 5, c))
+    C.assert_canvas_intact(canvas, 2, c)
+    canvas[2, 1, 1, C.GUARD_C + 4] = 0.0
+    with pytest.raises(AssertionError, match="1 elements outside the target"):
+        C.assert_canvas_intact(canvas, 2, c)
+    # and an input canvas carries NaN into a convolution that reads past its slice
+    xcan, xs = C.input_canvas(torch.ones(1, 3, 5, 8), device="cpu")
+    wide = C.nhwc(F.conv2d(C.nchw(xcan[:1, :, :, C.GUARD_C - 1:C.GUARD_C + 8].double()), torch.ones(1, 9, 3, 3, dtype=torch.float64),
+                           padding=1))
+    assert bool(torch.isnan(wide).all()) and torch.equal(xs.double(), torch.ones(1, 3, 5, 8, dtype=torch.float64))
+
+
+def test_conv_check_recorder_reads_profiler_names():
+    import conv_check as C
+
+    assert C.kernel_name("void (anonymous namespace)::conv3_pair_kernel<256, 2, 6, 1>((anonymous namespace)::PairArgs)") == \
+        "conv3_pair_kernel<256, 2, 6, 1>"
+    assert C.kernel_name("void (anonymous namespace)::conv3_res_kernel<64, 1, 3, 2, 9, 0, 0, true>((anonymous namespace)::ResArgs)") \
+        == "conv3_res_kernel<64, 1, 3, 2, 9, 0, 0, true>"
+    assert C.kernel_name("(anonymous namespace)::wgrad_swap3_kernel((anonymous namespace)::WgradArgs)") == "wgrad_swap3_kernel"
+
+
 def test_bench_dump_outputs_samples_each_array_by_its_own_size_within_budget(tmp_path, monkeypatch):
     """bench.py --dump-outputs: an array longer than the per-array cap is cut to a fixed seeded sample that depends only on
     its own size (identical from run to run, and when other arrays come or go, so two builds compare element for
