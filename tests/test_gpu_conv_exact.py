@@ -8,13 +8,15 @@ the target. The 3x3 shapes cover a one-pixel image, images smaller than a tile w
 CTA of a pair gets the out-of-range tile), an odd tile count, ragged tiles in both geometries, a deep persistent schedule
 (depth derived from conv3x3_stat_rows and asserted) and more than one channel slice (ntiles_n > 1).
 
-Not tested here, because the switches that reach them are read once per process from the environment:
-wgrad_swap_kernel<1> (the Cin = 64 weight gradient with B200UNET_WGRAD_SWAP3=0) and igemm_kernel<0, 256, 3, 4>
-(B200UNET_BN=256). The module skips when one of those variables, B200UNET_NO_WGRAD_SWAP or B200UNET_NO_BNRED is set, since
-the expected kernels would then be wrong."""
+The table's kernels are exactly the tensor-core instantiations compiled into libb200unet.so (checked against the library's
+machine code). The module skips when B200UNET_NO_WGRAD_SWAP or B200UNET_NO_BNRED is set: both are read once per process
+and change which kernel a case runs, so the expected kernels would be wrong."""
 import collections
 import math
 import os
+import re
+import shutil
+import subprocess
 import zlib
 from dataclasses import dataclass, field
 
@@ -25,7 +27,7 @@ import conv_check as C
 
 pytestmark = pytest.mark.gpu
 
-_ENV = [v for v in ("B200UNET_NO_WGRAD_SWAP", "B200UNET_WGRAD_SWAP3", "B200UNET_NO_BNRED", "B200UNET_BN") if v in os.environ]
+_ENV = [v for v in ("B200UNET_NO_WGRAD_SWAP", "B200UNET_NO_BNRED") if v in os.environ]
 if _ENV:
     pytest.skip(f"{', '.join(_ENV)} set: the kernel choice it controls is fixed per process, the expected kernels would be wrong",
                 allow_module_level=True)
@@ -102,12 +104,15 @@ def _cases():
     for s in ((1, 3, 5), (3, 20, 12)):
         out.append(Case(f"convt-stats-cin256-{'x'.join(map(str, s))}", "convt_stats", "igemm_kernel<1, 256, 3, 4>", RES, s, 256,
                         128))
-    gather = [(_res(128, 4, 4, 1, 1, 2), RES, 128), (_res(128, 8, 3, 1, 1, 2), RES, 256),
-              ("igemm_kernel<2, 128, 2, 4>", RES, 512), ("igemm_kernel<2, 128, 2, 4>", IGEMM, 128)]
-    for kern, choice, cin in gather:
+    # (kernel, choice, Cin, Cup); Cin = 192 is not a multiple of 128, so igemm takes 64 columns per tile
+    gather = [(_res(128, 4, 4, 1, 1, 2), RES, 128, 64), (_res(128, 8, 3, 1, 1, 2), RES, 256, 128),
+              ("igemm_kernel<2, 128, 2, 4>", RES, 512, 256), ("igemm_kernel<2, 128, 2, 4>", IGEMM, 128, 64),
+              ("igemm_kernel<2, 64, 3, 6>", RES, 192, 64)]
+    for kern, choice, cin, cup in gather:
+        cups = "" if cup == cin // 2 else f"-cup{cup}"
         for s, regime in (((1, 1, 1), C.SPARSE), ((2, 5, 9), C.SPARSE), ((3, 20, 12), C.DENSE)):
-            out.append(Case(f"convt-dgrad-{regime}-{_short(kern)}-cin{cin}-{'x'.join(map(str, s))}", "convt_dgrad", kern, choice,
-                            s, cin, cin // 2, regime))
+            out.append(Case(f"convt-dgrad-{regime}-{_short(kern)}-cin{cin}{cups}-{'x'.join(map(str, s))}", "convt_dgrad", kern,
+                            choice, s, cin, cup, regime))
     # 1x1 convolutions: igemm MODE_UP with bias + statistics, the resident K = 64 kernel (TAPS = 1) with and without statistics
     for kern, cout in (("igemm_kernel<1, 128, 2, 4>", 128), ("igemm_kernel<1, 64, 3, 6>", 64)):
         for s, regime in (((2, 5, 9), C.SPARSE), ((3, 20, 12), C.SPARSE), ((2, 20, 12), C.DENSE)):
@@ -479,6 +484,37 @@ RUNNERS = {
 def test_exact(ops, kernel_choice, case):
     kernel_choice(case.choice)
     RUNNERS[case.op](case, ops)
+
+
+def _cuda_tool(name):
+    for cand in (shutil.which(name), os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", name)):
+        if cand and os.path.exists(cand):
+            return cand
+    return None
+
+
+def _profiler_spelling(demangled):
+    """'void <unnamed>::conv3_res_kernel<(int)64, ..., (bool)1>(<unnamed>::ResArgs)' -> 'conv3_res_kernel<64, ..., true>'."""
+    s = re.sub(r"\(bool\)([01])", lambda m: "true" if m.group(1) == "1" else "false", demangled)
+    s = re.sub(r"\(int\)(-?\d+)", r"\1", s)
+    return C.kernel_name(s.replace("<unnamed>::", ""))
+
+
+def test_library_instantiations_are_the_table():
+    """Every tensor-core instantiation compiled into libb200unet.so has a case in the table, and every kernel the table names
+    is compiled: a new instantiation without a case fails here."""
+    from unet_torch_b200 import _lib
+
+    cuobjdump, cufilt = _cuda_tool("cuobjdump"), _cuda_tool("cu++filt")
+    if cuobjdump is None or cufilt is None:
+        pytest.skip("cuobjdump / cu++filt not found")
+    sass = subprocess.run([cuobjdump, "-sass", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    mangled = re.findall(r"Function : (\S+)", sass)
+    demangled = subprocess.run([cufilt], input="\n".join(mangled), capture_output=True, text=True, check=True).stdout.splitlines()
+    assert len(demangled) == len(mangled)
+    built = {n for n in map(_profiler_spelling, demangled) if n.split("<")[0] in TC_FAMILIES}
+    table = {c.kernel for c in CASES}
+    assert built == table, f"compiled without a case: {sorted(built - table)}; in the table but not compiled: {sorted(table - built)}"
 
 
 def test_every_instantiation_in_the_table_ran():

@@ -75,6 +75,17 @@ int make_tmap_4d(CUtensorMap* m, const void* base, uint64_t d0, uint64_t d1, uin
   return 0;
 }
 
+int make_pixel_shuffle_maps(CUtensorMap m[4], const void* canvas, int C, int pitch, int N, int H, int W, int H2, int W2,
+                            int pad_top, int pad_left, uint32_t box_w, uint32_t box_h) {
+  const uint64_t s = static_cast<uint64_t>(pitch) * 2;
+  for (int ij = 0; ij < 4; ++ij) {
+    const int i = ij >> 1, j = ij & 1;
+    const uint8_t* base = static_cast<const uint8_t*>(canvas) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * s;
+    if (int e = make_tmap_4d(&m[ij], base, C, W, H, N, 2 * s, 2 * s * W2, s * W2 * H2, box_w, box_h)) return e;
+  }
+  return 0;
+}
+
 int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t k, uint64_t rows, uint32_t box_rows) {
   EncodeTiledFn enc = get_encode();
   if (!enc) {

@@ -358,14 +358,8 @@ using PairKernel = void (*)(PairArgs);
 template <class P>
 int launch_pair(PairKernel kern, const PairArgs& a, cudaStream_t st) {
   const char* name = P::RESIDENT ? "conv3_res2" : "conv3_pair";
-  static unsigned long long configured = 0;  // one bit per CUDA device
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("%s: cudaFuncSetAttribute(smem=%d): %s", name, P::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
+  static unsigned long long configured = 0;
+  if (int e = b2h::opt_in_smem(kern, P::TOTAL, configured, name)) return e;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3(2 * a.workers * a.ntiles_n);
   cfg.blockDim = dim3(192);
@@ -455,10 +449,9 @@ static int pair_args(PairArgs* a, const void* x, int x_cs, const void* w, void* 
   a->stats = stats_partial;
   a->scale = scale;
   a->shift = shift;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  if (int e = make_tmap_4d(&a->tmA, x, Cin, W, H, N, xs, xs * W, xs * W * H, IN_W, IN_H)) return e;
+  if (int e = make_nhwc_map(&a->tmA, x, Cin, x_cs, N, H, W, IN_W, IN_H)) return e;
   if (int e = make_tmap_2d(&a->tmW, w, static_cast<uint64_t>(9) * Cin, Cout, bn / 2)) return e;
-  return make_tmap_4d(&a->tmO, y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH);
+  return make_nhwc_map(&a->tmO, y, Cout, y_cs, N, H, W, RTW, RTH);
 }
 
 int conv3_res2_stat_rows(int N, int H, int W, int Cin, int Cout) {

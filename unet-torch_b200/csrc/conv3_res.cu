@@ -426,15 +426,9 @@ __global__ void __launch_bounds__(res_threads(KIND, OB), 1) conv3_res_kernel(con
 template <int BN, int KB, int NA, int OB, int TAPS, int KIND = RES_CONV, int CIN = 0, bool BNRED = false>
 int launch_res(const ResArgs& a, cudaStream_t st) {
   using P = ResPlan<BN, KB, NA, OB, TAPS, KIND, BNRED>;
-  static unsigned long long configured = 0;  // one bit per CUDA device
+  static unsigned long long configured = 0;
   auto kern = conv3_res_kernel<BN, KB, NA, OB, TAPS, KIND, CIN, BNRED>;
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("conv3_res: cudaFuncSetAttribute(smem=%d): %s", P::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
+  if (int e = b2h::opt_in_smem(kern, P::TOTAL, configured, "conv3_res")) return e;
   kern<<<a.workers * a.ntiles_n, res_threads(KIND, OB), P::TOTAL, st>>>(a);
   return b2h::check_launch("conv3_res");
 }
@@ -460,21 +454,26 @@ bool conv3_res_applicable(int Cin, int Cout) {
 
 static int res_bn(int Cin, int Cout) { return (Cin == 64 && Cout % 128 == 0) ? 128 : 64; }
 
-// geometry shared by the launchers and the statistics-row queries
-static void res_geometry(int N, int H, int W, int bn, int Cout, int* ntn, int* workers, int* tiles) {
-  *ntn = Cout / bn;
-  *tiles = N * ceil_div(H, RTH) * ceil_div(W, RTW);
-  int w = num_sms() / *ntn;
-  if (w < 1) w = 1;
-  if (w > *tiles) w = *tiles;
-  *workers = w;
+// Geometry of a persistent launch over an N x H x W pixel grid with ncols GEMM columns in bn-wide channel slices (shared by
+// the launchers and the statistics-row queries); one column group, every optional pointer null, tensor maps to be encoded
+// by the caller.
+static ResArgs res_args(int N, int H, int W, int ncols, int bn) {
+  ResArgs a = {};
+  a.tiles_w = ceil_div(W, RTW);
+  a.tiles_h = ceil_div(H, RTH);
+  a.tiles_total = N * a.tiles_w * a.tiles_h;
+  a.H = H;
+  a.W = W;
+  a.ncols = ncols;
+  a.cup = ncols;
+  a.ntiles_n = ncols / bn;
+  a.workers = num_sms() / a.ntiles_n;
+  if (a.workers < 1) a.workers = 1;
+  if (a.workers > a.tiles_total) a.workers = a.tiles_total;
+  return a;
 }
 
-int conv3_res_stat_rows(int N, int H, int W, int Cin, int Cout) {
-  int ntn, workers, tiles;
-  res_geometry(N, H, W, res_bn(Cin, Cout), Cout, &ntn, &workers, &tiles);
-  return workers;
-}
+int conv3_res_stat_rows(int N, int H, int W, int Cin, int Cout) { return res_args(N, H, W, Cout, res_bn(Cin, Cout)).workers; }
 
 // BatchNorm-backward reduction fused into a backward-data launch (Cin = Cout = 64: the level-0 layers, where the separate
 // reduce pass reads 1.07 GB): bn_y = pre-BN tensor of the BatchNorm whose OUTPUT gradient this launch produces.
@@ -483,109 +482,62 @@ bool conv3_res_bnred_applicable(int Cin, int Cout) { return Cin == 64 && Cout ==
 int conv3_res_bnred_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, const void* bn_y, int bn_y_cs,
                            const float* scale, const float* shift, const float* mean, const float* rstd, float* partial, int N,
                            int H, int W, int Cin, int Cout, cudaStream_t st) {
-  ResArgs a;
-  res_geometry(N, H, W, 64, Cout, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cout;
+  ResArgs a = res_args(N, H, W, Cout, 64);
   a.stats = partial;
   a.scale = scale;
   a.shift = shift;
   a.bn_mean = mean;
   a.bn_rstd = rstd;
-  a.cup = Cout;
-  a.bias = nullptr;
-  a.x_nchw = nullptr;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2, bs = static_cast<uint64_t>(bn_y_cs) * 2;
-  if (int e = make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TileGeom<9>::IN_W, TileGeom<9>::IN_H)) return e;
+  if (int e = make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, TileGeom<9>::IN_W, TileGeom<9>::IN_H)) return e;
   if (int e = make_tmap_2d(&a.tmW, w, static_cast<uint64_t>(9) * Cin, Cout, 64)) return e;
-  if (int e = make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH)) return e;
-  if (int e = make_tmap_4d(&a.tmY, bn_y, Cout, W, H, N, bs, bs * W, bs * W * H, RTW, RTH)) return e;
-  for (int i = 1; i < 4; ++i) { a.tmA[i] = a.tmA[0]; a.tmO[i] = a.tmO[0]; }
+  if (int e = make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, RTW, RTH)) return e;
+  if (int e = make_nhwc_map(&a.tmY, bn_y, Cout, bn_y_cs, N, H, W, RTW, RTH)) return e;
   return launch_res<64, 1, 3, 2, 9, RES_CONV, 0, true>(a, st);
 }
 
 int conv3_res_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,
                      int W, int Cin, int Cout, cudaStream_t st, const float* scale,
                      const float* shift) {
-  ResArgs a;
   const int bn = res_bn(Cin, Cout);
-  res_geometry(N, H, W, bn, Cout, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cout;
+  ResArgs a = res_args(N, H, W, Cout, bn);
   a.stats = stats_partial;
   a.scale = scale;
   a.shift = shift;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  a.cup = Cout;
-  a.bias = nullptr;
-  a.x_nchw = nullptr;
-  if (int e = make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TileGeom<9>::IN_W, TileGeom<9>::IN_H)) return e;
+  if (int e = make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, TileGeom<9>::IN_W, TileGeom<9>::IN_H)) return e;
   if (int e = make_tmap_2d(&a.tmW, w, static_cast<uint64_t>(9) * Cin, Cout, bn)) return e;
-  if (int e = make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH)) return e;
-  for (int i = 1; i < 4; ++i) { a.tmA[i] = a.tmA[0]; a.tmO[i] = a.tmO[0]; }
+  if (int e = make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, RTW, RTH)) return e;
   if (Cin == 64 && bn == 64) return launch_res<64, 1, 4, 2, 9>(a, st);
   if (Cin == 64 && bn == 128) return launch_res<128, 1, 2, 1, 9>(a, st);
   return launch_res<64, 2, 2, 2, 9>(a, st);
 }
 
 // 1x1 convolution of a 64-channel NHWC tensor (the im2col'ed network input) with a [Cout][64] bf16 operand.
-int conv1x1_c64_stat_rows(int N, int H, int W, int Cout) {
-  int ntn, workers, tiles;
-  res_geometry(N, H, W, 64, Cout, &ntn, &workers, &tiles);
-  return workers;
-}
+int conv1x1_c64_stat_rows(int N, int H, int W, int Cout) { return res_args(N, H, W, Cout, 64).workers; }
 
 int conv1x1_c64_launch(const void* x, int x_cs, const void* w, void* y, int y_cs, float* stats_partial, int N, int H,
                        int W, int Cout, cudaStream_t st, const float* scale,
                      const float* shift) {
-  ResArgs a;
-  res_geometry(N, H, W, 64, Cout, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cout;
+  ResArgs a = res_args(N, H, W, Cout, 64);
   a.stats = stats_partial;
   a.scale = scale;
   a.shift = shift;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  a.cup = Cout;
-  a.bias = nullptr;
-  a.x_nchw = nullptr;
-  if (int e = make_tmap_4d(&a.tmA[0], x, 64, W, H, N, xs, xs * W, xs * W * H, RTW, RTH)) return e;
+  if (int e = make_nhwc_map(&a.tmA[0], x, 64, x_cs, N, H, W, RTW, RTH)) return e;
   if (int e = make_tmap_2d(&a.tmW, w, 64, Cout, 64)) return e;
-  if (int e = make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH)) return e;
-  for (int i = 1; i < 4; ++i) { a.tmA[i] = a.tmA[0]; a.tmO[i] = a.tmO[0]; }
+  if (int e = make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, RTW, RTH)) return e;
   return launch_res<64, 1, 4, 2, 1>(a, st);
 }
 
 // inc.conv1 straight from the fp32 NCHW network input: the im2col rows are built in shared memory (RES_FIRST).
 int conv3x3_first_launch(const float* x_nchw, const void* w1, void* y, int y_cs, float* stats_partial, int N, int H, int W,
                          int Cin, int Cout, cudaStream_t st, const float* scale, const float* shift) {
-  ResArgs a;
-  res_geometry(N, H, W, 64, Cout, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cout;
+  ResArgs a = res_args(N, H, W, Cout, 64);
   a.stats = stats_partial;
   a.scale = scale;
   a.shift = shift;
-  a.cup = Cout;
-  a.bias = nullptr;
   a.x_nchw = x_nchw;
-  const uint64_t ys = static_cast<uint64_t>(y_cs) * 2;
   if (int e = make_tmap_2d(&a.tmW, w1, 64, Cout, 64)) return e;
-  if (int e = make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, RTW, RTH)) return e;
-  for (int i = 0; i < 4; ++i) a.tmA[i] = a.tmO[0];  // unused by RES_FIRST (prefetch target only)
-  for (int i = 1; i < 4; ++i) a.tmO[i] = a.tmO[0];
+  if (int e = make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, RTW, RTH)) return e;
+  a.tmA[0] = a.tmO[0];  // unused by RES_FIRST (prefetch target only)
   switch (Cin) {
     case 1: return launch_res<64, 1, 4, 2, 1, RES_FIRST, 1>(a, st);
     case 2: return launch_res<64, 1, 4, 2, 1, RES_FIRST, 2>(a, st);
@@ -606,29 +558,13 @@ bool convt_res_applicable(int Cin, int Cup) { return (Cin == 128 || Cin == 256 |
 
 int convt_res_fprop_launch(const void* x, int x_cs, const void* w_fprop, const float* bias, void* out, int out_cs, int N,
                            int H, int W, int Cin, int Cup, int H2, int W2, int pad_top, int pad_left, cudaStream_t st) {
-  ResArgs a;
   const int bn = (Cin == 128) ? 256 : 128;
-  res_geometry(N, H, W, bn, 4 * Cup, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = 4 * Cup;
+  ResArgs a = res_args(N, H, W, 4 * Cup, bn);
   a.cup = Cup;
-  a.stats = nullptr;
-  a.scale = nullptr;
-  a.shift = nullptr;
-  a.x_nchw = nullptr;
   a.bias = bias;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, os = static_cast<uint64_t>(out_cs) * 2;
-  if (int e = make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, RTW, RTH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmA[i] = a.tmA[0];
+  if (int e = make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, RTW, RTH)) return e;
   if (int e = make_tmap_2d(&a.tmW, w_fprop, Cin, static_cast<uint64_t>(4) * Cup, bn)) return e;
-  for (int ij = 0; ij < 4; ++ij) {
-    const int i = ij >> 1, j = ij & 1;
-    const uint8_t* base = static_cast<const uint8_t*>(out) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * os;
-    if (int e = make_tmap_4d(&a.tmO[ij], base, Cup, W, H, N, 2 * os, 2 * os * W2, os * W2 * H2, RTW, RTH)) return e;
-  }
+  if (int e = make_pixel_shuffle_maps(a.tmO, out, Cup, out_cs, N, H, W, H2, W2, pad_top, pad_left, RTW, RTH)) return e;
   if (Cin == 128) return launch_res<256, 2, 4, 1, 1, RES_UP>(a, st);
   if (Cin == 256) return launch_res<128, 4, 4, 1, 1, RES_UP>(a, st);
   return launch_res<128, 8, 3, 1, 1, RES_UP>(a, st);
@@ -639,28 +575,10 @@ bool convt_res_dgrad_applicable(int Cin, int Cup) { return (Cin == 128 || Cin ==
 
 int convt_res_dgrad_launch(const void* du, int du_cs, const void* w_dgrad, void* dx, int dx_cs, int N, int H, int W,
                            int Cin, int Cup, int H2, int W2, int pad_top, int pad_left, cudaStream_t st) {
-  ResArgs a;
-  res_geometry(N, H, W, 128, Cin, &a.ntiles_n, &a.workers, &a.tiles_total);
-  a.tiles_w = ceil_div(W, RTW);
-  a.tiles_h = ceil_div(H, RTH);
-  a.H = H;
-  a.W = W;
-  a.ncols = Cin;
-  a.cup = Cin;
-  a.stats = nullptr;
-  a.scale = nullptr;
-  a.shift = nullptr;
-  a.x_nchw = nullptr;
-  a.bias = nullptr;
-  const uint64_t us = static_cast<uint64_t>(du_cs) * 2, xs = static_cast<uint64_t>(dx_cs) * 2;
-  for (int ij = 0; ij < 4; ++ij) {
-    const int i = ij >> 1, j = ij & 1;
-    const uint8_t* base = static_cast<const uint8_t*>(du) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * us;
-    if (int e = make_tmap_4d(&a.tmA[ij], base, Cup, W, H, N, 2 * us, 2 * us * W2, us * W2 * H2, RTW, RTH)) return e;
-  }
+  ResArgs a = res_args(N, H, W, Cin, 128);
+  if (int e = make_pixel_shuffle_maps(a.tmA, du, Cup, du_cs, N, H, W, H2, W2, pad_top, pad_left, RTW, RTH)) return e;
   if (int e = make_tmap_2d(&a.tmW, w_dgrad, static_cast<uint64_t>(4) * Cup, Cin, 128)) return e;
-  if (int e = make_tmap_4d(&a.tmO[0], dx, Cin, W, H, N, xs, xs * W, xs * W * H, RTW, RTH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmO[i] = a.tmO[0];
+  if (int e = make_nhwc_map(&a.tmO[0], dx, Cin, dx_cs, N, H, W, RTW, RTH)) return e;
   if (Cin == 128) return launch_res<128, 4, 4, 1, 1, RES_GATHER>(a, st);
   return launch_res<128, 8, 3, 1, 1, RES_GATHER>(a, st);
 }

@@ -19,6 +19,17 @@ int make_tmap_4d(CUtensorMap* m, const void* base, uint64_t d0, uint64_t d1, uin
 // 2-D K-major bf16 matrix [rows][k] (pitch k elements), box = {64, box_rows}, 128B swizzle.
 int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t k, uint64_t rows, uint32_t box_rows);
 
+// C channels of an NHWC bf16 tensor [N][H][W][pitch] (a channel slice when C < pitch).
+inline int make_nhwc_map(CUtensorMap* m, const void* base, int C, int pitch, int N, int H, int W, uint32_t box_w,
+                         uint32_t box_h) {
+  const uint64_t s = static_cast<uint64_t>(pitch) * 2;
+  return make_tmap_4d(m, base, C, W, H, N, s, s * W, s * W * H, box_w, box_h);
+}
+// The four pixel-shuffle sub-grids of a ConvTranspose2d(k2, s2) map: m[2i + j] is the H x W grid of canvas pixels
+// (pad_top + 2h + i, pad_left + 2w + j), C channels, of the NHWC bf16 canvas [N][H2][W2][pitch].
+int make_pixel_shuffle_maps(CUtensorMap m[4], const void* canvas, int C, int pitch, int N, int H, int W, int H2, int W2,
+                            int pad_top, int pad_left, uint32_t box_w, uint32_t box_h);
+
 #define B2_REQUIRE(cond, ...)        \
   do {                               \
     if (!(cond)) {                   \
@@ -30,14 +41,20 @@ int make_tmap_2d(CUtensorMap* m, const void* base, uint64_t k, uint64_t rows, ui
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
 // Kernel attributes (opt-in dynamic shared memory) are per device: each kernel instantiation keeps one bit per CUDA device
-// and configures itself on its first launch there (a process may drive several GPUs).
-inline bool first_use_on_device(unsigned long long& mask) {
+// in `configured` and opts in to `bytes` on its first launch there (a process may drive several GPUs). 0, or 2 + message.
+template <class Kernel>
+int opt_in_smem(Kernel* kern, int bytes, unsigned long long& configured, const char* what) {
   int dev = 0;
   cudaGetDevice(&dev);
   const unsigned long long bit = 1ull << (dev & 63);
-  if (mask & bit) return false;
-  mask |= bit;
-  return true;
+  if (configured & bit) return 0;
+  configured |= bit;
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  if (e != cudaSuccess) {
+    set_error("%s: cudaFuncSetAttribute(smem=%d): %s", what, bytes, cudaGetErrorString(e));
+    return 2;
+  }
+  return 0;
 }
 
 // scale/shift (optional, [Cout] each): eval-mode BatchNorm + ReLU folded into the epilogue (stats_partial must be null)

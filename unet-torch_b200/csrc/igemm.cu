@@ -277,43 +277,47 @@ __global__ void __launch_bounds__(192) igemm_kernel(const __grid_constant__ Igem
 }
 
 // ----------------------------------------------------------------------------------------------- host side
+// Geometry of a launch over an H x W pixel grid, K = ktap per tap, ncols GEMM columns in groups of cup (statistics rows of
+// cup channels); every optional pointer null, tensor maps to be encoded by the caller.
+IgemmArgs igemm_args(int H, int W, int ktap, int ncols, int cup) {
+  IgemmArgs a = {};
+  a.tiles_w = b2h::ceil_div(W, TW);
+  a.tiles_h = b2h::ceil_div(H, TH);
+  a.H = H;
+  a.W = W;
+  a.kblocks = ktap / 64;
+  a.ktap = ktap;
+  a.ncols = ncols;
+  a.cup = cup;
+  a.stat_c = cup;
+  return a;
+}
+
 template <int MODE, int BN, int NA, int NB>
-int launch_t(const IgemmArgs& a, int mtiles, cudaStream_t st) {
+int launch_t(const IgemmArgs& a, int N, cudaStream_t st) {
   using Plan = SmemPlan<MODE, BN, NA, NB>;
-  static unsigned long long configured = 0;  // one bit per CUDA device
+  static unsigned long long configured = 0;
   auto kern = igemm_kernel<MODE, BN, NA, NB>;
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Plan::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("igemm: cudaFuncSetAttribute(smem=%d): %s", Plan::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
-  const long long grid = static_cast<long long>(mtiles) * a.ntiles_n;
+  if (int e = b2h::opt_in_smem(kern, Plan::TOTAL, configured, "igemm")) return e;
+  const long long grid = static_cast<long long>(N) * a.tiles_w * a.tiles_h * a.ntiles_n;
   kern<<<static_cast<unsigned>(grid), 192, Plan::TOTAL, st>>>(a);
   return b2h::check_launch("igemm");
 }
 
-int env_bn() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("B200UNET_BN");
-    v = e ? atoi(e) : 0;
-  }
-  return v;
-}
-
+// BN = 256 only for the ConvTranspose2d forward (all four (i,j) sub-positions of 64 channels per CTA)
 template <int MODE>
-int launch_mode(IgemmArgs& a, int bn, int mtiles, cudaStream_t st) {
+int launch_mode(IgemmArgs& a, int bn, int N, cudaStream_t st) {
   a.ntiles_n = a.ncols / bn;
-  switch (bn) {
-    case 64: return launch_t<MODE, 64, 3, 6>(a, mtiles, st);
-    case 128: return launch_t<MODE, 128, 2, 4>(a, mtiles, st);
-    case 256: return launch_t<MODE, 256, 3, 4>(a, mtiles, st);
+  if (bn == 64) return launch_t<MODE, 64, 3, 6>(a, N, st);
+  if (bn == 128) return launch_t<MODE, 128, 2, 4>(a, N, st);
+  if constexpr (MODE == MODE_UP) {
+    if (bn == 256) return launch_t<MODE, 256, 3, 4>(a, N, st);
   }
   b2h::set_error("igemm: bad BN %d", bn);
   return 1;
 }
+
+int pick_bn(int ncols) { return ncols % 128 == 0 ? 128 : 64; }
 
 // Kernel-selection overrides: -1 = automatic (measured rules below), 0 = off, 1 = forced on. Initialised from the
 // environment (B200UNET_NO_RES, B200UNET_RES2, B200UNET_PAIR), changeable at run time with b200unet_set_kernel_choice.
@@ -335,29 +339,25 @@ bool use_resident(int Cin, int Cout) {
   return g_opt_res != 0 && b2h::conv3_res_applicable(Cin, Cout);
 }
 
-// CTA pairs (conv3_res2_kernel, conv3_pair.cu) for the resident-weight layers. Measured on B200 (profiles/): pairs win 25-35 % when a
-// tile carries two K blocks (Cin = 128: 128->128, 128->256 and 128->64 up to 256^2), and lose when the per-tile MMA
-// burst is short (Cin = 64) or for 128->64 at 512^2 and above, where the cluster-wide barrier round trip per tile is
-// exposed. B200UNET_RES2=0 / 1 forces the choice off / on for every resident-weight layer.
-bool use_pairs(int N, int H, int W, int Cin, int Cout) {
-  init_opts();
-  if (g_opt_res2 >= 0) return g_opt_res2 == 1;
-  if (Cin != 128) return false;
-  return Cout >= 128 || static_cast<long long>(N) * H * W <= 16ll * 256 * 256;
-}
+enum class Conv3Path { RESIDENT, RESIDENT_PAIRS, STREAMING_PAIRS, IGEMM };
 
-// streaming CTA-pair kernel (conv3_pair.cu) for the deep layers; B200UNET_PAIR=0 keeps the one-tile-per-CTA igemm
-bool use_stream_pairs(int Cin, int Cout) {
+// The kernel a 3x3 convolution runs on. The launch and the statistics-row queries all read this one decision, so a buffer
+// sized from a query always matches the kernel that fills it.
+Conv3Path conv3_path(int N, int H, int W, int Cin, int Cout) {
   init_opts();
-  return g_opt_pair != 0 && b2h::conv3_pair_applicable(Cin, Cout);
-}
-
-int pick_bn(int ncols, int limit) {
-  int want = env_bn();
-  if (want != 64 && want != 128 && want != 256) want = 128;
-  int bn = want;
-  while (bn > 64 && (ncols % bn != 0 || bn > limit)) bn >>= 1;
-  return bn;
+  if (use_resident(Cin, Cout)) {
+    // CTA pairs (conv3_res2_kernel, conv3_pair.cu) for the resident-weight layers. Measured on B200 (profiles/): pairs win
+    // 25-35 % when a tile carries two K blocks (Cin = 128: 128->128, 128->256 and 128->64 up to 256^2), and lose when the
+    // per-tile MMA burst is short (Cin = 64) or for 128->64 at 512^2 and above, where the cluster-wide barrier round trip per
+    // tile is exposed. B200UNET_RES2=0 / 1 forces the choice off / on for every resident-weight layer.
+    bool pairs;
+    if (g_opt_res2 >= 0) pairs = g_opt_res2 == 1;
+    else pairs = Cin == 128 && (Cout >= 128 || static_cast<long long>(N) * H * W <= 16ll * 256 * 256);
+    return pairs ? Conv3Path::RESIDENT_PAIRS : Conv3Path::RESIDENT;
+  }
+  // streaming CTA-pair kernel (conv3_pair.cu) for the deep layers; B200UNET_PAIR=0 keeps the one-tile-per-CTA igemm
+  if (g_opt_pair != 0 && b2h::conv3_pair_applicable(Cin, Cout)) return Conv3Path::STREAMING_PAIRS;
+  return Conv3Path::IGEMM;
 }
 
 // conv3x3 dispatch shared by the training entry point (BN statistics epilogue) and the eval entry point (BatchNorm + ReLU
@@ -367,38 +367,26 @@ int conv3x3_dispatch(const void* x, int x_cs, const void* w, void* y, int y_cs, 
   B2_REQUIRE(Cin % 64 == 0 && Cout % 64 == 0, "conv3x3_igemm: Cin (%d) and Cout (%d) must be multiples of 64", Cin, Cout);
   B2_REQUIRE(N > 0 && H > 0 && W > 0, "conv3x3_igemm: empty tensor");
   B2_REQUIRE(x_cs >= Cin && y_cs >= Cout && x_cs % 8 == 0 && y_cs % 8 == 0, "conv3x3_igemm: bad pitches %d %d", x_cs, y_cs);
-  if (use_resident(Cin, Cout)) {
-    if (use_pairs(N, H, W, Cin, Cout))
-      return b2h::conv3_res2_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, static_cast<cudaStream_t>(stream),
-                                    scale, shift);
-    return b2h::conv3_res_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, static_cast<cudaStream_t>(stream),
-                                 scale, shift);
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  switch (conv3_path(N, H, W, Cin, Cout)) {
+    case Conv3Path::RESIDENT:
+      return b2h::conv3_res_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, st, scale, shift);
+    case Conv3Path::RESIDENT_PAIRS:
+      return b2h::conv3_res2_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, st, scale, shift);
+    case Conv3Path::STREAMING_PAIRS:
+      return b2h::conv3_pair_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, st, scale, shift);
+    case Conv3Path::IGEMM:
+      break;
   }
-  if (use_stream_pairs(Cin, Cout))
-    return b2h::conv3_pair_launch(x, x_cs, w, y, y_cs, stats_partial, N, H, W, Cin, Cout, static_cast<cudaStream_t>(stream),
-                                  scale, shift);
-  IgemmArgs a;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.H = H;
-  a.W = W;
-  a.kblocks = Cin / 64;
-  a.ktap = Cin;
-  a.ncols = Cout;
-  a.cup = Cout;
-  a.stat_c = Cout;
+  IgemmArgs a = igemm_args(H, W, Cin, Cout, Cout);
   a.stats = stats_partial;
   a.scale = scale;
   a.shift = shift;
-  a.bias = nullptr;
-  const int bn = pick_bn(Cout, 256);
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH + 2)) return e;
-  for (int i = 1; i < 4; ++i) a.tmA[i] = a.tmA[0];
+  const int bn = pick_bn(Cout);
+  if (int e = b2h::make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, TW, TH + 2)) return e;
   if (int e = b2h::make_tmap_2d(&a.tmB, w, static_cast<uint64_t>(9) * Cin, Cout, bn)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmO[i] = a.tmO[0];
-  return launch_mode<MODE_CONV3>(a, bn, N * a.tiles_w * a.tiles_h, static_cast<cudaStream_t>(stream));
+  if (int e = b2h::make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, TW, TH)) return e;
+  return launch_mode<MODE_CONV3>(a, bn, N, st);
 }
 
 int convt2x2_fprop_impl(const void* x, int x_cs, const void* w_fprop, const float* bias, void* out, int out_cs, float* stats,
@@ -411,31 +399,15 @@ int convt2x2_fprop_impl(const void* x, int x_cs, const void* w_fprop, const floa
   if (stats == nullptr && use_resident(64, 64) && b2h::convt_res_applicable(Cin, Cup))
     return b2h::convt_res_fprop_launch(x, x_cs, w_fprop, bias, out, out_cs, N, H, W, Cin, Cup, H2, W2, pad_top, pad_left,
                                        static_cast<cudaStream_t>(stream));
-  IgemmArgs a;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.H = H;
-  a.W = W;
-  a.kblocks = Cin / 64;
-  a.ktap = Cin;
-  a.ncols = 4 * Cup;
-  a.cup = Cup;
+  IgemmArgs a = igemm_args(H, W, Cin, 4 * Cup, Cup);
   a.stat_c = stat_c;
   a.stats = stats;
-  a.scale = nullptr;
-  a.shift = nullptr;
   a.bias = bias;
-  const int bn = (env_bn() == 0) ? 256 : pick_bn(4 * Cup, 256);  // all four (i,j) sub-positions of 64 channels per CTA
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, os = static_cast<uint64_t>(out_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmA[i] = a.tmA[0];
+  const int bn = 256;  // all four (i,j) sub-positions of 64 channels per CTA
+  if (int e = b2h::make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, TW, TH)) return e;
   if (int e = b2h::make_tmap_2d(&a.tmB, w_fprop, Cin, static_cast<uint64_t>(4) * Cup, bn)) return e;
-  for (int ij = 0; ij < 4; ++ij) {
-    const int i = ij >> 1, j = ij & 1;
-    const uint8_t* base = static_cast<const uint8_t*>(out) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * os;
-    if (int e = b2h::make_tmap_4d(&a.tmO[ij], base, Cup, W, H, N, 2 * os, 2 * os * W2, os * W2 * H2, TW, TH)) return e;
-  }
-  return launch_mode<MODE_UP>(a, bn, N * a.tiles_w * a.tiles_h, static_cast<cudaStream_t>(stream));
+  if (int e = b2h::make_pixel_shuffle_maps(a.tmO, out, Cup, out_cs, N, H, W, H2, W2, pad_top, pad_left, TW, TH)) return e;
+  return launch_mode<MODE_UP>(a, bn, N, static_cast<cudaStream_t>(stream));
 }
 
 
@@ -457,7 +429,7 @@ int b200unet_conv3x3_bn_relu_igemm(const void* x, int x_cs, const void* w, const
 }
 
 int b200unet_conv3x3_dgrad_bnred_rows(int N, int H, int W, int Cin, int Cout) {
-  if (!(use_resident(Cin, Cout) && !use_pairs(N, H, W, Cin, Cout) && b2h::conv3_res_bnred_applicable(Cin, Cout))) return 0;
+  if (!(conv3_path(N, H, W, Cin, Cout) == Conv3Path::RESIDENT && b2h::conv3_res_bnred_applicable(Cin, Cout))) return 0;
   static int off = -1;
   if (off < 0) {
     const char* e = getenv("B200UNET_NO_BNRED");
@@ -489,9 +461,12 @@ int b200unet_set_kernel_choice(int resident, int resident_pairs, int streaming_p
 }
 
 int b200unet_conv3x3_stat_rows(int N, int H, int W, int Cin, int Cout) {
-  if (use_resident(Cin, Cout))
-    return use_pairs(N, H, W, Cin, Cout) ? b2h::conv3_res2_stat_rows(N, H, W, Cin, Cout) : b2h::conv3_res_stat_rows(N, H, W, Cin, Cout);
-  if (use_stream_pairs(Cin, Cout)) return b2h::conv3_pair_stat_rows(N, H, W, Cin, Cout);
+  switch (conv3_path(N, H, W, Cin, Cout)) {
+    case Conv3Path::RESIDENT: return b2h::conv3_res_stat_rows(N, H, W, Cin, Cout);
+    case Conv3Path::RESIDENT_PAIRS: return b2h::conv3_res2_stat_rows(N, H, W, Cin, Cout);
+    case Conv3Path::STREAMING_PAIRS: return b2h::conv3_pair_stat_rows(N, H, W, Cin, Cout);
+    case Conv3Path::IGEMM: break;
+  }
   return N * b2h::ceil_div(H, TH) * b2h::ceil_div(W, TW);
 }
 
@@ -525,28 +500,16 @@ int b200unet_conv1x1_fprop(const void* x, int x_cs, const void* w, const float* 
   // a one-tile-per-CTA launch - the persistent resident-weight kernel streams the tiles instead
   if (Cin == 64 && bias == nullptr && stats_partial == nullptr && use_resident(64, 64))
     return b2h::conv1x1_c64_launch(x, x_cs, w, y, y_cs, nullptr, N, H, W, Cout, static_cast<cudaStream_t>(stream));
-  IgemmArgs a;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.H = H;
-  a.W = W;
-  a.kblocks = Cin / 64;
-  a.ktap = Cin;
-  a.ncols = Cout;
-  a.cup = Cout;  // one column group: the scatter epilogue of the ConvTranspose2d mode degenerates to a plain NHWC store
+  // one column group: the scatter epilogue of the ConvTranspose2d mode degenerates to a plain NHWC store
+  IgemmArgs a = igemm_args(H, W, Cin, Cout, Cout);
   a.stat_c = stat_channels;
   a.stats = stats_partial;
-  a.scale = nullptr;
-  a.shift = nullptr;
   a.bias = bias;
-  const int bn = pick_bn(Cout, 256);
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(y_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmA[i] = a.tmA[0];
+  const int bn = pick_bn(Cout);
+  if (int e = b2h::make_nhwc_map(&a.tmA[0], x, Cin, x_cs, N, H, W, TW, TH)) return e;
   if (int e = b2h::make_tmap_2d(&a.tmB, w, Cin, Cout, bn)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmO[0], y, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmO[i] = a.tmO[0];
-  return launch_mode<MODE_UP>(a, bn, N * a.tiles_w * a.tiles_h, static_cast<cudaStream_t>(stream));
+  if (int e = b2h::make_nhwc_map(&a.tmO[0], y, Cout, y_cs, N, H, W, TW, TH)) return e;
+  return launch_mode<MODE_UP>(a, bn, N, static_cast<cudaStream_t>(stream));
 }
 
 
@@ -558,31 +521,12 @@ int b200unet_convt2x2_dgrad(const void* du, int du_cs, const void* w_dgrad, void
   if (use_resident(64, 64) && b2h::convt_res_dgrad_applicable(Cin, Cup))
     return b2h::convt_res_dgrad_launch(du, du_cs, w_dgrad, dx, dx_cs, N, H, W, Cin, Cup, H2, W2, pad_top, pad_left,
                                        static_cast<cudaStream_t>(stream));
-  IgemmArgs a;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.H = H;
-  a.W = W;
-  a.kblocks = Cup / 64;
-  a.ktap = Cup;
-  a.ncols = Cin;
-  a.cup = Cin;
-  a.stat_c = Cin;
-  a.stats = nullptr;
-  a.scale = nullptr;
-  a.shift = nullptr;
-  a.bias = nullptr;
-  const int bn = pick_bn(Cin, 256);
-  const uint64_t us = static_cast<uint64_t>(du_cs) * 2, xs = static_cast<uint64_t>(dx_cs) * 2;
-  for (int ij = 0; ij < 4; ++ij) {
-    const int i = ij >> 1, j = ij & 1;
-    const uint8_t* base = static_cast<const uint8_t*>(du) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * us;
-    if (int e = b2h::make_tmap_4d(&a.tmA[ij], base, Cup, W, H, N, 2 * us, 2 * us * W2, us * W2 * H2, TW, TH)) return e;
-  }
+  IgemmArgs a = igemm_args(H, W, Cup, Cin, Cin);
+  const int bn = pick_bn(Cin);
+  if (int e = b2h::make_pixel_shuffle_maps(a.tmA, du, Cup, du_cs, N, H, W, H2, W2, pad_top, pad_left, TW, TH)) return e;
   if (int e = b2h::make_tmap_2d(&a.tmB, w_dgrad, static_cast<uint64_t>(4) * Cup, Cin, bn)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmO[0], dx, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmO[i] = a.tmO[0];
-  return launch_mode<MODE_GATHER4>(a, bn, N * a.tiles_w * a.tiles_h, static_cast<cudaStream_t>(stream));
+  if (int e = b2h::make_nhwc_map(&a.tmO[0], dx, Cin, dx_cs, N, H, W, TW, TH)) return e;
+  return launch_mode<MODE_GATHER4>(a, bn, N, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

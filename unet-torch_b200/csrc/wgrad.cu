@@ -323,15 +323,9 @@ int pick_splits(int base_ctas, int tiles_total) {
 template <int KIND, int BNC, int CIN = 0>
 int launch_wgrad(const WgradArgs& a, cudaStream_t st) {
   using P = WPlan<KIND, BNC>;
-  static unsigned long long configured = 0;  // one bit per CUDA device
+  static unsigned long long configured = 0;
   auto kern = wgrad_kernel<KIND, BNC, CIN>;
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("wgrad: cudaFuncSetAttribute(smem=%d): %s", P::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
+  if (int e = b2h::opt_in_smem(kern, P::TOTAL, configured, "wgrad")) return e;
   const int grid = a.mtiles * a.ntiles * (KIND == KIND_CONV3 ? 3 : 1) * a.splits;
   kern<<<grid, wgrad_threads(KIND), P::TOTAL, st>>>(a);
   return b2h::check_launch("wgrad");
@@ -341,30 +335,27 @@ int launch_wgrad(const WgradArgs& a, cudaStream_t st) {
 // ---------------------------------------------------------------------------------------------------------------------
 // Cout = 64 layers (inc.conv2, up4.conv1, up4.conv2 at 512^2: 20 % of the wgrad FLOPs). With dy on the M side half of
 // every 128-row MMA would be idle, so the roles are swapped: M = x channels, N = the 64 dy channels.
-// One CTA covers ALL NINE taps of its pixel tiles from ONE x tile with a full halo (10 rows x 18 pixels): a K step is
-// the 16 pixels of one tile row, i.e. 16 consecutive 128-byte rows of the halo tile starting at pixel row
-// (k + r) * 18 + s - any start works because the swizzle is a function of the absolute address (tests/test_gpu_probe.py).
-// One x + one dy tile per 8x16 pixels instead of three of each keeps the kernel off the L2->SM limit it hit with one
-// CTA per horizontal tap (ncu: 3.4x the tensor bytes, 58 % tensor-pipe active).
-//   CB = 2 (Cin = 128): M = 128 x channels; one MMA per tap, 9 accumulators of 64 columns would need 576 TMEM columns,
-//                       so the CTA runs the taps of ONE horizontal shift s (grid x3), 3 accumulators.
-//   CB = 1 (Cin = 64) : two vertical taps are STACKED in M: the second 64-row block of the MN-major A descriptor is
-//                       "the same 64 channels one halo row further down" (LBO = 18 pixels = 2304 B), so taps (0,s),(1,s)
-//                       are one M = 128 MMA and tap (2,s) rides in a second one (upper half discarded): 6 accumulators
-//                       of 64 columns, all 9 taps in one CTA.
+// A CTA covers the three vertical taps of one horizontal shift s (grid x3) of its pixel tiles from ONE x tile with a full
+// halo (10 rows x 18 pixels): a K step is the 16 pixels of one tile row, i.e. 16 consecutive 128-byte rows of the halo tile
+// starting at pixel row (k + r) * 18 + s - any start works because the swizzle is a function of the absolute address
+// (tests/test_gpu_probe.py). One x + one dy tile per 8x16 pixels instead of three of each keeps the kernel off the L2->SM
+// limit it hit with one CTA per horizontal tap (ncu: 3.4x the tensor bytes, 58 % tensor-pipe active).
+// CB = 2 (Cin = 128, the only instantiation): M = 128 x channels, one MMA per tap; 9 accumulators of 64 columns would need
+// 576 TMEM columns, hence one s per CTA and 3 accumulators. Cin = 64 runs wgrad_swap3_kernel below.
 // Partials: [z][tap][Cin][64].
 template <int CB>
 struct WSPlan {
+  static_assert(CB == 2, "Cin = 128: two 64-channel x boxes per stage");
   static constexpr int HW_ = TW + 2;                       // halo tile width in pixels
   static constexpr int X_BOX = (TH + 2) * HW_ * 128;       // 23040
-  static constexpr int X_BOX_PAD = (X_BOX + 2 * HW_ * 128 + 1023) / 1024 * 1024;  // + the junk rows tap "3" touches
+  // + two spare halo rows: not read, kept so the stage layout stays the one the kernel was measured with
+  static constexpr int X_BOX_PAD = (X_BOX + 2 * HW_ * 128 + 1023) / 1024 * 1024;
   static constexpr int Y_BOX = BM * 128;                   // 16384
   static constexpr int STAGE = CB * X_BOX_PAD + Y_BOX;
   static constexpr int NS_MAX = (227 * 1024 - 2048) / STAGE;
   static constexpr int NS = NS_MAX > 5 ? 5 : NS_MAX;
-  static constexpr int S_PER_CTA = (CB == 1) ? 3 : 1;      // horizontal taps handled by one CTA
-  static constexpr int NACC = (CB == 1) ? 6 : 3;
-  static constexpr int TMEM_COLS = (CB == 1) ? 512 : 256;
+  static constexpr int NACC = 3;
+  static constexpr int TMEM_COLS = 256;
   static constexpr int BAR_OFF = NS * STAGE;
   static constexpr int TOTAL = BAR_OFF + 256 + 1024;
 };
@@ -383,8 +374,8 @@ __global__ void __launch_bounds__(192, 1) wgrad_swap_kernel(const __grid_constan
   const uint32_t tmem_slot = acc_full + 8;
   volatile uint32_t* tmem_slot_gen = reinterpret_cast<volatile uint32_t*>(smem_gen + P::BAR_OFF + 8 * (2 * NS) + 8);
   const int warp = warp_idx_uniform(), lane = threadIdx.x & 31;
-  const int s_cta = (P::S_PER_CTA == 1) ? static_cast<int>(blockIdx.x % 3) : 0;
-  const int z = (P::S_PER_CTA == 1) ? static_cast<int>(blockIdx.x / 3) : static_cast<int>(blockIdx.x);
+  const int s_cta = static_cast<int>(blockIdx.x % 3);
+  const int z = static_cast<int>(blockIdx.x / 3);
   const int t_begin = static_cast<int>(static_cast<long long>(args.tiles_total) * z / args.splits);
   const int t_end = static_cast<int>(static_cast<long long>(args.tiles_total) * (z + 1) / args.splits);
 
@@ -437,19 +428,10 @@ __global__ void __launch_bounds__(192, 1) wgrad_swap_kernel(const __grid_constan
 #pragma unroll
         for (int k = 0; k < BM / 16; ++k) {  // 16 pixels (one tile row) per MMA
           const uint32_t b_lo = umma_desc_lo(sY + k * 2048, P::Y_BOX);
-          if (CB == 2) {
 #pragma unroll
-            for (int r = 0; r < 3; ++r)
-              umma_bf16_lh(tmem_base + r * 64, umma_desc_lo(sX + ((k + r) * HW_ + s_cta) * 128, P::X_BOX_PAD), d_hi, b_lo,
-                           d_hi, idesc, acc);
-          } else {
-#pragma unroll
-            for (int s = 0; s < 3; ++s)
-#pragma unroll
-              for (int pr = 0; pr < 2; ++pr)
-                umma_bf16_lh(tmem_base + (s * 2 + pr) * 64, umma_desc_lo(sX + ((k + 2 * pr) * HW_ + s) * 128, HW_ * 128),
-                             d_hi, b_lo, d_hi, idesc, acc);
-          }
+          for (int r = 0; r < 3; ++r)
+            umma_bf16_lh(tmem_base + r * 64, umma_desc_lo(sX + ((k + r) * HW_ + s_cta) * 128, P::X_BOX_PAD), d_hi, b_lo,
+                         d_hi, idesc, acc);
           acc = 1;
         }
         umma_commit(empty(st));
@@ -466,22 +448,18 @@ __global__ void __launch_bounds__(192, 1) wgrad_swap_kernel(const __grid_constan
     const int Cin = args.Cb;
 #pragma unroll 1
     for (int a = 0; a < P::NACC; ++a) {
-      int r, s, c;
-      if (CB == 2) { r = a; s = s_cta; c = row; }
-      else { s = a >> 1; r = 2 * (a & 1) + (row >> 6); c = row & 63; }
+      const int r = a, s = s_cta, c = row;
       float* dst = args.partial + ((static_cast<size_t>(z) * 9 + (r * 3 + s)) * Cin + c) * 64;
 #pragma unroll 1
       for (int h = 0; h < 2; ++h) {
         uint32_t v[32];
         tmem_ld32(tmem_base + (static_cast<uint32_t>(quad * 32) << 16) + a * 64 + h * 32, v);
         tmem_ld_wait();
-        if (r < 3) {
-          float4* d4 = reinterpret_cast<float4*>(dst + h * 32);
+        float4* d4 = reinterpret_cast<float4*>(dst + h * 32);
 #pragma unroll
-          for (int j = 0; j < 8; ++j)
-            d4[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]),
-                                __uint_as_float(v[4 * j + 3]));
-        }
+        for (int j = 0; j < 8; ++j)
+          d4[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]), __uint_as_float(v[4 * j + 2]),
+                              __uint_as_float(v[4 * j + 3]));
       }
     }
     tc_fence_before();
@@ -491,11 +469,12 @@ __global__ void __launch_bounds__(192, 1) wgrad_swap_kernel(const __grid_constan
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Cin = Cout = 64 (inc.conv2, up4.conv2 at 512^2), round 2: the THREE HORIZONTAL TAPS STACKED ON N.
-// wgrad_swap_kernel<1> issues six 128x64x16 MMAs per 16-pixel K step; each reads 4 KB (A) + 2 KB (B) of shared memory per 32
-// tensor cycles = 192 B/clk against the 128 B/clk the SM delivers (ncu: 51 % of the bf16 peak, tensor pipe 58 %). Here the
-// dy operand carries a one-pixel horizontal halo and its MN-major descriptor takes N = 192 = three 64-channel blocks ONE PIXEL
-// (LBO = 128 B) apart: block b is "dy shifted by b pixels", i.e. tap s = 2 - b, because
+// Cin = Cout = 64 (inc.conv2, up4.conv2 at 512^2): the THREE HORIZONTAL TAPS STACKED ON N.
+// With only the vertical taps stacked on M (a second 64-row block of the MN-major A descriptor one halo row further down),
+// a 16-pixel K step is six 128x64x16 MMAs; each reads 4 KB (A) + 2 KB (B) of shared memory per 32 tensor cycles = 192 B/clk
+// against the 128 B/clk the SM delivers (ncu: 51 % of the bf16 peak, tensor pipe 58 %). Here the dy operand carries a
+// one-pixel horizontal halo and its MN-major descriptor takes N = 192 = three 64-channel blocks ONE PIXEL (LBO = 128 B)
+// apart: block b is "dy shifted by b pixels", i.e. tap s = 2 - b, because
 //     dW[k,c,r,s] = sum_q x[q + (r-1, 0), c] * dy[q + (0, 1-s), k]          (the sum re-indexed by the x pixel q).
 // With the two vertical taps stacked on M as before (LBO = one x row = 2048 B) a K step is TWO 128x192x16 MMAs (taps
 // (0..1, 0..2) and (2..3, 0..2), r = 3 discarded): 4 KB + 6 KB per 96 cycles = 107 B/clk - no longer bound by shared memory.
@@ -620,27 +599,10 @@ __global__ void __launch_bounds__(192, 1) wgrad_swap3_kernel(const __grid_consta
 }
 
 int launch_wgrad_swap3(const WgradArgs& a, cudaStream_t st) {
-  using P = WS3Plan;
-  static unsigned long long configured = 0;  // one bit per CUDA device
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_swap3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("wgrad_swap3: cudaFuncSetAttribute(smem=%d): %s", P::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
-  wgrad_swap3_kernel<<<a.splits, 192, P::TOTAL, st>>>(a);
+  static unsigned long long configured = 0;
+  if (int e = b2h::opt_in_smem(wgrad_swap3_kernel, WS3Plan::TOTAL, configured, "wgrad_swap3")) return e;
+  wgrad_swap3_kernel<<<a.splits, 192, WS3Plan::TOTAL, st>>>(a);
   return b2h::check_launch("wgrad_swap3");
-}
-
-// B200UNET_WGRAD_SWAP3=0 keeps wgrad_swap_kernel<1> for the 64 -> 64 layers
-bool use_swap3() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("B200UNET_WGRAD_SWAP3");
-    on = (e == nullptr || atoi(e) != 0) ? 1 : 0;
-  }
-  return on == 1;
 }
 
 // partial [Z][9][C][64] -> dw OIHW [64][C][3][3]
@@ -654,19 +616,11 @@ __global__ void reduce_conv3_swapped_kernel(const float* __restrict__ partial, f
   }
 }
 
-template <int CB>
 int launch_wgrad_swap(const WgradArgs& a, cudaStream_t st) {
-  using P = WSPlan<CB>;
-  static unsigned long long configured = 0;  // one bit per CUDA device
-  auto kern = wgrad_swap_kernel<CB>;
-  if (b2h::first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P::TOTAL);
-    if (e != cudaSuccess) {
-      b2h::set_error("wgrad_swap: cudaFuncSetAttribute(smem=%d): %s", P::TOTAL, cudaGetErrorString(e));
-      return 2;
-    }
-  }
-  kern<<<P::S_PER_CTA == 1 ? 3 * a.splits : a.splits, 192, P::TOTAL, st>>>(a);
+  using P = WSPlan<2>;
+  static unsigned long long configured = 0;
+  if (int e = b2h::opt_in_smem(wgrad_swap_kernel<2>, P::TOTAL, configured, "wgrad_swap")) return e;
+  wgrad_swap_kernel<2><<<3 * a.splits, 192, P::TOTAL, st>>>(a);
   return b2h::check_launch("wgrad_swap");
 }
 
@@ -677,6 +631,39 @@ bool use_swap(int Cin, int Cout) {
     off = (e && atoi(e) != 0) ? 1 : 0;
   }
   return !off && Cout == 64 && (Cin == 64 || Cin == 128);
+}
+
+// Pixel-tile fields and CTA grid of wgrad_kernel<KIND_UP / KIND_PLAIN / KIND_FIRST, 64> over N x H x W: 128 A-side x 64
+// B-side channels per CTA, split over the pixel tiles; every optional pointer null, tensor maps to be encoded by the caller.
+WgradArgs wgrad_args(int N, int H, int W, int Ca, int Cb, float* partial) {
+  WgradArgs a = {};
+  a.tiles_w = b2h::ceil_div(W, TW);
+  a.tiles_h = b2h::ceil_div(H, TH);
+  a.tiles_total = N * a.tiles_w * a.tiles_h;
+  a.mtiles = b2h::ceil_div(Ca, 128);
+  a.ntiles = Cb / 64;
+  a.splits = pick_splits(a.mtiles * a.ntiles, a.tiles_total);
+  a.Ca = Ca;
+  a.Cb = Cb;
+  a.partial = partial;
+  a.H = H;
+  a.W = W;
+  return a;
+}
+
+// the 3x3 weight gradient: A = dy (Cout), B = x (Cin). wgrad_kernel and wgrad_swap_kernel run one horizontal tap per CTA
+// (grid x3), wgrad_swap3_kernel all nine
+WgradArgs conv3_wgrad_args(int N, int H, int W, int Cin, int Cout, float* partial) {
+  WgradArgs a = wgrad_args(N, H, W, Cout, Cin, partial);
+  if (use_swap(Cin, Cout)) {
+    a.mtiles = 1;
+    a.ntiles = 1;
+    a.splits = pick_splits(Cin == 64 ? 1 : 3, a.tiles_total);
+  } else {
+    a.ntiles = Cin / conv3_bnc(Cin);
+    a.splits = pick_splits(a.mtiles * a.ntiles * 3, a.tiles_total);
+  }
+  return a;
 }
 
 }  // namespace
@@ -699,73 +686,33 @@ int b200unet_prep_convt2x2_weight(const float* w, void* w_fprop, void* w_dgrad, 
   return b2h::check_launch("prep_convt2x2_weight");
 }
 
-static void conv3_wgrad_geometry(int N, int H, int W, int Cin, int Cout, int* bnc, int* mtiles, int* ntiles, int* tiles,
-                                 int* splits) {
-  *bnc = conv3_bnc(Cin);
-  *mtiles = b2h::ceil_div(Cout, 128);
-  *ntiles = Cin / *bnc;
-  *tiles = N * b2h::ceil_div(H, TH) * b2h::ceil_div(W, TW);
-  if (use_swap(Cin, Cout)) {
-    *mtiles = 1;
-    *ntiles = 1;
-    *splits = pick_splits(Cin == 64 ? 1 : 3, *tiles);
-    return;
-  }
-  *splits = pick_splits(*mtiles * *ntiles * 3, *tiles);
-}
-
 int64_t b200unet_conv3x3_wgrad_workspace_floats(int N, int H, int W, int Cin, int Cout) {
-  int bnc, mt, nt, tiles, z;
-  conv3_wgrad_geometry(N, H, W, Cin, Cout, &bnc, &mt, &nt, &tiles, &z);
-  return static_cast<int64_t>(z) * Cout * 9 * Cin;
+  return static_cast<int64_t>(conv3_wgrad_args(N, H, W, Cin, Cout, nullptr).splits) * Cout * 9 * Cin;
 }
 
 int b200unet_conv3x3_wgrad(const void* x, int x_cs, const void* dy, int dy_cs, float* partial, float* dw_oihw, int N,
                            int H, int W, int Cin, int Cout, b200_stream_t stream) {
   B2_REQUIRE(Cin % 64 == 0 && Cout % 64 == 0, "conv3x3_wgrad: Cin (%d) and Cout (%d) must be multiples of 64", Cin, Cout);
   B2_REQUIRE(x_cs % 8 == 0 && dy_cs % 8 == 0, "conv3x3_wgrad: pitches must be multiples of 8");
-  WgradArgs a;
-  int bnc;
-  conv3_wgrad_geometry(N, H, W, Cin, Cout, &bnc, &a.mtiles, &a.ntiles, &a.tiles_total, &a.splits);
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.Ca = Cout;
-  a.Cb = Cin;
-  a.partial = partial;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(dy_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA, dy, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmB[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH + 2)) return e;
-  for (int i = 1; i < 4; ++i) a.tmB[i] = a.tmB[0];
+  WgradArgs a = conv3_wgrad_args(N, H, W, Cin, Cout, partial);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (use_swap(Cin, Cout)) {
-    if (Cin == 64 && use_swap3()) {  // the three horizontal taps stacked on N: x with a vertical, dy with a horizontal halo
-      if (int e = b2h::make_tmap_4d(&a.tmB[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH + 2)) return e;
-      if (int e = b2h::make_tmap_4d(&a.tmA, dy, Cout, W, H, N, ys, ys * W, ys * W * H, TW + 2, TH)) return e;
-      if (int e = launch_wgrad_swap3(a, st)) return e;
-    } else {
-      if (int e = b2h::make_tmap_4d(&a.tmB[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW + 2, TH + 2)) return e;
-      if (int e = (Cin == 64) ? launch_wgrad_swap<1>(a, st) : launch_wgrad_swap<2>(a, st)) return e;
-    }
+  const bool swap = use_swap(Cin, Cout), swap3 = swap && Cin == 64;
+  // halos: x vertical (split-tap kernel, swap3) or full (swap); dy none, or horizontal for swap3 (taps stacked on N)
+  if (int e = b2h::make_nhwc_map(&a.tmA, dy, Cout, dy_cs, N, H, W, swap3 ? TW + 2 : TW, TH)) return e;
+  if (int e = b2h::make_nhwc_map(&a.tmB[0], x, Cin, x_cs, N, H, W, swap && !swap3 ? TW + 2 : TW, TH + 2)) return e;
+  if (swap) {
+    if (int e = swap3 ? launch_wgrad_swap3(a, st) : launch_wgrad_swap(a, st)) return e;
     reduce_conv3_swapped_kernel<<<b2h::ceil_div(9 * Cin * 64, 256), 256, 0, st>>>(partial, dw_oihw, a.splits, Cin);
     return b2h::check_launch("conv3x3_wgrad_reduce");
   }
-  int e = (bnc == 128) ? launch_wgrad<KIND_CONV3, 128>(a, st) : launch_wgrad<KIND_CONV3, 64>(a, st);
+  int e = (conv3_bnc(Cin) == 128) ? launch_wgrad<KIND_CONV3, 128>(a, st) : launch_wgrad<KIND_CONV3, 64>(a, st);
   if (e) return e;
   reduce_conv3_kernel<<<dim3(Cin / 64, Cout), 192, 0, st>>>(partial, dw_oihw, a.splits, Cout, Cin);
   return b2h::check_launch("conv3x3_wgrad_reduce");
 }
 
-static void up_wgrad_geometry(int N, int H, int W, int Cin, int Cup, int* mtiles, int* ntiles, int* tiles, int* splits) {
-  *mtiles = b2h::ceil_div(Cin, 128);
-  *ntiles = Cup / 64;
-  *tiles = N * b2h::ceil_div(H, TH) * b2h::ceil_div(W, TW);
-  *splits = pick_splits(*mtiles * *ntiles, *tiles);
-}
-
 int64_t b200unet_convt2x2_wgrad_workspace_floats(int N, int H, int W, int Cin, int Cup) {
-  int mt, nt, tiles, z;
-  up_wgrad_geometry(N, H, W, Cin, Cup, &mt, &nt, &tiles, &z);
-  return static_cast<int64_t>(z) * Cin * 4 * Cup;
+  return static_cast<int64_t>(wgrad_args(N, H, W, Cin, Cup, nullptr).splits) * Cin * 4 * Cup;
 }
 
 int b200unet_convt2x2_wgrad(const void* x, int x_cs, const void* du, int du_cs, float* partial, float* dw, int N, int H,
@@ -773,20 +720,9 @@ int b200unet_convt2x2_wgrad(const void* x, int x_cs, const void* du, int du_cs, 
   B2_REQUIRE(Cin % 64 == 0 && Cup % 64 == 0, "convt2x2_wgrad: Cin (%d) and Cup (%d) must be multiples of 64", Cin, Cup);
   B2_REQUIRE(pad_top >= 0 && pad_left >= 0 && 2 * H + pad_top <= H2 && 2 * W + pad_left <= W2, "convt2x2_wgrad: bad canvas");
   B2_REQUIRE(x_cs % 8 == 0 && du_cs % 8 == 0, "convt2x2_wgrad: pitches must be multiples of 8");
-  WgradArgs a;
-  up_wgrad_geometry(N, H, W, Cin, Cup, &a.mtiles, &a.ntiles, &a.tiles_total, &a.splits);
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.Ca = Cin;
-  a.Cb = Cup;
-  a.partial = partial;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, us = static_cast<uint64_t>(du_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA, x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH)) return e;
-  for (int ij = 0; ij < 4; ++ij) {
-    const int i = ij >> 1, j = ij & 1;
-    const uint8_t* base = static_cast<const uint8_t*>(du) + (static_cast<uint64_t>(pad_top + i) * W2 + pad_left + j) * us;
-    if (int e = b2h::make_tmap_4d(&a.tmB[ij], base, Cup, W, H, N, 2 * us, 2 * us * W2, us * W2 * H2, TW, TH)) return e;
-  }
+  WgradArgs a = wgrad_args(N, H, W, Cin, Cup, partial);
+  if (int e = b2h::make_nhwc_map(&a.tmA, x, Cin, x_cs, N, H, W, TW, TH)) return e;
+  if (int e = b2h::make_pixel_shuffle_maps(a.tmB, du, Cup, du_cs, N, H, W, H2, W2, pad_top, pad_left, TW, TH)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int e = launch_wgrad<KIND_UP, 64>(a, st)) return e;
   const size_t total = static_cast<size_t>(Cin) * 4 * Cup;
@@ -795,51 +731,25 @@ int b200unet_convt2x2_wgrad(const void* x, int x_cs, const void* du, int du_cs, 
   return b2h::check_launch("convt2x2_wgrad_reduce");
 }
 
-static void plain_wgrad_geometry(int N, int H, int W, int Cout, int* mtiles, int* tiles, int* splits) {
-  *mtiles = b2h::ceil_div(Cout, 128);
-  *tiles = N * b2h::ceil_div(H, TH) * b2h::ceil_div(W, TW);
-  *splits = pick_splits(*mtiles, *tiles);
-}
-
 int64_t b200unet_conv1x1_c64_wgrad_workspace_floats(int N, int H, int W, int Cout) {
-  int mt, tiles, z;
-  plain_wgrad_geometry(N, H, W, Cout, &mt, &tiles, &z);
-  return static_cast<int64_t>(z) * Cout * 64;
+  return static_cast<int64_t>(wgrad_args(N, H, W, Cout, 64, nullptr).splits) * Cout * 64;
 }
 
 int b200unet_conv1x1_c64_wgrad(const void* col, int col_cs, const void* dy, int dy_cs, float* partial, float* dw, int N,
                                int H, int W, int T, int Cout, b200_stream_t stream) {
   B2_REQUIRE(Cout % 64 == 0 && T >= 1 && T <= 64, "conv1x1_c64_wgrad: Cout=%d must be a multiple of 64 and T=%d in [1,64]", Cout, T);
   B2_REQUIRE(col_cs % 8 == 0 && dy_cs % 8 == 0 && col_cs >= 64, "conv1x1_c64_wgrad: bad pitches");
-  WgradArgs a;
-  plain_wgrad_geometry(N, H, W, Cout, &a.mtiles, &a.tiles_total, &a.splits);
-  a.ntiles = 1;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.Ca = Cout;
-  a.Cb = 64;
-  a.partial = partial;
-  const uint64_t cs = static_cast<uint64_t>(col_cs) * 2, ys = static_cast<uint64_t>(dy_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA, dy, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmB[0], col, 64, W, H, N, cs, cs * W, cs * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmB[i] = a.tmB[0];
+  WgradArgs a = wgrad_args(N, H, W, Cout, 64, partial);
+  if (int e = b2h::make_nhwc_map(&a.tmA, dy, Cout, dy_cs, N, H, W, TW, TH)) return e;
+  if (int e = b2h::make_nhwc_map(&a.tmB[0], col, 64, col_cs, N, H, W, TW, TH)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int e = launch_wgrad<KIND_PLAIN, 64>(a, st)) return e;
   reduce_plain_kernel<<<b2h::ceil_div(Cout * T, 256), 256, 0, st>>>(partial, dw, a.splits, Cout, Cout, T, 64);
   return b2h::check_launch("conv1x1_c64_wgrad_reduce");
 }
 
-static void conv1x1_wgrad_geometry(int N, int H, int W, int Cin, int Cout, int* mtiles, int* ntiles, int* tiles, int* splits) {
-  *mtiles = b2h::ceil_div(Cout, 128);
-  *ntiles = Cin / 64;
-  *tiles = N * b2h::ceil_div(H, TH) * b2h::ceil_div(W, TW);
-  *splits = pick_splits(*mtiles * *ntiles, *tiles);
-}
-
 int64_t b200unet_conv1x1_wgrad_workspace_floats(int N, int H, int W, int Cin, int Cout) {
-  int mt, nt, tiles, z;
-  conv1x1_wgrad_geometry(N, H, W, Cin, Cout, &mt, &nt, &tiles, &z);
-  return static_cast<int64_t>(z) * Cout * Cin;
+  return static_cast<int64_t>(wgrad_args(N, H, W, Cout, Cin, nullptr).splits) * Cout * Cin;
 }
 
 int b200unet_conv1x1_wgrad(const void* x, int x_cs, const void* dy, int dy_cs, float* partial, float* dw, int N, int H, int W,
@@ -848,17 +758,9 @@ int b200unet_conv1x1_wgrad(const void* x, int x_cs, const void* dy, int dy_cs, f
   B2_REQUIRE(Cin % 64 == 0 && Cout % 64 == 0 && Cout_real >= 1 && Cout_real <= Cout,
              "conv1x1_wgrad: Cin=%d and Cout=%d must be multiples of 64, Cout_real=%d in [1, Cout]", Cin, Cout, Cout_real);
   B2_REQUIRE(x_cs % 8 == 0 && dy_cs % 8 == 0 && x_cs >= Cin && dy_cs >= Cout, "conv1x1_wgrad: bad pitches");
-  WgradArgs a;
-  conv1x1_wgrad_geometry(N, H, W, Cin, Cout, &a.mtiles, &a.ntiles, &a.tiles_total, &a.splits);
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.Ca = Cout;
-  a.Cb = Cin;
-  a.partial = partial;
-  const uint64_t xs = static_cast<uint64_t>(x_cs) * 2, ys = static_cast<uint64_t>(dy_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA, dy, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  if (int e = b2h::make_tmap_4d(&a.tmB[0], x, Cin, W, H, N, xs, xs * W, xs * W * H, TW, TH)) return e;
-  for (int i = 1; i < 4; ++i) a.tmB[i] = a.tmB[0];
+  WgradArgs a = wgrad_args(N, H, W, Cout, Cin, partial);
+  if (int e = b2h::make_nhwc_map(&a.tmA, dy, Cout, dy_cs, N, H, W, TW, TH)) return e;
+  if (int e = b2h::make_nhwc_map(&a.tmB[0], x, Cin, x_cs, N, H, W, TW, TH)) return e;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (int e = launch_wgrad<KIND_PLAIN, 64>(a, st)) return e;
   const int total = Cout_real * Cin;
@@ -875,20 +777,10 @@ int b200unet_conv3x3_first_tc_wgrad(const float* x_nchw, const void* dy, int dy_
                                     int W, int Cin, int Cout, b200_stream_t stream) {
   B2_REQUIRE(Cin >= 1 && Cin <= 7 && Cout % 64 == 0 && Cout > 0, "conv3x3_first_tc_wgrad: Cin=%d must be in [1,7], Cout=%d a multiple of 64", Cin, Cout);
   B2_REQUIRE(x_nchw && dy && partial && dw_oihw && dy_cs % 8 == 0 && dy_cs >= Cout, "conv3x3_first_tc_wgrad: bad arguments");
-  WgradArgs a;
-  plain_wgrad_geometry(N, H, W, Cout, &a.mtiles, &a.tiles_total, &a.splits);
-  a.ntiles = 1;
-  a.tiles_w = b2h::ceil_div(W, TW);
-  a.tiles_h = b2h::ceil_div(H, TH);
-  a.Ca = Cout;
-  a.Cb = 64;
-  a.partial = partial;
+  WgradArgs a = wgrad_args(N, H, W, Cout, 64, partial);
   a.x_nchw = x_nchw;
-  a.H = H;
-  a.W = W;
-  const uint64_t ys = static_cast<uint64_t>(dy_cs) * 2;
-  if (int e = b2h::make_tmap_4d(&a.tmA, dy, Cout, W, H, N, ys, ys * W, ys * W * H, TW, TH)) return e;
-  for (int i = 0; i < 4; ++i) a.tmB[i] = a.tmA;  // unused (prefetch target only)
+  if (int e = b2h::make_nhwc_map(&a.tmA, dy, Cout, dy_cs, N, H, W, TW, TH)) return e;
+  a.tmB[0] = a.tmA;  // unused (prefetch target only)
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int e = 1;
   switch (Cin) {
