@@ -290,6 +290,21 @@ int64_t b200unet_channel_sum_workspace_floats(int C);
 int b200unet_channel_sum(const void* x, int x_cs, float* workspace, float* out, int64_t pixels, int C,
                          b200_stream_t stream);
 
+/* ---- nn.Dropout (Model.py:34-39 after the pooling of Down, :80-81 after the concat of Up) ------------------------- */
+/* In place over channels [c_lo, c_lo + nc) of a site tensor [N][H][W][C_site]; x points at channel c_lo of pixel 0, pixel
+ * pitch x_cs. For the site element e = ((n*H + h)*W + w)*C_site + c:
+ *   (r0..r3) = Philox4x32-10(counter = (lo32(e/4), hi32(e/4), site, 0), key = (lo32(*seed), hi32(*seed)))
+ *   x = r[e % 4] < threshold ? bf16(float(x) * scale) : 0
+ * threshold in [0, 2^32), scale: the caller's 1/(1-p). The mask depends on (seed, site, e) only, so forward and backward
+ * call this with the same arguments. seed: one int64 on the device (no host read: the launch may be captured in a graph).
+ * partial (nullable): per-block sums of the OUTPUT channels [sum_lo, sum_lo + sum_n) of the slice, [rows][sum_n] fp32 with
+ * rows = b200unet_dropout_partial_rows(N, H, W, nc); reduce with b200unet_partial_colsum(partial, rows, sum_n, 0, sum_n, out)
+ * (the ConvTranspose2d bias gradient of a dropped concat gradient). Requires nc and x_cs multiples of 8, x 16-byte aligned,
+ * and nc <= 2048 when partial != NULL. */
+int b200unet_dropout_partial_rows(int N, int H, int W, int nc);
+int b200unet_dropout_mul(void* x, int x_cs, int N, int H, int W, int C_site, int c_lo, int nc, int site, const int64_t* seed,
+                         int64_t threshold, float scale, float* partial, int sum_lo, int sum_n, b200_stream_t stream);
+
 /* ---- losses (loss.py:442-516) ----------------------------------------------------------------------------- */
 /* 'dice_bce_mc' (loss.py:488-500) and 'CE' (loss.py:468-469) forward. logits fp32 NCHW, target fp32 [N][H][W]
  * (class index stored as float, as the reference DataLoader produces). sums: fp64 scratch of

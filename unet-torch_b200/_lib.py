@@ -76,6 +76,8 @@ SIGNATURES = {
     "b200unet_nhwc_add": (c_int, [_P, _I, _P, _I, _P, _I, _L, _I, _P]),
     "b200unet_channel_sum_workspace_floats": (c_int64, [_I]),
     "b200unet_channel_sum": (c_int, [_P, _I, _P, _P, _L, _I, _P]),
+    "b200unet_dropout_partial_rows": (c_int, [_I, _I, _I, _I]),
+    "b200unet_dropout_mul": (c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _L, _F, _P, _I, _I, _P]),
     "b200unet_loss_sums_doubles": (c_int, []),
     "b200unet_loss_ce_dice_fwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P]),
     "b200unet_loss_ce_dice_bwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P]),

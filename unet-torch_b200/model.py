@@ -181,7 +181,8 @@ class _GateOp:
 
 
 class _Saved:
-    __slots__ = ("x", "enc", "dec", "head_in", "shapes", "dp")
+    # drop: (int64 device seed or None, drop probability per dropout site) of this forward; backward regenerates the masks
+    __slots__ = ("x", "enc", "dec", "head_in", "shapes", "dp", "drop")
 
 
 def _dc(mod) -> nn.Sequential:
@@ -211,6 +212,10 @@ class UNetEngine:
         # UNet_attention: one gate per decoder block (j = 0..3 <-> attenion4..attenion1), else None
         gates = net._attention_gates() if hasattr(net, "_attention_gates") else None
         self.gates = [_GateOp(a) for a in gates] if gates else None
+        # the nn.Dropout holder of each dropout site (0..3 = down1..4 after the pooling, 4..7 = up1..4 after the concat), or
+        # None; their `p` is read at every forward, as the reference's modules do
+        self.drop = ([next((m for m in d.maxpool_conv if isinstance(m, nn.Dropout)), None) for d in downs]
+                     + [u.dropout if getattr(u, "dropout_flag", False) else None for u in decoders[0][0]])
         self._graphs = {}     # (shape, device, training, save) -> _GraphedStep
         self._seen = set()    # keys that already ran once eagerly (kernel attributes configured, allocator warm)
         # B200UNET_WGRAD_STREAM=1: weight-gradient kernels on a second stream (nothing downstream in backward depends on
@@ -235,6 +240,16 @@ class UNetEngine:
         if self.trace is not None:
             self.trace.append((kind, kw))
 
+    def _drop_ps(self, training):
+        """Drop probability of each of the 8 dropout sites for this forward (0.0 = the site does nothing)."""
+        return tuple(float(m.p) if (training and m is not None) else 0.0 for m in self.drop)
+
+    def _dropout(self, t, site, seed, p, sums=None, backward=False):
+        before = t.clone() if self.trace is not None else None
+        ops.dropout_mul(t, site, seed, p, sums=sums)
+        if before is not None:
+            self._tr("dropout", site=site, p=p, seed=seed, before=before, after=t.clone(), backward=backward)
+
     def graphed_step(self, x, training, save):
         """The captured step for this input, or None when the call must run eagerly: graphs disabled, data parallel
         over a backend whose collectives cannot be captured, or first call for this shape (eager warm-up: kernel
@@ -247,7 +262,8 @@ class UNetEngine:
             return None
         if torch.cuda.is_current_stream_capturing():
             return None
-        key = (tuple(x.shape), x.device.index, bool(training), bool(save), dp is not None)
+        # the drop probabilities are launch arguments of the captured graph (and decide which passes it holds)
+        key = (tuple(x.shape), x.device.index, bool(training), bool(save), dp is not None, self._drop_ps(training))
         st = self._graphs.get(key)
         if st is None:
             if key not in self._seen:
@@ -480,6 +496,10 @@ class UNetEngine:
         cat = [torch.empty((n, hs[l], wsz[l], 2 * ch[l]), dtype=BF16, device=dev) for l in range(4)]
         saved = _Saved() if save else None
         enc_rec, dec_rec = [], []
+        # dropout: one seed per training forward, drawn on the device from torch's CUDA generator (a captured graph draws a
+        # new one at every replay); the masks are functions of (seed, site, element) and are regenerated in backward
+        drop_ps = self._drop_ps(training)
+        seed = torch.empty(1, dtype=torch.int64, device=dev).random_() if any(p > 0 for p in drop_ps) else None
 
         def conv_bn_relu(cb: _ConvBN, inp, c_out, hh, ww, a_out, pooled=None, pool_idx=None):
             if not training and not save and self.fold_eval_bn:
@@ -535,6 +555,8 @@ class UNetEngine:
                 pooled = torch.empty((n, hs[l + 1], wsz[l + 1], ch[l]), dtype=BF16, device=dev)
                 idx = torch.empty((n, hs[l + 1], wsz[l + 1], ch[l]), dtype=torch.uint8, device=dev) if save else None
                 r2 = conv_bn_relu(c2, a1, ch[l], hs[l], wsz[l], a2, pooled, idx)
+                if drop_ps[l] > 0:  # Down: MaxPool2d -> Dropout (the pool indices are those of the undropped maxima)
+                    self._dropout(pooled, l, seed, drop_ps[l])
                 inp = pooled
             else:
                 a2 = torch.empty((n, hs[l], wsz[l], ch[l]), dtype=BF16, device=dev)
@@ -561,6 +583,8 @@ class UNetEngine:
                 wf, _ = upo.operands()
                 ops.convt2x2(d_in, wf, upo.up.bias.detach(), catk[l][..., ch[l]:])
                 self._tr("convt", up=upo, x=d_in, out=catk[l][..., ch[l]:], cat=catk[l], skip=enc_rec[l][2])
+                if drop_ps[4 + j] > 0:  # Up: cat -> Dropout over both halves; nothing reads the skip half after this
+                    self._dropout(catk[l], 4 + j, seed, drop_ps[4 + j])
                 c1, c2 = dec[j]
                 a1 = torch.empty((n, hs[l], wsz[l], ch[l]), dtype=BF16, device=dev)
                 r1 = conv_bn_relu(c1, catk[l], ch[l], hs[l], wsz[l], a1)
@@ -587,6 +611,7 @@ class UNetEngine:
             saved.x, saved.enc, saved.dec, saved.head_in = x, enc_rec, dec_rec, heads_in
             saved.shapes = (n, ch, hs, wsz)
             saved.dp = dp
+            saved.drop = (seed, drop_ps)
         return out, saved
 
     # ------------------------------------------------------------------ backward
@@ -599,6 +624,7 @@ class UNetEngine:
         dlogits_all = [(torch.zeros((n, dc[2].weight.shape[0], hs[0], wsz[0]), dtype=torch.float32, device=dev)
                         if d is None else d.contiguous().float()) for d, dc in zip(dlogits_all, self.decoders)]
         dp = saved.dp
+        seed, drop_ps = saved.drop
         grads = {}
         flat = dp.make_flat_grads(self.params_in_backward_order()) if dp is not None else None
 
@@ -704,7 +730,11 @@ class UNetEngine:
                 g, pre = bn_conv_bwd(c2, r2, g, None, None, hs[l], wsz[l], True, fuse_next=r1)
                 upo = ups[j]
                 db, dwu = gbuf(upo.up.bias), gbuf(upo.up.weight)
-                dcat = bn_conv_bwd(c1, r1, g, None, None, hs[l], wsz[l], True, dx_colsum=(ch[l], db), pre=pre)
+                p_up = drop_ps[4 + j]
+                dcat = bn_conv_bwd(c1, r1, g, None, None, hs[l], wsz[l], True, dx_colsum=None if p_up > 0 else (ch[l], db),
+                                   pre=pre)
+                if p_up > 0:  # the concat's mask on both halves; the bias gradient sums the masked upsampled half
+                    self._dropout(dcat, 4 + j, seed, p_up, sums=(ch[l], db), backward=True)
                 dq_gate = None
                 # the side stream reads dcat's upsampled half (ConvTranspose2d weight gradient below). A plain single-decoder
                 # network keeps the storage referenced through skip_grads; behind a gate, or for a second decoder, nothing else
@@ -742,6 +772,8 @@ class UNetEngine:
             else:
                 g1, pre = bn_conv_bwd(c2, r2, skip_grads[l], g_pool, idx, hs[l], wsz[l], True, fuse_next=r1)
             g_pool = bn_conv_bwd(c1, r1, g1, None, None, hs[l], wsz[l], need_dx=(l > 0), pre=pre)
+            if l > 0 and drop_ps[l - 1] > 0:  # gradient w.r.t. the pooled tensor of level l - 1, through its mask
+                self._dropout(g_pool, l - 1, seed, drop_ps[l - 1], backward=True)
         if side is not None:
             torch.cuda.current_stream().wait_stream(side)  # join
         if flat is not None:
@@ -926,14 +958,15 @@ class UNet(nn.Module):
     def _fast_supported(self) -> bool:
         """Can the tensor-core engine run this architecture at all (input size is checked per call)?"""
         # widths: the BN / head kernels take power-of-two channel counts in [64, 2048] -> base width 64 or 128
-        return (self.initial_feature_map in (64, 128) and self.n_channels <= 7 and self.n_classes <= 8 and not self.dropout)
+        return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and self.n_classes <= 8
 
     def _get_engine(self) -> UNetEngine:
         """The tensor-core engine; raises if the architecture is outside its envelope."""
         if self._engine is None:
             if not self._fast_supported():
-                raise ValueError("tensor-core engine needs initial_feature_map in (64, 128), n_channels <= 7, "
-                                 "n_classes <= 8 and dropout=False; other variants run on the generic fp32 engine")
+                raise ValueError("tensor-core engine needs initial_feature_map in (64, 128), n_channels <= 7 and "
+                                 "n_classes <= 8 (UNet_attention: width 64 and dropout=False); other variants run on the "
+                                 "generic fp32 engine")
             object.__setattr__(self, "_engine", UNetEngine(self))
         return self._engine
 

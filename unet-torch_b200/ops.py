@@ -462,6 +462,40 @@ def nhwc_add(a, b, out=None):
     return out
 
 
+def dropout_threshold_scale(p):
+    """(threshold, scale) of the dropout mask for drop probability p, in double as DESIGN.md §4 fixes them: an element is kept
+    when its 32-bit Philox word is below threshold = min(2^32 - 1, floor((1 - p) 2^32)); kept elements are multiplied by
+    float(1 / (1 - p)). p = 1 keeps nothing and scales by 0 (no inf * 0)."""
+    p = float(p)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError(f"dropout probability has to be between 0 and 1, but got {p}")
+    if p == 1.0:
+        return 0, 0.0
+    return min(2 ** 32 - 1, int((1.0 - p) * 2.0 ** 32)), float(torch.tensor(1.0 / (1.0 - p), dtype=torch.float32))
+
+
+def dropout_mul(x, site, seed, p, c_site=None, c_lo=0, sums=None):
+    """nn.Dropout(p) in place on x (NHWC bf16, possibly a channel slice), mask of `site` (0..3 = down1..4, 4..7 = up1..4)
+    drawn from the int64 device tensor `seed`. x holds channels [c_lo, c_lo + C) of a site tensor with c_site channels
+    (default: x is the whole site tensor). sums = (lo, out): out[c] = sum over pixels of the dropped x[..., lo + c], for the
+    channels lo.. of x (fp32 [C - lo], fixed-order reduction)."""
+    xp, xcs, n, h, w, c = _nhwc(x)
+    if seed.dtype != torch.int64 or not seed.is_cuda or seed.numel() != 1:
+        raise ValueError("dropout_mul: seed must be one int64 on the device")
+    threshold, scale = dropout_threshold_scale(p)
+    part, lo, cnt, rows = None, 0, 0, 0
+    if sums is not None:
+        lo, out = sums
+        cnt = c - lo
+        rows = _lib.query("b200unet_dropout_partial_rows", n, h, w, c)
+        part = torch.empty(rows * cnt, dtype=torch.float32, device=x.device)
+    _lib.call("b200unet_dropout_mul", xp, xcs, n, h, w, c if c_site is None else c_site, c_lo, c, site, seed.data_ptr(),
+              threshold, scale, _ptr(part), lo, cnt, _stream())
+    if sums is not None:
+        partial_colsum(part, rows, cnt, 0, cnt, out)
+    return x
+
+
 def channel_sum(x, out):
     xp, xcs, n, h, w, c = _nhwc(x)
     ws = _workspace(_lib.query("b200unet_channel_sum_workspace_floats", c), x.device)
