@@ -211,6 +211,16 @@ int64_t b200unet_head_bwd_workspace_floats(int N, int H, int W, int Cin, int ncl
 int b200unet_head_bwd(const float* dz_nchw, const void* a, int a_cs, const float* w, void* da, int da_cs,
                       float* partial, float* dw, float* db, int N, int H, int W, int Cin, int ncls,
                       b200_stream_t stream);
+/* The same head for 1 <= ncls <= 256 (head_many.cu), Cin 64 or 128: classes in compile-time chunks of 8, so one kernel
+ * serves every count; at ncls <= 8 the logits are bit-identical to b200unet_head_fprop, which stays faster there.
+ * Backward: da bf16 NHWC, dw fp32 [ncls][Cin], db fp32 [ncls], reduced in a fixed order (fp64) from per-block partials in
+ * `partial` (b200unet_head_many_bwd_workspace_floats floats). */
+int b200unet_head_many_fprop(const void* a, int a_cs, const float* w, const float* bias, float* logits_nchw, int N,
+                             int H, int W, int Cin, int ncls, b200_stream_t stream);
+int64_t b200unet_head_many_bwd_workspace_floats(int N, int H, int W, int Cin, int ncls);
+int b200unet_head_many_bwd(const float* dz_nchw, const void* a, int a_cs, const float* w, void* da, int da_cs,
+                           float* partial, float* dw, float* db, int N, int H, int W, int Cin, int ncls,
+                           b200_stream_t stream);
 
 /* ---- BatchNorm2d + ReLU (+ MaxPool2d(2)) bandwidth kernels (Model.py:17-18,21-22,36,42) ------------------- */
 /* Reduce the per-tile partials of the conv epilogue into batch statistics and the affine (scale, shift):
@@ -306,12 +316,19 @@ int b200unet_dropout_mul(void* x, int x_cs, int N, int H, int W, int C_site, int
                          int64_t threshold, float scale, float* partial, int sum_lo, int sum_n, b200_stream_t stream);
 
 /* ---- losses (loss.py:442-516) ----------------------------------------------------------------------------- */
-/* 'dice_bce_mc' (loss.py:488-500) and 'CE' (loss.py:468-469) forward. logits fp32 NCHW, target fp32 [N][H][W]
+/* 'dice_bce_mc' (loss.py:488-500) and 'CE' (loss.py:468-469) forward, any ncls >= 1. logits fp32 NCHW, target fp32 [N][H][W]
  * (class index stored as float, as the reference DataLoader produces). sums: fp64 scratch of
  * b200unet_loss_sums_doubles() doubles ([sum CE, I_c, Z_c, Y_c], one scalar per 128-byte line), handed unchanged to
  * the backward. loss_out[0] = total loss, [1] = CE, [2] = Dice. mode: 0 = 0.5*CE+0.5*Dice, 1 = CE only.
  * err_flag: set to 1 if a target is outside [0, ncls) (the reference raises). */
 int b200unet_loss_sums_doubles(void);
+/* `sums` size for a class count: b200unet_loss_sums_doubles() up to 8 classes; past 8 the layout is [CE, I[ncls], Z[ncls],
+ * Y[ncls]], the backward's per-class Dice coefficients, then the forward's per-block rows (the per-class sums are reduced
+ * in a fixed order). */
+int64_t b200unet_loss_sums_doubles_n(int ncls);
+/* The leading doubles of `sums` that b200unet_loss_ce_dice_bwd reads: past 8 classes the rest is forward-only scratch, so a
+ * caller that keeps `sums` until the backward may keep just this prefix. */
+int64_t b200unet_loss_sums_saved_doubles_n(int ncls);
 int b200unet_loss_ce_dice_fwd(const float* logits, const float* target, double* sums, float* loss_out,
                               int* err_flag, int N, int ncls, int64_t HW, int mode, b200_stream_t stream);
 /* dlogits = grad_out[0] * dL/dlogits. */
@@ -324,7 +341,7 @@ int b200unet_mse_fwd(const float* pred, const float* target, double* sum, float*
 int b200unet_mse_bwd(const float* pred, const float* target, const float* grad_out, float* dpred, int64_t n,
                      int relu_input, b200_stream_t stream);
 
-/* ---- inference head (test_mc3serousv5.py:880-881): fp32 softmax over classes, then first-maximum argmax --- */
+/* ---- inference head (test_mc3serousv5.py:880-881): fp32 softmax over classes, then first-maximum argmax (any ncls) */
 int b200unet_softmax_argmax(const float* logits, int64_t* mask, int N, int ncls, int64_t HW, b200_stream_t stream);
 
 /* ---- the steps either side of the network (edge.cu; SURVEY.md 8f ranks 3 and 4) ------------------------------------ */
@@ -346,6 +363,12 @@ int b200unet_head_sigmoid_mask(const void* a, int a_cs, const float* w, const fl
  * reference; 1 = plain F.relu(model(x))) -> fp32 NCHW maps; counts (nullable): [N][ncls] fp64 sums of the stored maps. */
 int b200unet_head_density(const void* a, int a_cs, const float* w, const float* bias, float* out_nchw, double* counts,
                           int N, int H, int W, int Cin, int ncls, float divisor, b200_stream_t stream);
+/* b200unet_head_mask / b200unet_head_density for 1 <= ncls <= 256 and Cin 64 or 128 (head_many.cu): the mask equals
+ * b200unet_head_many_fprop followed by b200unet_softmax_argmax, the maps equal F.relu(logits) / divisor of its logits. */
+int b200unet_head_many_mask(const void* a, int a_cs, const float* w, const float* bias, uint8_t* mask, int N, int H, int W,
+                            int Cin, int ncls, b200_stream_t stream);
+int b200unet_head_many_density(const void* a, int a_cs, const float* w, const float* bias, float* out_nchw, double* counts,
+                               int N, int H, int W, int Cin, int ncls, float divisor, b200_stream_t stream);
 
 /* ---- SyncBN over NVLink peer memory (nvl_sync.cu; SURVEY.md 8e): one-shot all-reduce of a small fp64 vector through
  * symmetric buffers mapped into every rank (peer_bufs = HOST array of `world` device pointers, index = rank; each

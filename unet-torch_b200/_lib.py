@@ -56,6 +56,9 @@ SIGNATURES = {
     "b200unet_head_fprop": (c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "b200unet_head_bwd_workspace_floats": (c_int64, [_I, _I, _I, _I, _I]),
     "b200unet_head_bwd": (c_int, [_P, _P, _I, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "b200unet_head_many_fprop": (c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "b200unet_head_many_bwd_workspace_floats": (c_int64, [_I, _I, _I, _I, _I]),
+    "b200unet_head_many_bwd": (c_int, [_P, _P, _I, _P, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "b200unet_bn_reduce_partials": (c_int, [_P, _L, _I, _P, _P]),
     "b200unet_fold_rows": (c_int, [_P, _L, _I, _P, _I, _P]),
     "b200unet_bn_finalize": (c_int, [_P, _D, _P, _P, _F, _F, _P, _P, _P, _P, _P, _P, _I, _P]),
@@ -79,6 +82,8 @@ SIGNATURES = {
     "b200unet_dropout_partial_rows": (c_int, [_I, _I, _I, _I]),
     "b200unet_dropout_mul": (c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _P, _L, _F, _P, _I, _I, _P]),
     "b200unet_loss_sums_doubles": (c_int, []),
+    "b200unet_loss_sums_doubles_n": (c_int64, [_I]),
+    "b200unet_loss_sums_saved_doubles_n": (c_int64, [_I]),
     "b200unet_loss_ce_dice_fwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P]),
     "b200unet_loss_ce_dice_bwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _L, _I, _P]),
     "b200unet_mse_fwd": (c_int, [_P, _P, _P, _P, _L, _I, _P]),
@@ -111,6 +116,8 @@ SIGNATURES = {
     "b200unet_head_mask": (c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "b200unet_head_sigmoid_mask": (c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P]),
     "b200unet_head_density": (c_int, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P]),
+    "b200unet_head_many_mask": (c_int, [_P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "b200unet_head_many_density": (c_int, [_P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P]),
     "b200unet_nvl_buffer_bytes": (c_int64, []),
     "b200unet_nvl_allreduce_f64": (c_int, [_P, _P, _I, _P, _I, _I, _L, _P]),
     "b200unet_nvl_bn_sync_finalize": (c_int, [_P, _P, _P, _I, _I, _L, _D, _P, _P, _F, _F, _P, _P, _P, _P, _P, _P, _I, _P]),

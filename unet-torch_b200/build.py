@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libb200unet.so")
 OBJ_DIR = os.path.join(HERE, "build")
-SOURCES = ["api.cu", "igemm.cu", "conv3_res.cu", "conv3_pair.cu", "first_layer.cu", "wgrad.cu", "elementwise.cu", "small.cu", "loss.cu", "optim.cu", "generic_f32.cu", "nvl_sync.cu", "edge.cu", "gate.cu", "dropout.cu"]
+SOURCES = ["api.cu", "igemm.cu", "conv3_res.cu", "conv3_pair.cu", "first_layer.cu", "wgrad.cu", "elementwise.cu", "small.cu", "loss.cu", "optim.cu", "generic_f32.cu", "nvl_sync.cu", "edge.cu", "gate.cu", "dropout.cu", "head_many.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

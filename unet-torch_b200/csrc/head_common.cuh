@@ -106,4 +106,79 @@ __device__ __forceinline__ void logits_warp32(const __nv_bfloat16* __restrict__ 
   }
 }
 
+// ---- more than MAXC classes (head_many.cu). Each lane keeps its pixel's KC x 64 channels (packed bf16) in registers and
+// the classes are walked in compile-time chunks of CHUNK over zero-padded weight / bias rows in shared memory, so no FMA
+// carries a class predicate. Every logit is still bias, then fmaf over the channels in order: the same bits as
+// logits_warp32_n at the same class count.
+constexpr int CHUNK = 8;
+constexpr int MANY_MAXC = 256;
+
+__host__ __device__ inline int pad_classes(int ncls) { return (ncls + CHUNK - 1) / CHUNK * CHUNK; }
+// [pad_classes][Cin] weights, [pad_classes] bias, then one staging tile per warp
+__host__ __device__ inline int many_smem_bytes(int Cin, int ncls, int warps) {
+  return pad_classes(ncls) * (Cin + 1) * 4 + warps * STAGE_BYTES_PER_WARP;
+}
+__device__ __forceinline__ void load_weights_padded(float* wsm, float* bsm, const float* __restrict__ w,
+                                                    const float* __restrict__ bias, int Cin, int ncls) {
+  const int np = pad_classes(ncls);
+  for (int i = threadIdx.x; i < np * Cin; i += blockDim.x) wsm[i] = (i < ncls * Cin) ? w[i] : 0.f;
+  for (int j = threadIdx.x; j < np; j += blockDim.x) bsm[j] = (j < ncls) ? bias[j] : 0.f;
+}
+
+// Rows p0 + lane (rows >= P read as zero) -> row[] of this lane. The whole warp must call.
+template <int KC>
+__device__ __forceinline__ void load_rows_warp32(const __nv_bfloat16* __restrict__ a, int a_cs, uint32_t* stage,
+                                                 long long p0, long long P, uint4 (&row)[KC * 8]) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int kc = 0; kc < KC; ++kc) {
+    uint4 v[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int e = i * 32 + lane;
+      const long long p = p0 + (e >> 3);
+      v[i] = (p < P) ? __ldg(reinterpret_cast<const uint4*>(a + p * a_cs + kc * 64 + (e & 7) * 8)) : make_uint4(0, 0, 0, 0);
+    }
+    __syncwarp();
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int e = i * 32 + lane;
+      *reinterpret_cast<uint4*>(stage + (e >> 3) * ROW_WORDS + (e & 7) * 4) = v[i];
+    }
+    __syncwarp();
+#pragma unroll
+    for (int c8 = 0; c8 < 8; ++c8) row[kc * 8 + c8] = *reinterpret_cast<const uint4*>(stage + lane * ROW_WORDS + c8 * 4);
+  }
+  __syncwarp();
+}
+
+// z[j] = logit of class j0 + j of this lane's row, j < CHUNK (padded classes give 0)
+template <int KC>
+__device__ __forceinline__ void logits_chunk(const uint4 (&row)[KC * 8], const float* wsm, const float* bsm, int j0,
+                                             float (&z)[CHUNK]) {
+  constexpr int Cin = KC * 64;
+#pragma unroll
+  for (int j = 0; j < CHUNK; ++j) z[j] = bsm[j0 + j];
+#pragma unroll
+  for (int c8 = 0; c8 < KC * 8; ++c8) {
+    float f[8];
+    unpack8(row[c8], f);
+#pragma unroll
+    for (int j = 0; j < CHUNK; ++j) {
+      const float4 w0 = *reinterpret_cast<const float4*>(wsm + (j0 + j) * Cin + c8 * 8);
+      const float4 w1 = *reinterpret_cast<const float4*>(wsm + (j0 + j) * Cin + c8 * 8 + 4);
+      float t = z[j];
+      t = fmaf(f[0], w0.x, t);
+      t = fmaf(f[1], w0.y, t);
+      t = fmaf(f[2], w0.z, t);
+      t = fmaf(f[3], w0.w, t);
+      t = fmaf(f[4], w1.x, t);
+      t = fmaf(f[5], w1.y, t);
+      t = fmaf(f[6], w1.z, t);
+      t = fmaf(f[7], w1.w, t);
+      z[j] = t;
+    }
+  }
+}
+
 }  // namespace b2head

@@ -958,14 +958,14 @@ class UNet(nn.Module):
     def _fast_supported(self) -> bool:
         """Can the tensor-core engine run this architecture at all (input size is checked per call)?"""
         # widths: the BN / head kernels take power-of-two channel counts in [64, 2048] -> base width 64 or 128
-        return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and self.n_classes <= 8
+        return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and 1 <= self.n_classes <= ops.HEAD_MAX_CLASSES
 
     def _get_engine(self) -> UNetEngine:
         """The tensor-core engine; raises if the architecture is outside its envelope."""
         if self._engine is None:
             if not self._fast_supported():
                 raise ValueError("tensor-core engine needs initial_feature_map in (64, 128), n_channels <= 7 and "
-                                 "n_classes <= 8 (UNet_attention: width 64 and dropout=False); other variants run on the "
+                                 "n_classes <= 256 (UNet_attention: width 64 and dropout=False); other variants run on the "
                                  "generic fp32 engine")
             object.__setattr__(self, "_engine", UNetEngine(self))
         return self._engine
@@ -1066,12 +1066,12 @@ class UNet_multitask(UNet):
             ([getattr(self, f"up{i}_decod{d}") for i in (1, 2, 3, 4)], getattr(self, f"outc_decod{d}")) for d in (1, 2)]
 
     def _fast_supported(self) -> bool:
-        return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and self.n_classes <= 8
+        return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and 1 <= self.n_classes <= ops.HEAD_MAX_CLASSES
 
     def _engine_for(self, x):
         if x.dim() != 4 or x.shape[2] % 16 or x.shape[3] % 16 or not self._fast_supported():
             raise ValueError("UNet_multitask runs on the tensor-core engine only: H and W multiples of 16, "
-                             "initial_feature_map in (64, 128), n_channels <= 7, n_classes <= 8")
+                             "initial_feature_map in (64, 128), n_channels <= 7, n_classes <= 256")
         return self._get_engine()
 
     def set_check_mode(self, flag: bool = True):
@@ -1141,7 +1141,7 @@ class UNet_attention(UNet):
 
     def _fast_supported(self) -> bool:
         # the gate kernels take hidden widths 32..256 (csrc/gate.cu): base width 64
-        return self.initial_feature_map == 64 and self.n_channels <= 7 and self.n_classes <= 8 and not self.dropout
+        return self.initial_feature_map == 64 and self.n_channels <= 7 and 1 <= self.n_classes <= ops.HEAD_MAX_CLASSES and not self.dropout
 
     def _engine_for(self, x):
         if x.dim() == 4 and (x.shape[2] % 16 or x.shape[3] % 16):

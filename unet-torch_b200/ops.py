@@ -298,11 +298,20 @@ def conv3x3_first_wgrad(x_nchw, dy, dw_out):
     return dw_out
 
 
+# The OutConv kernels compiled per class count cover up to HEAD_FIXED_CLASSES classes; the head_many family takes
+# 1..HEAD_MAX_CLASSES (uint8 class masks) with the class count at run time.
+HEAD_FIXED_CLASSES, HEAD_MAX_CLASSES = 8, 256
+
+
+def _head(name, ncls):
+    return name.replace("head_", "head_many_", 1) if ncls > HEAD_FIXED_CLASSES else name
+
+
 def head_fprop(a, w, bias, logits_nchw):
     ap, acs, n, h, wd, cin = _nhwc(a)
     ncls = w.shape[0]
-    _lib.call("b200unet_head_fprop", ap, acs, _f32(w.view(ncls, cin)), _f32(bias), _f32(logits_nchw), n, h, wd, cin,
-              ncls, _stream())
+    _lib.call(_head("b200unet_head_fprop", ncls), ap, acs, _f32(w.view(ncls, cin)), _f32(bias), _f32(logits_nchw), n, h,
+              wd, cin, ncls, _stream())
     return logits_nchw
 
 
@@ -310,9 +319,9 @@ def head_bwd(dz_nchw, a, w, da, dw, db):
     ap, acs, n, h, wd, cin = _nhwc(a)
     dp, dcs, *_ = _nhwc(da)
     ncls = w.shape[0]
-    ws = _workspace(_lib.query("b200unet_head_bwd_workspace_floats", n, h, wd, cin, ncls), a.device)
-    _lib.call("b200unet_head_bwd", _f32(dz_nchw), ap, acs, _f32(w.view(ncls, cin)), dp, dcs, ws.data_ptr(), _f32(dw),
-              _f32(db), n, h, wd, cin, ncls, _stream())
+    ws = _workspace(_lib.query(_head("b200unet_head_bwd_workspace_floats", ncls), n, h, wd, cin, ncls), a.device)
+    _lib.call(_head("b200unet_head_bwd", ncls), _f32(dz_nchw), ap, acs, _f32(w.view(ncls, cin)), dp, dcs, ws.data_ptr(),
+              _f32(dw), _f32(db), n, h, wd, cin, ncls, _stream())
 
 
 # --------------------------------------------------------------------------------------------- BN / ReLU / pool
@@ -644,11 +653,14 @@ def gate_bwd_apply(q1, x1, aff_q, aff_x, gamma_q, gamma_x, w_psi, ds, sums, sums
 # --------------------------------------------------------------------------------------------- losses / inference
 def loss_ce_dice_fwd(logits, target, mode):
     n, ncls, h, w = logits.shape
-    sums = torch.empty((_lib.query("b200unet_loss_sums_doubles"),), dtype=torch.float64, device=logits.device)
+    sums = torch.empty((_lib.query("b200unet_loss_sums_doubles_n", ncls),), dtype=torch.float64, device=logits.device)
     out = torch.empty((3,), dtype=torch.float32, device=logits.device)
     err = torch.empty((1,), dtype=torch.int32, device=logits.device)
     _lib.call("b200unet_loss_ce_dice_fwd", _f32(logits), _f32(target), sums.data_ptr(), out.data_ptr(), err.data_ptr(),
               n, ncls, h * w, mode, _stream())
+    keep = _lib.query("b200unet_loss_sums_saved_doubles_n", ncls)
+    if keep < sums.numel():  # past 8 classes the rest is forward-only scratch: do not keep it alive until the backward
+        sums = sums[:keep].clone()
     return out, sums, err
 
 
@@ -705,14 +717,16 @@ def head_mask(a, w, bias):
     ap, acs, n, h, wd, cin = _nhwc(a)
     ncls = w.shape[0]
     mask = torch.empty((n, h, wd), dtype=torch.uint8, device=a.device)
-    _lib.call("b200unet_head_mask", ap, acs, _f32(w.view(ncls, cin)), _f32(bias), mask.data_ptr(), n, h, wd, cin, ncls,
-              _stream())
+    _lib.call(_head("b200unet_head_mask", ncls), ap, acs, _f32(w.view(ncls, cin)), _f32(bias), mask.data_ptr(), n, h, wd,
+              cin, ncls, _stream())
     return mask
 
 
 def head_sigmoid_mask(a, w, bias, threshold=0.5):
     """OutConv channel 0 + sigmoid + `>= threshold` -> {0,1} uint8 [N,H,W] (test.py:393-399); a: NHWC bf16."""
     ap, acs, n, h, wd, cin = _nhwc(a)
+    if w.shape[0] > HEAD_FIXED_CLASSES:  # only channel 0 is thresholded: its row and bias make a 1-class head
+        w, bias = w[:1], bias[:1]
     ncls = w.shape[0]
     mask = torch.empty((n, h, wd), dtype=torch.uint8, device=a.device)
     _lib.call("b200unet_head_sigmoid_mask", ap, acs, _f32(w.view(ncls, cin)), _f32(bias), mask.data_ptr(), n, h, wd, cin,
@@ -726,6 +740,6 @@ def head_density(a, w, bias, divisor=200.0, with_counts=True):
     ncls = w.shape[0]
     out = torch.empty((n, ncls, h, wd), dtype=torch.float32, device=a.device)
     counts = torch.empty((n, ncls), dtype=torch.float64, device=a.device) if with_counts else None
-    _lib.call("b200unet_head_density", ap, acs, _f32(w.view(ncls, cin)), _f32(bias), _f32(out),
+    _lib.call(_head("b200unet_head_density", ncls), ap, acs, _f32(w.view(ncls, cin)), _f32(bias), _f32(out),
               counts.data_ptr() if counts is not None else None, n, h, wd, cin, ncls, float(divisor), _stream())
     return out, counts
