@@ -243,7 +243,8 @@ int b200unet_bn_reduce_finalize(const float* stats_partial, int64_t rows, int C,
                                 const float* beta, float eps, float momentum, float* running_mean, float* running_var,
                                 int64_t* num_batches_tracked, float* mean, float* rstd, float* scale, float* shift,
                                 b200_stream_t stream);
-/* eval mode: scale/shift from running statistics. */
+/* eval mode: scale/shift from running statistics; running_mean / running_var must not be NULL (a BatchNorm without running
+ * statistics has no eval-mode affine). */
 int b200unet_bn_eval_affine(const float* gamma, const float* beta, const float* running_mean,
                             const float* running_var, float eps, float* scale, float* shift, int C,
                             b200_stream_t stream);

@@ -79,6 +79,24 @@ def test_bad_shapes_are_errors_not_fallbacks(lib):
         lib.call("b200unet_sgemm_strided", 1, 1, 1, None, 0, 4, 4, 1, 1, 1, 1, 1, 1, 1, 0, 0, 0, 0, None)
 
 
+def test_bn_statistics_entry_points_validate_before_launch(lib):
+    # a BatchNorm built with track_running_stats=False has no running buffers: eval mode has no affine to compute
+    with pytest.raises(RuntimeError, match="null running statistics"):
+        lib.call("b200unet_bn_eval_affine", 1, 1, None, None, 1e-5, 1, 1, 64, None)
+    with pytest.raises(RuntimeError, match="null running statistics"):
+        lib.call("b200unet_bn_eval_affine", 1, 1, 1, None, 1e-5, 1, 1, 64, None)
+    with pytest.raises(RuntimeError, match="null argument"):
+        lib.call("b200unet_bn_eval_stats", None, None, 1e-5, 1, 1, 64, None)
+    # fold_rows: the column width of a block is a power of two <= 256 or a multiple of 256
+    for ncols in (192, 384):
+        with pytest.raises(RuntimeError, match=f"ncols={ncols}"):
+            lib.call("b200unet_fold_rows", 1, 5000, ncols, 1, 296, None)
+    with pytest.raises(RuntimeError, match="bad arguments"):
+        lib.call("b200unet_fold_rows", 1, 100, 64, 1, 296, None)    # more output rows than input rows
+    with pytest.raises(RuntimeError, match="bad column range"):
+        lib.call("b200unet_partial_colsum", 1, 8, 64, 40, 25, 1, None)
+
+
 def test_header_is_plain_c_and_a_c_host_links_the_library(lib, tmp_path):
     """The boundary is a C ABI: include/b200unet.h must compile as C99 (no C++ in the signatures), and a C host program
     must link libb200unet.so and reach the host-only entry points (what a cgo / JNI / FFI binding does)."""

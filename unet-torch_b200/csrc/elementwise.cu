@@ -642,6 +642,8 @@ int b200unet_bn_reduce_finalize(const float* stats_partial, int64_t rows, int C,
 
 int b200unet_bn_eval_affine(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
                             float eps, float* scale, float* shift, int C, b200_stream_t stream) {
+  B2_REQUIRE(running_mean && running_var, "bn_eval_affine: null running statistics (BatchNorm2d(track_running_stats=False))");
+  B2_REQUIRE(gamma && beta && scale && shift && C > 0, "bn_eval_affine: null argument");
   bn_eval_affine_kernel<<<(C + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(gamma, beta, running_mean,
                                                                                       running_var, eps, scale, shift, C);
   return b2h::check_launch("bn_eval_affine");

@@ -20,6 +20,10 @@ import torch
 import torch.distributed as dist
 
 
+def _ptr(t):
+    return None if t is None else t.data_ptr()
+
+
 class FlatGrads:
     def __init__(self, ctx: "DataParallelContext", params, flat=None):
         self.ctx = ctx
@@ -180,28 +184,28 @@ class DataParallelContext:
 
     nvl_max_doubles = 2048  # slot size of the symmetric buffer (csrc/nvl_sync.cu SLOT_DOUBLES); longer vectors go through NCCL
 
-    def bn_sync_finalize(self, sums, global_count, bn, eps, momentum, track, mean, rstd, scale, shift):
-        """All-reduce the fp64 [sum, sum^2] vector over NVLink and finalise BatchNorm in the same kernel."""
+    def bn_sync_finalize(self, sums, global_count, bn, eps, momentum, running_mean, running_var, mean, rstd, scale, shift):
+        """All-reduce the fp64 [sum, sum^2] vector over NVLink and finalise BatchNorm in the same kernel (running buffers may
+        be None: see ops.bn_train_buffers)."""
         from . import _lib
 
         c = bn.num_features
         # seq = 0: device-side reduction counter, so the launch can be captured in a CUDA graph and replayed
         _lib.call("b200unet_nvl_bn_sync_finalize", sums.data_ptr(), sums.data_ptr(), self._nvl[2], self.world_size,
                   self.rank, 0, float(global_count), bn.weight.data_ptr(), bn.bias.data_ptr(), float(eps),
-                  float(momentum), bn.running_mean.data_ptr() if track else None,
-                  bn.running_var.data_ptr() if track else None, mean.data_ptr(), rstd.data_ptr(), scale.data_ptr(),
+                  float(momentum), _ptr(running_mean), _ptr(running_var), mean.data_ptr(), rstd.data_ptr(), scale.data_ptr(),
                   shift.data_ptr(), c, torch.cuda.current_stream().cuda_stream)
 
-    def bn_rows_sync_finalize(self, stats_partial, rows, global_count, bn, eps, momentum, track, mean, rstd, scale, shift):
+    def bn_rows_sync_finalize(self, stats_partial, rows, global_count, bn, eps, momentum, running_mean, running_var,
+                              num_batches_tracked, mean, rstd, scale, shift):
         """Forward SyncBN in ONE kernel: reduce this rank's partial statistics rows, exchange them over NVLink, finalise
-        BatchNorm (running statistics and num_batches_tracked included)."""
+        BatchNorm (running statistics and num_batches_tracked included; None: not updated)."""
         from . import _lib
 
         _lib.call("b200unet_nvl_bn_rows_sync_finalize", stats_partial.data_ptr(), int(rows), bn.num_features, self._nvl[2],
                   self.world_size, self.rank, float(global_count), bn.weight.data_ptr(), bn.bias.data_ptr(), float(eps),
-                  float(momentum), bn.running_mean.data_ptr() if track else None, bn.running_var.data_ptr() if track else None,
-                  bn.num_batches_tracked.data_ptr() if track else None, mean.data_ptr(), rstd.data_ptr(), scale.data_ptr(),
-                  shift.data_ptr(), torch.cuda.current_stream().cuda_stream)
+                  float(momentum), _ptr(running_mean), _ptr(running_var), _ptr(num_batches_tracked), mean.data_ptr(),
+                  rstd.data_ptr(), scale.data_ptr(), shift.data_ptr(), torch.cuda.current_stream().cuda_stream)
 
     def rows_allreduce(self, partial, rows, c, sums_local, sums_global):
         """Backward SyncBN: block partials [rows][2][c] -> local and all-rank fp64 sums [2c], one kernel over NVLink."""

@@ -96,6 +96,8 @@ class GenericEngine:
         mean = rstd = None
         count = n * h * w
         if not training:
+            if bn.running_mean is None:
+                raise RuntimeError("eval-mode BatchNorm2d without running statistics (track_running_stats=False) is not supported")
             ops.bn_eval_affine(bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.eps, scale, shift)
             if save:
                 mean = torch.empty(k, dtype=torch.float32, device=dev)
@@ -109,12 +111,11 @@ class GenericEngine:
                 count = count * dp.world_size
             mean = torch.empty(k, dtype=torch.float32, device=dev)
             rstd = torch.empty(k, dtype=torch.float32, device=dev)
-            mom = bn.momentum if bn.momentum is not None else 0.1
-            track = bn.track_running_stats and bn.running_mean is not None
-            ops.bn_finalize(sums, count, bn.weight, bn.bias, bn.eps, mom, bn.running_mean if track else None,
-                            bn.running_var if track else None, mean, rstd, scale, shift)
-            if track:
+            mom, rm, rv, nbt = ops.bn_train_buffers(bn)
+            ops.bn_finalize(sums, count, bn.weight, bn.bias, bn.eps, mom, rm, rv, mean, rstd, scale, shift)
+            if nbt is not None:
                 bn.num_batches_tracked += 1
+            ops.bn_cumulative_update(bn, rm, rv)
         return scale, shift, mean, rstd, count, not training
 
     def _conv1x1_bn(self, seq, inp, act, training, dp, save):

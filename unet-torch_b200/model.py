@@ -321,31 +321,25 @@ class UNetEngine:
         mean = torch.empty(c, dtype=torch.float32, device=dev)
         rstd = torch.empty(c, dtype=torch.float32, device=dev)
         stats_partial, rows = ops.fold_rows(stats_partial, rows, 2 * c)
-        mom = bn.momentum if bn.momentum is not None else 0.1
-        track = bn.track_running_stats and bn.running_mean is not None
+        mom, rm, rv, nbt = ops.bn_train_buffers(bn)
         if dp is None or not dp.sync_bn:  # single GPU: partial rows -> statistics -> affine -> running buffers, one launch
-            ops.bn_reduce_finalize(stats_partial, rows, count, bn.weight, bn.bias, bn.eps, mom,
-                                   bn.running_mean if track else None, bn.running_var if track else None,
-                                   bn.num_batches_tracked if track else None, mean, rstd, scale, shift)
-            return scale, shift, mean, rstd, count
-        if dp.supports_rows(c):  # SyncBN over NVLink: rows -> exchange -> finalise in one multi-block kernel
+            ops.bn_reduce_finalize(stats_partial, rows, count, bn.weight, bn.bias, bn.eps, mom, rm, rv, nbt, mean, rstd, scale,
+                                   shift)
+        elif dp.supports_rows(c):  # SyncBN over NVLink: rows -> exchange -> finalise in one multi-block kernel
             count = count * dp.world_size
-            dp.bn_rows_sync_finalize(stats_partial, rows, count, bn, bn.eps, mom, track, mean, rstd, scale, shift)
-            return scale, shift, mean, rstd, count
-        sums = torch.empty(2 * c, dtype=torch.float64, device=dev)
-        ops.bn_reduce_partials(stats_partial, rows, c, sums)
-        if dp is not None and dp.sync_bn:
+            dp.bn_rows_sync_finalize(stats_partial, rows, count, bn, bn.eps, mom, rm, rv, nbt, mean, rstd, scale, shift)
+        else:
+            sums = torch.empty(2 * c, dtype=torch.float64, device=dev)
+            ops.bn_reduce_partials(stats_partial, rows, c, sums)
             count = count * dp.world_size
             if dp.has_nvl and 2 * c <= dp.nvl_max_doubles:  # one kernel: NVLink one-shot all-reduce of [sum, sum^2] + finalisation
-                dp.bn_sync_finalize(sums, count, bn, bn.eps, mom, track, mean, rstd, scale, shift)
-                if track:
-                    bn.num_batches_tracked += 1
-                return scale, shift, mean, rstd, count
-            dp.all_reduce_sum(sums)
-        ops.bn_finalize(sums, count, bn.weight, bn.bias, bn.eps, mom, bn.running_mean if track else None,
-                        bn.running_var if track else None, mean, rstd, scale, shift)
-        if track:
-            bn.num_batches_tracked += 1
+                dp.bn_sync_finalize(sums, count, bn, bn.eps, mom, rm, rv, mean, rstd, scale, shift)
+            else:
+                dp.all_reduce_sum(sums)
+                ops.bn_finalize(sums, count, bn.weight, bn.bias, bn.eps, mom, rm, rv, mean, rstd, scale, shift)
+            if nbt is not None:
+                bn.num_batches_tracked += 1
+        ops.bn_cumulative_update(bn, rm, rv)
         return scale, shift, mean, rstd, count
 
     # ------------------------------------------------------------------ attention gates

@@ -356,13 +356,37 @@ def fold_rows(stats_partial, rows, ncols):
     return out, FOLD_ROWS_TO
 
 
+def bn_train_buffers(bn):
+    """(momentum, running_mean, running_var, num_batches_tracked) for the training finalisation of `bn`; the three buffers are
+    None when it tracks no running statistics. momentum=None (torch: cumulative average with factor 1/num_batches_tracked)
+    finalises with momentum 1.0 into scratch buffers, which bn_cumulative_update then folds into the running ones."""
+    if not bn.track_running_stats or bn.running_mean is None:
+        return 0.0, None, None, None
+    if bn.momentum is None:  # zeroed: the kernels compute (1 - 1) * buffer, and 0 * NaN of uninitialised memory is NaN
+        return 1.0, torch.zeros_like(bn.running_mean), torch.zeros_like(bn.running_var), bn.num_batches_tracked
+    return bn.momentum, bn.running_mean, bn.running_var, bn.num_batches_tracked
+
+
+def bn_cumulative_update(bn, batch_mean, batch_var):
+    """momentum=None, after the finalisation has incremented num_batches_tracked: running += (batch - running) / count. The
+    factor is read from the counter on the device, so a captured CUDA graph applies the count of each replay."""
+    if bn.momentum is None and batch_mean is not None:
+        w = bn.num_batches_tracked.reciprocal()  # fp32; lerp with weight 1 returns the batch value exactly
+        bn.running_mean.lerp_(batch_mean, w)
+        bn.running_var.lerp_(batch_var, w)
+
+
 def bn_eval_affine(gamma, beta, running_mean, running_var, eps, scale, shift):
+    if running_mean is None or running_var is None:
+        raise RuntimeError("bn_eval_affine: no running statistics (BatchNorm2d(track_running_stats=False))")
     _lib.call("b200unet_bn_eval_affine", _f32(gamma), _f32(beta), _f32(running_mean), _f32(running_var), eps,
               _f32(scale), _f32(shift), gamma.numel(), _stream())
 
 
 def bn_eval_stats(running_mean, running_var, eps, mean, rstd):
     """mean = running_mean, rstd = rsqrt(running_var + eps): what the backward kernels need after an eval-mode forward."""
+    if running_mean is None or running_var is None:
+        raise RuntimeError("bn_eval_stats: no running statistics (BatchNorm2d(track_running_stats=False))")
     _lib.call("b200unet_bn_eval_stats", _f32(running_mean), _f32(running_var), eps, _f32(mean), _f32(rstd), mean.numel(),
               _stream())
 
