@@ -97,6 +97,31 @@ def test_bn_statistics_entry_points_validate_before_launch(lib):
         lib.call("b200unet_partial_colsum", 1, 8, 64, 40, 25, 1, None)
 
 
+def test_bn_relu_backward_passes_validate_the_pool_arguments_before_launch(lib):
+    """Both BatchNorm+ReLU backward passes refuse a call without a gradient source, and a pooled gradient without window
+    positions or with an odd H or W: the kernels read pool_idx and the 2x2 windows of y unchecked."""
+    launches = lib.query("b200unet_launch_count")
+
+    def reduce_rows(g1, g_pool, pool_idx, h, w, c=64):
+        lib.call("b200unet_bn_relu_bwd_reduce_rows", g1, c, g_pool, pool_idx, 1, c, 1, 1, 1, 1, 1, 1, 2, h, w, c, None)
+
+    def apply(g1, g_pool, pool_idx, h, w, c=64):
+        lib.call("b200unet_bn_relu_bwd_apply", g1, c, g_pool, pool_idx, 1, c, 1, 1, 1, 1, 1, 1, 8.0, None, 1, c, 1, 1, 2, h, w,
+                 c, None)
+
+    for fn, name in ((reduce_rows, "bn_relu_bwd_reduce"), (apply, "bn_relu_bwd_apply")):
+        with pytest.raises(RuntimeError, match=f"{name}: C=96 must be a power of two"):
+            fn(1, None, None, 4, 4, c=96)
+        with pytest.raises(RuntimeError, match=f"{name}: no gradient source"):
+            fn(None, None, None, 4, 4)
+        with pytest.raises(RuntimeError, match=rf"{name}\(pool\): bad arguments"):
+            fn(1, 1, None, 4, 4)            # pooled gradient without window positions
+        for h, w in ((3, 4), (4, 5)):
+            with pytest.raises(RuntimeError, match=rf"{name}\(pool\): bad arguments"):
+                fn(1, 1, 1, h, w)
+    assert lib.query("b200unet_launch_count") == launches
+
+
 def test_header_is_plain_c_and_a_c_host_links_the_library(lib, tmp_path):
     """The boundary is a C ABI: include/b200unet.h must compile as C99 (no C++ in the signatures), and a C host program
     must link libb200unet.so and reach the host-only entry points (what a cgo / JNI / FFI binding does)."""

@@ -1,4 +1,5 @@
-"""-m gpu: bandwidth kernels (BN / ReLU / pool / loss / head / first conv) against the oracle on the same inputs."""
+"""-m gpu: bandwidth kernels (BN statistics / pool / loss / head / first conv) against the oracle on the same inputs. The
+BatchNorm+ReLU forward and backward kernels are checked exactly in tests/test_gpu_bn_relu_exact.py."""
 import pytest
 import torch
 
@@ -45,77 +46,6 @@ def test_bn_stats_finalize_and_apply(ops, c, n, h, w):
     a = torch.empty_like(yd)
     ops.bn_relu_fwd(yd, scale, shift, a)
     assert rel_l2(from_nhwc(a), O.relu(want)) < 4e-3  # bf16 output rounding
-
-
-@pytest.mark.parametrize("c,n,h,w", [(64, 2, 16, 32), (128, 1, 8, 8)])
-def test_bn_relu_pool_indices_bit_exact(ops, c, n, h, w):
-    y, gamma, beta = _bn_setup(c, n, h, w, 2)
-    y[0, 0, 0:2, 0:2] = 0.75  # a tie inside one window
-    yd = to_nhwc_bf16(y)
-    scale = (gamma * 0.8).cuda()
-    shift = beta.cuda()
-    # write `a` into the left half of a wider (concat-style) buffer
-    cat = torch.zeros(n, h, w, 2 * c, dtype=BF16, device="cuda")
-    pooled = torch.empty(n, h // 2, w // 2, c, dtype=BF16, device="cuda")
-    idx = torch.empty(n, h // 2, w // 2, c, dtype=torch.uint8, device="cuda")
-    ops.bn_relu_fwd(yd, scale, shift, cat[..., :c], pooled, idx)
-    a = from_nhwc(cat[..., :c])
-    assert float(cat[..., c:].float().abs().max()) == 0.0
-    # identical input (the stored bf16 activation) through the oracle's pooling: bit-exact values and positions
-    pv, pos, flat = O.maxpool2x2(a)
-    assert torch.equal(from_nhwc(pooled), pv)
-    assert torch.equal(idx.permute(0, 3, 1, 2).cpu().long(), pos)
-    # and the activation itself
-    want = O.relu(y * scale.cpu()[None, :, None, None] + shift.cpu()[None, :, None, None])
-    assert rel_l2(a, want) < 4e-3
-
-
-@pytest.mark.parametrize("pool", [False, True])
-def test_bn_relu_backward(ops, pool):
-    c, n, h, w = 64, 2, 8, 16
-    y, gamma, beta = _bn_setup(c, n, h, w, 3)
-    g = torch.Generator().manual_seed(33)
-    yv = y.clone().requires_grad_(True)
-    gam = gamma.clone().requires_grad_(True)
-    bet = beta.clone().requires_grad_(True)
-    out, _, _ = O.batchnorm_train(yv, gam, bet)
-    a = O.relu(out)
-    # device-side statistics and (for the pooled case) the forward kernel on the same data
-    yd = to_nhwc_bf16(y)
-    mu = y.mean((0, 2, 3))
-    var = y.var((0, 2, 3), unbiased=False)
-    rstd = torch.rsqrt(var + 1e-5)
-    scale = (gamma * rstd).cuda()
-    shift = (beta - mu * gamma * rstd).cuda()
-    gpd = idx = None
-    if pool:
-        tmp_a = torch.empty_like(yd)
-        pooled = torch.empty(n, h // 2, w // 2, c, dtype=BF16, device="cuda")
-        idx = torch.empty(n, h // 2, w // 2, c, dtype=torch.uint8, device="cuda")
-        ops.bn_relu_fwd(yd, scale, shift, tmp_a, pooled, idx)
-        # the device pools the bf16 activation it stored: hand the oracle the IDENTICAL pooling input (straight-through
-        # for the rounding), so that near-ties pick the same window position on both sides
-        a_dev = from_nhwc(tmp_a)
-        assert rel_l2(a_dev, a.detach()) < 4e-3
-        a = a + (a_dev - a.detach())
-    else:
-        a = a + (bf16_round(a.detach()) - a.detach())
-    g1 = bf16_round(torch.randn(n, c, h, w, generator=g))
-    loss = (a * g1).sum()
-    gp = None
-    if pool:
-        pv, pos, flat = O.maxpool2x2(a)
-        assert torch.equal(idx.permute(0, 3, 1, 2).cpu().long(), pos)
-        gp = bf16_round(torch.randn(pv.shape, generator=g))
-        loss = loss + (pv * gp).sum()
-        gpd = to_nhwc_bf16(gp)
-    loss.backward()
-    dy = torch.empty_like(yd)
-    dgamma, dbeta = torch.empty(c, device="cuda"), torch.empty(c, device="cuda")
-    ops.bn_relu_bwd(to_nhwc_bf16(g1), gpd, idx, yd, gamma.cuda(), scale, shift, mu.cuda(), rstd.cuda(), dy, dgamma, dbeta)
-    assert rel_l2(from_nhwc(dy), yv.grad) < 1e-2
-    assert rel_l2(dgamma, gam.grad) < 2e-3
-    assert rel_l2(dbeta, bet.grad) < 2e-3
 
 
 def test_channel_sum(ops):

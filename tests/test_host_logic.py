@@ -426,3 +426,170 @@ def test_bench_dump_outputs_samples_each_array_by_its_own_size_within_budget(tmp
     monkeypatch.setattr(bench, "DUMP_BYTES", 30_000)
     with pytest.raises(RuntimeError, match="dump-outputs"):
         bench.dump_outputs(str(tmp_path / "d"), arrays)
+
+
+def _f32_of_fraction(q):
+    """Round an exact rational to fp32, nearest-even (subnormals included), as a Python float."""
+    import math
+    from fractions import Fraction
+
+    if q == 0:
+        return 0.0
+    sign, q = (-1 if q < 0 else 1), abs(q)
+    e = q.numerator.bit_length() - q.denominator.bit_length()
+    while Fraction(2) ** e > q:
+        e -= 1
+    while Fraction(2) ** (e + 1) <= q:
+        e += 1
+    ulp = Fraction(2) ** (max(e, -126) - 23)
+    m = q / ulp
+    fl = math.floor(m)
+    if m - fl > Fraction(1, 2) or (m - fl == Fraction(1, 2) and fl % 2 == 1):
+        fl += 1
+    return sign * float(fl * ulp)
+
+
+def test_ew_check_fmaf_is_exact():
+    """tests/ew_check.py: the fp64 emulation of fmaf equals exact rational arithmetic rounded once to fp32, on random fp32 x bf16
+    and fp32 x fp32 operands and on the constructed fp32-midpoint cases, which must all take the double-rounding branch. There,
+    rounding the fp64 sum to fp32 directly is wrong in one direction of the error term, and the forward's bf16 output tells
+    the two results apart."""
+    from fractions import Fraction
+
+    import ew_check as E
+
+    assert all(a * b == 2 ** 30 + rho and a < 2 ** 24 and b % 2 == 1 and b < 256 for a, b, rho in E.MIDPOINT_PRODUCTS)
+    g = torch.Generator().manual_seed(11)
+    n = 1500
+    sc = (torch.randn(n, generator=g, dtype=torch.float64) * torch.exp2(torch.randint(-30, 30, (n,), generator=g))).float()
+    y = (torch.randn(n, generator=g, dtype=torch.float64) * torch.exp2(torch.randint(-30, 30, (n,), generator=g))).bfloat16()
+    sh = (torch.randn(n, generator=g, dtype=torch.float64) * torch.exp2(torch.randint(-30, 30, (n,), generator=g))).float()
+    fb = torch.randn(n, generator=g).float()
+    cases = [(sc, y.float()), (sc, fb)]
+    mids = [E.midpoint_case(i, hb, j) for i in range(8) for hb in (0, 5, 63) for j in (-3, 0, 3)]
+    msc, my, msh = (torch.tensor(v, dtype=torch.float32) for v in zip(*mids))
+    assert torch.equal(my.bfloat16().float(), my)
+    for a, b in cases + [(msc, my)]:
+        c = sh[: a.numel()] if a.numel() == n else msh
+        got, mid = E.fmaf(a, b, c)
+        want = [_f32_of_fraction(Fraction(float(x)) * Fraction(float(z)) + Fraction(float(w))) for x, z, w in zip(a, b, c)]
+        assert got.tolist() == want
+    got, mid = E.fmaf(msc, my, msh)
+    assert bool(mid.all()), "a constructed midpoint case missed the double-rounding branch"
+    naive = (msc.double() * my.double() + msh.double()).float().double()
+    rho = torch.tensor([E.MIDPOINT_PRODUCTS[i][2] for i in range(8) for _ in range(9)])
+    assert bool((naive != got).all()), "rounding the fp64 sum to fp32 directly must get every constructed case wrong"
+    assert bool((naive.float().bfloat16() != got.float().bfloat16()).all()), "the branch must be visible in bf16"
+
+
+def test_ew_check_references_agree_with_autograd():
+    """tests/ew_check.py: the backward formulas (dgamma, dbeta and the k1..k3 form of dy) equal autograd through BatchNorm with
+    batch statistics + ReLU (+ MaxPool2d) in fp64; the pooling reference equals max_pool2d's indices; unpool equals autograd's
+    gradient through the pool."""
+    import torch.nn.functional as F
+
+    import ew_check as E
+
+    g = torch.Generator().manual_seed(12)
+    n, c, h, w = 2, 5, 6, 8
+    y = torch.randn(n, h, w, c, generator=g, dtype=torch.float64) * 2 + 0.5
+    gamma, beta = torch.randn(c, generator=g, dtype=torch.float64), torch.randn(c, generator=g, dtype=torch.float64)
+    g1 = torch.randn(n, h, w, c, generator=g, dtype=torch.float64)
+    gp = torch.randn(n, h // 2, w // 2, c, generator=g, dtype=torch.float64)
+    mean = y.mean((0, 1, 2))
+    rstd = (y.var((0, 1, 2), unbiased=False) + 1e-5).rsqrt()
+    yv, gv, bv = (t.clone().requires_grad_(True) for t in (y, gamma, beta))
+    m_, r_ = yv.mean((0, 1, 2)), (yv.var((0, 1, 2), unbiased=False) + 1e-5).rsqrt()
+    a = torch.relu((yv - m_) * r_ * gv + bv)
+    pooled, flat = F.max_pool2d(a.permute(0, 3, 1, 2), 2, return_indices=True)
+    ((a * g1).sum() + (pooled.permute(0, 2, 3, 1) * gp).sum()).backward()
+    ad = a.detach()
+    pv, idx = E.maxpool2x2(ad.float().to(torch.bfloat16))
+    k = idx.permute(0, 3, 1, 2).long()
+    hp, wp = torch.arange(h // 2).view(1, 1, -1, 1), torch.arange(w // 2).view(1, 1, 1, -1)
+    assert torch.equal((2 * hp + k // 2) * w + (2 * wp + k % 2), flat)   # no ties in bf16 here: same windows
+    da = torch.where(ad > 0, g1 + E.unpool(gp, idx, h, w), 0.0)
+    sums = E.bwd_sums(da, y)
+    dgamma, dbeta = E.param_grads(sums, mean, rstd)
+    assert torch.allclose(dgamma, gv.grad, rtol=1e-10, atol=1e-10) and torch.allclose(dbeta, bv.grad, rtol=1e-10, atol=1e-10)
+    dy, mag = E.dy_ref(da, y, gamma, mean, rstd, torch.stack([dbeta, dgamma]), n * h * w)
+    assert torch.allclose(dy, yv.grad, rtol=1e-9, atol=1e-9) and bool((mag >= dy.abs() * (1 - 1e-12)).all())
+    # grid formulas: config 2, level 0 (16 x 512 x 512 x 64): 443 pixels per backward thread, 1772 when pooled
+    assert E.grid("bwd", E.work_items(16, 512, 512, 64, False)) == (296, 75776)
+    assert E.terms_per_thread(16, 512, 512, 64, False) == 443 and E.terms_per_thread(16, 512, 512, 64, True) == 444
+    assert E.grid("fwd", 7) == (1, 256) and E.grid("ew", 10 ** 9) == (1184, 303104)
+
+
+def test_ew_check_flags_the_defects_rel_l2_accepts():
+    """A one-ulp error in one activation, a swapped tie position, a sum that dropped its last item and one overwritten
+    sentinel all pass the rel-L2 checks the BatchNorm+ReLU kernels used to have (4e-3 activations, 1e-2 dy, 2e-3 dgamma /
+    dbeta) and all fail tests/ew_check.py's comparisons."""
+    import conv_check as C
+    import ew_check as E
+
+    g = torch.Generator().manual_seed(13)
+    n, h, w, c = 4, 32, 32, 64
+    y = (torch.randn(n, h, w, c, generator=g) * 1.7 + 0.3).bfloat16()
+    y[:, 0::2, 1::2] = y[:, 0::2, 0::2]                      # a tie in every window (positions 0 and 1)
+    scale, shift = torch.rand(c, generator=g) + 0.5, torch.randn(c, generator=g) * 0.2
+    a, pre, _ = E.bn_relu_fwd(y, scale, shift)
+    # one ulp in one activation
+    bad = a.clone()
+    i = tuple((a > 0).nonzero()[100].tolist())
+    bad.view(torch.int16)[i] += 1
+    assert bad[i] != a[i] and C.rel_l2(bad, a) < 4e-3
+    with pytest.raises(AssertionError, match="1 of"):
+        E.assert_equal(bad, a, "activation")
+    # a tie resolved to the later position
+    pv, idx = E.maxpool2x2(a)
+    tied = (a[:, 0::2, 0::2] == a[:, 0::2, 1::2]) & (idx == 0) & (a[:, 0::2, 0::2] > 0)
+    i = tuple(tied.nonzero()[0].tolist())
+    swapped = idx.clone()
+    swapped[i] = 1
+    with pytest.raises(AssertionError, match="1 of"):
+        E.assert_equal(swapped, idx, "pool_idx")
+    g1 = (torch.randn(n, h, w, c, generator=g) * 0.5 + 1).bfloat16()   # sums that do not cancel: the old relative check
+    gp = (torch.randn(n, h // 2, w // 2, c, generator=g) * 0.5 + 1).bfloat16()  # is at its most sensitive
+    gamma = torch.rand(c, generator=g) + 0.5
+    mean, rstd = y.double().mean((0, 1, 2)).float(), (y.double().var((0, 1, 2)) + 1e-5).rsqrt().float()
+    count = n * h * w
+    da = E.bwd_da(y, g1, gp, idx, scale, shift)
+    sums = E.bwd_sums(da, y)
+    dgamma, dbeta = E.param_grads(sums, mean, rstd)
+    want, mag = E.dy_ref(da, y, gamma, mean, rstd, torch.stack([dbeta, dgamma]), count)
+    bound = E.dy_bound(want, mag, y, gamma, mean, rstd, count)
+    assert E.assert_within(E.to_bf16(want), want, bound, "dy") <= 1.0
+    da_s = E.bwd_da(y, g1, gp, swapped, scale, shift)
+    got, _ = E.dy_ref(da_s, y, gamma, mean, rstd, torch.stack([dbeta, dgamma]), count)
+    assert C.rel_l2(E.to_bf16(got), want) < 1e-2
+    with pytest.raises(AssertionError, match="outside the bound"):
+        E.assert_within(E.to_bf16(got), want, bound, "dy")
+    # the last pixel dropped from the sums (all channels)
+    k = E.terms_per_thread(n, h, w, c, True)
+    bg, bb = E.sum_bounds(sums, mean, rstd, k)
+    short = E.bwd_sums(da.reshape(-1, c)[:-1], y.reshape(-1, c)[:-1])
+    sg, sb = E.param_grads(short, mean, rstd)
+    assert C.rel_l2(sg, dgamma) < 2e-3 and C.rel_l2(sb, dbeta) < 2e-3
+    for got_, want_, b_, what in ((sg, dgamma, bg, "dgamma"), (sb, dbeta, bb, "dbeta")):
+        E.assert_within(want_.float(), want_, b_, what)
+        with pytest.raises(AssertionError, match="outside the bound"):
+            E.assert_within(got_.float(), want_, b_, what)
+    # sentinels: one element past a contiguous output, one in the other half of a concat canvas, one position byte unwritten
+    buf, view = E.guarded((2, 3, 4, 64), torch.bfloat16, device="cpu")
+    view.zero_()
+    E.assert_guard(buf, view.numel(), "pooled")
+    buf[view.numel() + 5] = 0.0
+    with pytest.raises(AssertionError, match="1 elements written past the end"):
+        E.assert_guard(buf, view.numel(), "pooled")
+    ibuf, iview = E.guarded((2, 3, 4, 64), torch.uint8, device="cpu")
+    iview.fill_(3)
+    E.assert_guard(ibuf, iview.numel(), "pool_idx")
+    ibuf[17] = E.U8_SENTINEL
+    with pytest.raises(AssertionError, match="1 elements left unwritten"):
+        E.assert_guard(ibuf, iview.numel(), "pool_idx")
+    cv, left = E.canvas2(1, 2, 2, 64, device="cpu")
+    left.zero_()
+    E.assert_right_half(cv, "a")
+    cv[0, 1, 0, 64 + 9] = 1.0
+    with pytest.raises(AssertionError, match="1 elements of the other half"):
+        E.assert_right_half(cv, "a")

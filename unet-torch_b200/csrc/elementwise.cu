@@ -728,12 +728,14 @@ int b200unet_bn_relu_bwd_apply(const void* g1, int g1_cs, const void* g_pool, co
                                const float* rstd, const double* sums, double count, const double* sums_local, void* dy,
                                int dy_cs, float* dgamma, float* dbeta, int N, int H, int W, int C, b200_stream_t stream) {
   B2_REQUIRE(ok_channels(C), "bn_relu_bwd_apply: C=%d must be a power of two in [64, 2048]", C);
+  B2_REQUIRE(g1 != nullptr || g_pool != nullptr, "bn_relu_bwd_apply: no gradient source");
   B2_REQUIRE(y && gamma && scale && shift && mean && rstd && sums && dy,
              "bn_relu_bwd_apply: null argument (eval-mode forwards must save mean/rstd: b200unet_bn_eval_stats)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   BwdSrc s{static_cast<const __nv_bfloat16*>(g1), g1_cs, static_cast<const __nv_bfloat16*>(g_pool), pool_idx,
            static_cast<const __nv_bfloat16*>(y), y_cs};
   const bool pool = g_pool != nullptr;
+  if (pool) B2_REQUIRE(H % 2 == 0 && W % 2 == 0 && pool_idx != nullptr, "bn_relu_bwd_apply(pool): bad arguments");
   const int blocks = bwd_blocks(N, H, W, C, pool);
   if (pool)
     bn_bwd_apply_kernel<true><<<blocks, EW_THREADS, 0, st>>>(s, gamma, scale, shift, mean, rstd, sums, count, sums_local,

@@ -391,11 +391,27 @@ def bn_eval_stats(running_mean, running_var, eps, mean, rstd):
               _stream())
 
 
+def _pool_operand(t, n, h, w, c, dtype, what):
+    """A pooled-resolution tensor the kernels address at pixel pitch C: contiguous [n, h // 2, w // 2, c] of `dtype`."""
+    if t.dtype != dtype or not t.is_cuda or tuple(t.shape) != (n, h // 2, w // 2, c) or not t.is_contiguous():
+        raise ValueError(f"{what}: expected a contiguous CUDA {dtype} tensor of shape {(n, h // 2, w // 2, c)}, got {t.dtype} "
+                         f"{tuple(t.shape)} strides {t.stride()} on {t.device}")
+    return t.data_ptr()
+
+
 def bn_relu_fwd(y, scale, shift, a, pooled=None, pool_idx=None):
+    """a = bf16(relu(scale * y + shift)); with `pooled`, also the 2x2 max pool of a (+ window positions into pool_idx).
+    y and a may be channel slices; pooled and pool_idx are contiguous."""
     yp, ycs, n, h, w, c = _nhwc(y)
-    ap, acs, *_ = _nhwc(a)
-    _lib.call("b200unet_bn_relu_fwd", yp, ycs, _f32(scale), _f32(shift), ap, acs, _ptr(pooled), _ptr(pool_idx), n, h, w,
-              c, _stream())
+    ap, acs, *sa = _nhwc(a)
+    if sa != [n, h, w, c]:
+        raise ValueError(f"bn_relu_fwd: a {tuple(a.shape)} does not match y {tuple(y.shape)}")
+    if pooled is None and pool_idx is not None:
+        raise ValueError("bn_relu_fwd: pool_idx without pooled")
+    if pooled is not None:
+        pooled = _pool_operand(pooled, n, h, w, c, BF16, "bn_relu_fwd: pooled")
+        pool_idx = None if pool_idx is None else _pool_operand(pool_idx, n, h, w, c, torch.uint8, "bn_relu_fwd: pool_idx")
+    _lib.call("b200unet_bn_relu_fwd", yp, ycs, _f32(scale), _f32(shift), ap, acs, pooled, pool_idx, n, h, w, c, _stream())
 
 
 def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dgamma, dbeta, count=None,
@@ -414,8 +430,20 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
     yp, ycs, n, h, w, c = _nhwc(y)
     g1p, g1cs = (None, 0)
     if g1 is not None:
-        g1p, g1cs, *_ = _nhwc(g1)
-    dp, dcs, *_ = _nhwc(dy)
+        g1p, g1cs, *s1 = _nhwc(g1)
+        if s1 != [n, h, w, c]:
+            raise ValueError(f"bn_relu_bwd: g1 {tuple(g1.shape)} does not match y {tuple(y.shape)}")
+    elif g_pool is None:
+        raise ValueError("bn_relu_bwd: no gradient source (g1 and g_pool are both None)")
+    gpp = idxp = None
+    if g_pool is not None:
+        if pool_idx is None:
+            raise ValueError("bn_relu_bwd: g_pool needs the forward's pool_idx")
+        gpp = _pool_operand(g_pool, n, h, w, c, BF16, "bn_relu_bwd: g_pool")
+        idxp = _pool_operand(pool_idx, n, h, w, c, torch.uint8, "bn_relu_bwd: pool_idx")
+    dp, dcs, *sd = _nhwc(dy)
+    if sd != [n, h, w, c]:
+        raise ValueError(f"bn_relu_bwd: dy {tuple(dy.shape)} does not match y {tuple(y.shape)}")
     ws = _workspace(_lib.query("b200unet_bn_bwd_workspace_floats", n, h, w, c), y.device)
     sums = torch.empty((2 * c,), dtype=torch.float64, device=y.device)
     sums_local = None
@@ -429,7 +457,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
             ws, nrows = pre
         else:
             rows = ctypes.c_int(0)
-            _lib.call("b200unet_bn_relu_bwd_reduce_rows", g1p, g1cs, _ptr(g_pool), _ptr(pool_idx), yp, ycs, _f32(scale),
+            _lib.call("b200unet_bn_relu_bwd_reduce_rows", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale),
                       _f32(shift), _f32(mean), _f32(rstd), ws.data_ptr(), ctypes.byref(rows), n, h, w, c, _stream())
             nrows = rows.value
         if use_rows:
@@ -444,7 +472,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
                 sums_local = sums.clone()
                 allreduce.all_reduce_sum(sums)
     else:
-        _lib.call("b200unet_bn_relu_bwd_reduce", g1p, g1cs, _ptr(g_pool), _ptr(pool_idx), yp, ycs, _f32(scale), _f32(shift),
+        _lib.call("b200unet_bn_relu_bwd_reduce", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale), _f32(shift),
                   _f32(mean), _f32(rstd), ws.data_ptr(), sums.data_ptr(), n, h, w, c, _stream())
         if frozen:
             sums_local = sums
@@ -452,7 +480,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
         elif allreduce is not None:
             sums_local = sums.clone()
             allreduce.all_reduce_sum(sums)
-    _lib.call("b200unet_bn_relu_bwd_apply", g1p, g1cs, _ptr(g_pool), _ptr(pool_idx), yp, ycs, _f32(gamma), _f32(scale),
+    _lib.call("b200unet_bn_relu_bwd_apply", g1p, g1cs, gpp, idxp, yp, ycs, _f32(gamma), _f32(scale),
               _f32(shift), _f32(mean), _f32(rstd), sums.data_ptr(), float(count), _ptr(sums_local), dp, dcs,
               _f32(dgamma), _f32(dbeta), n, h, w, c, _stream())
 
@@ -469,7 +497,8 @@ def maxpool2x2(a, pooled, pool_idx=None):
     pp, pcs, n2, h2, w2, c2 = _nhwc(pooled)
     if (n2, h2, w2, c2) != (n, h // 2, w // 2, c):
         raise ValueError(f"maxpool2x2: shapes {tuple(a.shape)} -> {tuple(pooled.shape)}")
-    _lib.call("b200unet_maxpool2x2_fwd", ap, acs, pp, pcs, _ptr(pool_idx), n, h, w, c, _stream())
+    idxp = None if pool_idx is None else _pool_operand(pool_idx, n, h, w, c, torch.uint8, "maxpool2x2: pool_idx")
+    _lib.call("b200unet_maxpool2x2_fwd", ap, acs, pp, pcs, idxp, n, h, w, c, _stream())
     return pooled
 
 
