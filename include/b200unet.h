@@ -260,7 +260,9 @@ int b200unet_bn_relu_fwd(const void* y, int y_cs, const float* scale, const floa
                          void* pooled, uint8_t* pool_idx, int N, int H, int W, int C, b200_stream_t stream);
 /* Backward of (BN -> ReLU [-> skip + pool]). g1 = gradient w.r.t. a arriving with pitch g1_cs (may be NULL if
  * pooled-only); g_pool/pool_idx = gradient w.r.t. the pooled tensor (NULL if the layer is not pooled).
- * Pass 1 (reduce): per-block partial sums of da and da*xhat where da = (g1 + unpool(g_pool)) * [a > 0]. */
+ * Pass 1 (reduce): per-block partial sums of da and da*xhat where da = (g1 + unpool(g_pool)) * [a > 0].
+ * Workspace (`partial`) of a reduce pass in floats: 148 x 8 rows of 2*C at even H and W, twice that when H or W is odd
+ * (the floor-mode pooled reduce appends the pad strip's rows, see the _floor variants below). */
 int64_t b200unet_bn_bwd_workspace_floats(int N, int H, int W, int C);
 /* (b200unet_bn_relu_bwd_reduce_rows: pass 1 only - leaves the block partials [*rows_out][2][C] in `partial` for a fused
  * cross-rank reduction, b200unet_nvl_rows_allreduce) */
@@ -280,6 +282,33 @@ int b200unet_bn_relu_bwd_apply(const void* g1, int g1_cs, const void* g_pool, co
                                const float* mean, const float* rstd, const double* sums, double count,
                                const double* sums_local, void* dy, int dy_cs, float* dgamma, float* dbeta, int N,
                                int H, int W, int C, b200_stream_t stream);
+/* Floor mode (nn.MaxPool2d(2) on a map of any H, W >= 2; the UNet's Down blocks at sizes that are not multiples of 16):
+ * the _floor variants of b200unet_bn_relu_fwd, _bwd_reduce_rows, _bwd_reduce and _bwd_apply take odd H and W. The 2x2
+ * windows cover the leading 2*(H/2) x 2*(W/2) pixels as above; the pixels of the pad strip (the last row when H is odd, the
+ * last column when W is odd) get their activation (forward) and their gradient with da = g1 * [a > 0] (backward) but enter
+ * no window. At even H and W they are the calls above. They also require N, H, W > 0, a 2x2 map when pooled, pool_idx with
+ * a pooled gradient and pixel pitches >= C. */
+int b200unet_bn_relu_fwd_floor(const void* y, int y_cs, const float* scale, const float* shift, void* a, int a_cs,
+                               void* pooled, uint8_t* pool_idx, int N, int H, int W, int C, b200_stream_t stream);
+int b200unet_bn_relu_bwd_reduce_rows_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx,
+                                           const void* y, int y_cs, const float* scale, const float* shift, const float* mean,
+                                           const float* rstd, float* partial, int* rows_out, int N, int H, int W, int C,
+                                           b200_stream_t stream);
+int b200unet_bn_relu_bwd_reduce_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
+                                      int y_cs, const float* scale, const float* shift, const float* mean, const float* rstd,
+                                      float* partial, double* sums, int N, int H, int W, int C, b200_stream_t stream);
+int b200unet_bn_relu_bwd_apply_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
+                                     int y_cs, const float* gamma, const float* scale, const float* shift, const float* mean,
+                                     const float* rstd, const double* sums, double count, const double* sums_local, void* dy,
+                                     int dy_cs, float* dgamma, float* dbeta, int N, int H, int W, int C,
+                                     b200_stream_t stream);
+/* The pad strip of an [N][H][W] map of C channels at pixel pitch x_cs (a channel slice; 16-byte aligned, C and x_cs
+ * multiples of 8): the pixels outside its leading 2*(H/2) x 2*(W/2) region. F.pad (Model.py:69-73) leaves it zero in the
+ * upsampled half of a concat buffer whose level is odd. pad_strip_zero writes zeros there; pad_strip_sub_colsum does
+ * out[c] -= sum over the strip of x[..., c] (fp64, fixed order) - the ConvTranspose2d bias gradient taken over the whole
+ * half minus the strip, which F.pad's backward discards. Both launch nothing when H and W are even. */
+int b200unet_pad_strip_zero(void* x, int x_cs, int N, int H, int W, int C, b200_stream_t stream);
+int b200unet_pad_strip_sub_colsum(const void* x, int x_cs, int N, int H, int W, int C, float* out, b200_stream_t stream);
 /* out[c] = sum_r partial[r][col_lo + c], c < n: per-channel sums from the [rows][row_pitch] statistics rows a conv
  * epilogue wrote (row_pitch = 2*Cout; columns [0,Cout) hold the sums). Used for the ConvTranspose2d bias gradient
  * (Model.py:56): db = sum over pixels of the upsampled half of the concat gradient. */
@@ -291,6 +320,9 @@ int b200unet_partial_colsum(const float* partial, int64_t rows, int row_pitch, i
  * already ran in the conv epilogue (b200unet_conv3x3_bn_relu_igemm). */
 int b200unet_maxpool2x2_fwd(const void* a, int a_cs, void* pooled, int p_cs, uint8_t* pool_idx, int N, int H, int W, int C,
                             b200_stream_t stream);
+/* Floor mode: any H, W >= 2 (the last row / column of an odd map enters no window). */
+int b200unet_maxpool2x2_fwd_floor(const void* a, int a_cs, void* pooled, int p_cs, uint8_t* pool_idx, int N, int H, int W,
+                                  int C, b200_stream_t stream);
 /* Two decoders over one encoder (UNet_multitask, Model.py:172-250): copy a channel slice of an NHWC bf16 buffer into another
  * (the skip half of the second decoder's concat buffer), and out = a + b over channel slices (sum of the two decoders'
  * gradients; out may alias a). Pitches in elements, multiples of 8. */

@@ -74,6 +74,14 @@ SIGNATURES = {
         [_P, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _D, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P],
     ),
     "b200unet_partial_colsum": (c_int, [_P, _L, _I, _I, _I, _P, _P]),
+    "b200unet_bn_relu_fwd_floor": (c_int, [_P, _I, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P]),
+    "b200unet_bn_relu_bwd_reduce_rows_floor": (c_int, [_P, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "b200unet_bn_relu_bwd_reduce_floor": (c_int, [_P, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "b200unet_bn_relu_bwd_apply_floor": (
+        c_int, [_P, _I, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _D, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P]),
+    "b200unet_pad_strip_zero": (c_int, [_P, _I, _I, _I, _I, _I, _P]),
+    "b200unet_pad_strip_sub_colsum": (c_int, [_P, _I, _I, _I, _I, _I, _P, _P]),
+    "b200unet_maxpool2x2_fwd_floor": (c_int, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P]),
     "b200unet_maxpool2x2_fwd": (c_int, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P]),
     "b200unet_nhwc_copy": (c_int, [_P, _I, _P, _I, _L, _I, _P]),
     "b200unet_nhwc_add": (c_int, [_P, _I, _P, _I, _P, _I, _L, _I, _P]),

@@ -179,8 +179,72 @@ __global__ void bn_eval_stats_kernel(const float* rm, const float* rv, float eps
   rstd[c] = 1.0f / sqrtf(rv[c] + eps);
 }
 
+// ------------------------------------------------------------------------------------------ pad strip
+// nn.MaxPool2d(2) in floor mode (Model.py:36,42) leaves the last row of an odd-H map and the last column of an odd-W map out
+// of every 2x2 window; on the way up, F.pad (Model.py:69-73) puts the same pixels of the concat buffer's upsampled half
+// after the 2h'x2w' ConvTranspose2d output as zeros. Both are "the pad strip" of an [N][H][W] map: the pixels outside its
+// leading 2*(H/2) x 2*(W/2) region, per image the bottom row (odd H) and then the right column above it (odd W).
+__host__ __device__ __forceinline__ long long strip_pixels_per_image(int H, int W) {
+  return static_cast<long long>(H & 1) * W + static_cast<long long>(W & 1) * (H & ~1);
+}
+
+// Strip work items (pixels x 8-channel groups) are counted in 32 bits (the host checks): 32-bit divisions stay inline, where
+// 64-bit ones would call a subroutine and make the pooled backward kernels, at their 128-register cap, spill.
+constexpr long long STRIP_MAX_ITEMS = 0x7fffffffLL - 148LL * 8 * EW_THREADS;
+
+// NHWC pixel index of strip pixel s (0 <= s < N * strip_pixels_per_image)
+__device__ __forceinline__ long long strip_pixel(int s, int H, int W) {
+  const int per = static_cast<int>(strip_pixels_per_image(H, W));
+  const int n = s / per;
+  const int r = s - n * per;
+  const int row = (H & 1) ? W : 0;
+  if (r < row) return (static_cast<long long>(n) * H + H - 1) * W + r;
+  return (static_cast<long long>(n) * H + (r - row)) * W + W - 1;
+}
+
+__global__ void __launch_bounds__(EW_THREADS) pad_strip_zero_kernel(__nv_bfloat16* __restrict__ x, int x_cs, int N, int H,
+                                                                    int W, int C) {
+  const int cgs = C >> 3;
+  const int total = static_cast<int>(N * strip_pixels_per_image(H, W) * cgs);
+  const int stride = gridDim.x * blockDim.x;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+    const int s = i / cgs;
+    *reinterpret_cast<uint4*>(x + strip_pixel(s, H, W) * x_cs + (i - s * cgs) * 8) = make_uint4(0, 0, 0, 0);
+  }
+}
+
+// out[c] -= sum over the pad strip of x[..., c] (fp64, fixed order). A block owns 32 channels (four 8-channel groups) and
+// walks the strip with 64 pixel lanes; the lanes are summed in lane order.
+constexpr int STRIP_LANES = 64;
+__global__ void __launch_bounds__(256) pad_strip_sub_colsum_kernel(const __nv_bfloat16* __restrict__ x, int x_cs, int N,
+                                                                   int H, int W, int C, float* __restrict__ out) {
+  __shared__ double sh[STRIP_LANES][33];
+  const int g = threadIdx.x & 3, lane = threadIdx.x >> 2;
+  const int c0 = blockIdx.x * 32 + g * 8;
+  const int pixels = static_cast<int>(N * strip_pixels_per_image(H, W));
+  double acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  if (c0 < C) {
+    for (int s = lane; s < pixels; s += STRIP_LANES) {
+      float f[8];
+      unpack8(ldg128(x + strip_pixel(s, H, W) * x_cs + c0), f);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) acc[j] += static_cast<double>(f[j]);
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 8; ++j) sh[lane][g * 8 + j] = acc[j];
+  __syncthreads();
+  if (threadIdx.x < 32 && blockIdx.x * 32 + static_cast<int>(threadIdx.x) < C) {
+    double t = 0.0;
+    for (int l = 0; l < STRIP_LANES; ++l) t += sh[l][threadIdx.x];
+    const int c = blockIdx.x * 32 + threadIdx.x;
+    out[c] = static_cast<float>(static_cast<double>(out[c]) - t);
+  }
+}
+
 // ------------------------------------------------------------------------------------------ forward
-template <bool POOL>
+// STRIP (with !POOL): the pixels are those of the pad strip (floor-mode pooling leaves them out of every window)
+template <bool POOL, bool STRIP = false>
 __global__ void __launch_bounds__(EW_THREADS) bn_relu_fwd_kernel(const __nv_bfloat16* __restrict__ y, int y_cs,
                                                                  const float* __restrict__ scale,
                                                                  const float* __restrict__ shift,
@@ -201,7 +265,7 @@ __global__ void __launch_bounds__(EW_THREADS) bn_relu_fwd_kernel(const __nv_bflo
   const long long tid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
   if (!POOL) {
-    const long long total = static_cast<long long>(N) * H * W * cgs;
+    const long long total = (STRIP ? N * strip_pixels_per_image(H, W) : static_cast<long long>(N) * H * W) * cgs;
     constexpr int U = 4;  // independent 128-bit loads in flight per thread
     for (long long i0 = tid; i0 < total; i0 += stride * U) {
       uint4 raw[U];
@@ -210,6 +274,7 @@ __global__ void __launch_bounds__(EW_THREADS) bn_relu_fwd_kernel(const __nv_bflo
       for (int u = 0; u < U; ++u) {
         const long long i = i0 + u * stride;
         pix[u] = (rev ? total - 1 - i : i) / cgs;
+        if (STRIP) pix[u] = strip_pixel(static_cast<int>(pix[u]), H, W);
         if (i < total) raw[u] = ldg128(y + pix[u] * y_cs + cg * 8);
       }
 #pragma unroll
@@ -327,12 +392,14 @@ struct BwdRaw {
   long long pix[NP];
 };
 
-template <bool POOL>
+// STRIP (with !POOL): item k is the k-th pixel of the pad strip
+template <bool POOL, bool STRIP>
 __device__ __forceinline__ void bwd_load(const BwdSrc& s, long long item, int cg, int C, int H, int W, BwdRaw<POOL>& r) {
   if (!POOL) {
-    r.pix[0] = item;
-    r.y[0] = ldg128(s.y + item * s.y_cs + cg * 8);
-    r.g[0] = s.g1 != nullptr ? ldg128(s.g1 + item * s.g1_cs + cg * 8) : make_uint4(0, 0, 0, 0);
+    const long long pix = STRIP ? strip_pixel(static_cast<int>(item), H, W) : item;
+    r.pix[0] = pix;
+    r.y[0] = ldg128(s.y + pix * s.y_cs + cg * 8);
+    r.g[0] = s.g1 != nullptr ? ldg128(s.g1 + pix * s.g1_cs + cg * 8) : make_uint4(0, 0, 0, 0);
   } else {
     const int Hp = H >> 1, Wp = W >> 1;
     const int wp = static_cast<int>(item % Wp);
@@ -369,7 +436,7 @@ __device__ __forceinline__ void bwd_decode(const BwdRaw<POOL>& r, int k, const f
     if (!(fmaf(sc[j], yv[j], sh[j]) > 0.f)) da[j] = 0.f;
 }
 
-template <bool POOL>
+template <bool POOL, bool STRIP = false>
 __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_reduce_kernel(BwdSrc s, const float* __restrict__ scale,
                                                                       const float* __restrict__ shift,
                                                                       const float* __restrict__ mean,
@@ -388,7 +455,9 @@ __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_reduce_kernel(BwdSrc s, 
     s1[i] = 0.f;
     s2[i] = 0.f;
   }
-  const long long items = POOL ? static_cast<long long>(N) * (H >> 1) * (W >> 1) : static_cast<long long>(N) * H * W;
+  const long long items = POOL    ? static_cast<long long>(N) * (H >> 1) * (W >> 1)
+                          : STRIP ? N * strip_pixels_per_image(H, W)
+                                  : static_cast<long long>(N) * H * W;
   const long long total = items * cgs;
   const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
   for (long long i0 = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i0 < total; i0 += stride * U) {
@@ -396,7 +465,7 @@ __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_reduce_kernel(BwdSrc s, 
 #pragma unroll
     for (int u = 0; u < U; ++u)
       if (i0 + u * stride < total)
-        bwd_load<POOL>(s, (rev ? total - 1 - (i0 + u * stride) : (i0 + u * stride)) / cgs, cg, C, H, W, raw[u]);
+        bwd_load<POOL, STRIP>(s, (rev ? total - 1 - (i0 + u * stride) : (i0 + u * stride)) / cgs, cg, C, H, W, raw[u]);
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       if (i0 + u * stride < total) {
@@ -435,7 +504,7 @@ __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_reduce_kernel(BwdSrc s, 
   }
 }
 
-template <bool POOL>
+template <bool POOL, bool STRIP = false>
 __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_apply_kernel(BwdSrc s, const float* __restrict__ gamma,
                                                                      const float* __restrict__ scale,
                                                                      const float* __restrict__ shift,
@@ -471,7 +540,9 @@ __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_apply_kernel(BwdSrc s, c
       dgamma[c] = static_cast<float>(sl[C + c]);
     }
   }
-  const long long items = POOL ? static_cast<long long>(N) * (H >> 1) * (W >> 1) : static_cast<long long>(N) * H * W;
+  const long long items = POOL    ? static_cast<long long>(N) * (H >> 1) * (W >> 1)
+                          : STRIP ? N * strip_pixels_per_image(H, W)
+                                  : static_cast<long long>(N) * H * W;
   const long long total = items * cgs;
   const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
   for (long long i0 = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i0 < total; i0 += stride * U) {
@@ -479,7 +550,7 @@ __global__ void __launch_bounds__(EW_THREADS, 2) bn_bwd_apply_kernel(BwdSrc s, c
 #pragma unroll
     for (int u = 0; u < U; ++u)
       if (i0 + u * stride < total)
-        bwd_load<POOL>(s, (rev ? total - 1 - (i0 + u * stride) : (i0 + u * stride)) / cgs, cg, C, H, W, raw[u]);
+        bwd_load<POOL, STRIP>(s, (rev ? total - 1 - (i0 + u * stride) : (i0 + u * stride)) / cgs, cg, C, H, W, raw[u]);
 #pragma unroll
     for (int u = 0; u < U; ++u) {
       if (i0 + u * stride < total) {
@@ -580,16 +651,25 @@ bool ok_channels(int C) { return C >= 64 && C <= 2048 && (C & (C - 1)) == 0; }
 // as four waves, each paying its own ramp-up, block reduction and tail (ncu: bn_bwd_reduce at 4.9 TB/s, 24 % warps
 // active). One wave of exactly-resident blocks that loop longer removes that. B200UNET_BWD_BLOCKS_PER_SM overrides (8 =
 // the former grid).
-int bwd_blocks(int N, int H, int W, int C, bool pool) {
+int bwd_blocks_for(long long items, int C) {
   static int per_sm = 0;
   if (per_sm == 0) {
     const char* e = getenv("B200UNET_BWD_BLOCKS_PER_SM");
     per_sm = e != nullptr ? atoi(e) : 2;
     if (per_sm < 1 || per_sm > 8) per_sm = 2;
   }
-  const long long items = pool ? static_cast<long long>(N) * (H / 2) * (W / 2) : static_cast<long long>(N) * H * W;
   const int b = ew_blocks(items * (C / 8));
   return b < 148 * per_sm ? b : 148 * per_sm;
+}
+
+int bwd_blocks(int N, int H, int W, int C, bool pool) {
+  return bwd_blocks_for(pool ? static_cast<long long>(N) * (H / 2) * (W / 2) : static_cast<long long>(N) * H * W, C);
+}
+
+// floor-mode pooled passes: the pad strip runs as a second, unpooled launch over its pixels (none at even H and W, where
+// the pooled kernels are exactly those of the even-size path)
+long long floor_strip_pixels(bool floor_mode, bool pool, int N, int H, int W) {
+  return floor_mode && pool ? N * strip_pixels_per_image(H, W) : 0;
 }
 
 }  // namespace
@@ -657,8 +737,12 @@ int b200unet_bn_eval_stats(const float* running_mean, const float* running_var, 
   return b2h::check_launch("bn_eval_stats");
 }
 
-int b200unet_bn_relu_fwd(const void* y, int y_cs, const float* scale, const float* shift, void* a, int a_cs, void* pooled,
-                         uint8_t* pool_idx, int N, int H, int W, int C, b200_stream_t stream) {
+}  // extern "C"
+
+namespace {
+
+int bn_relu_fwd_impl(const void* y, int y_cs, const float* scale, const float* shift, void* a, int a_cs, void* pooled,
+                     uint8_t* pool_idx, int N, int H, int W, int C, bool floor_mode, b200_stream_t stream) {
   B2_REQUIRE(ok_channels(C), "bn_relu_fwd: C=%d must be a power of two in [64, 2048]", C);
   B2_REQUIRE(y_cs % 8 == 0 && a_cs % 8 == 0, "bn_relu_fwd: pitches must be multiples of 8");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -676,19 +760,144 @@ int b200unet_bn_relu_fwd(const void* y, int y_cs, const float* scale, const floa
     bn_relu_fwd_kernel<false><<<blocks, EW_THREADS, 0, st>>>(yy, y_cs, scale, shift, aa, a_cs, nullptr, nullptr, N, H, W, C,
                                                              ew_rev(0));
   } else {
-    B2_REQUIRE(H % 2 == 0 && W % 2 == 0, "bn_relu_fwd(pool): H=%d W=%d must be even", H, W);
+    if (!floor_mode) B2_REQUIRE(H % 2 == 0 && W % 2 == 0, "bn_relu_fwd(pool): H=%d W=%d must be even", H, W);
     int blocks = ew_blocks(static_cast<long long>(N) * (H / 2) * (W / 2) * (C / 8));
     if (blocks > 148 * fwd_per_sm) blocks = 148 * fwd_per_sm;
     bn_relu_fwd_kernel<true><<<blocks, EW_THREADS, 0, st>>>(yy, y_cs, scale, shift, aa, a_cs,
                                                             static_cast<__nv_bfloat16*>(pooled), pool_idx, N, H, W, C,
                                                             ew_rev(0));
+    if (const long long strip = floor_strip_pixels(floor_mode, true, N, H, W)) {
+      if (int e = b2h::check_launch("bn_relu_fwd")) return e;
+      int sb = ew_blocks(strip * (C / 8));
+      if (sb > 148 * fwd_per_sm) sb = 148 * fwd_per_sm;
+      bn_relu_fwd_kernel<false, true><<<sb, EW_THREADS, 0, st>>>(yy, y_cs, scale, shift, aa, a_cs, nullptr, nullptr, N, H, W,
+                                                                 C, ew_rev(0));
+    }
   }
   return b2h::check_launch("bn_relu_fwd");
 }
 
+int bn_relu_bwd_reduce_rows_impl(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
+                                 int y_cs, const float* scale, const float* shift, const float* mean, const float* rstd,
+                                 float* partial, int* rows_out, int N, int H, int W, int C, bool floor_mode,
+                                 b200_stream_t stream) {
+  B2_REQUIRE(ok_channels(C), "bn_relu_bwd_reduce: C=%d must be a power of two in [64, 2048]", C);
+  B2_REQUIRE(g1 != nullptr || g_pool != nullptr, "bn_relu_bwd_reduce: no gradient source");
+  B2_REQUIRE(y && scale && shift && mean && rstd && partial && rows_out,
+             "bn_relu_bwd_reduce: null argument (eval-mode forwards must save mean/rstd: b200unet_bn_eval_stats)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  BwdSrc s{static_cast<const __nv_bfloat16*>(g1), g1_cs, static_cast<const __nv_bfloat16*>(g_pool), pool_idx,
+           static_cast<const __nv_bfloat16*>(y), y_cs};
+  const bool pool = g_pool != nullptr;
+  if (pool) B2_REQUIRE((floor_mode || (H % 2 == 0 && W % 2 == 0)) && pool_idx != nullptr, "bn_relu_bwd_reduce(pool): bad arguments");
+  const int blocks = bwd_blocks(N, H, W, C, pool);
+  if (pool)
+    bn_bwd_reduce_kernel<true><<<blocks, EW_THREADS, 0, st>>>(s, scale, shift, mean, rstd, partial, N, H, W, C, ew_rev(1));
+  else
+    bn_bwd_reduce_kernel<false><<<blocks, EW_THREADS, 0, st>>>(s, scale, shift, mean, rstd, partial, N, H, W, C, ew_rev(1));
+  *rows_out = blocks;
+  if (const long long strip = floor_strip_pixels(floor_mode, pool, N, H, W)) {
+    // the strip's partial rows follow the windows'. Each launch is capped at 148 x per_sm <= EW_MAX_BLOCKS blocks
+    // (B200UNET_BWD_BLOCKS_PER_SM up to 8), so the two together need up to 2 x EW_MAX_BLOCKS rows: what
+    // b200unet_bn_bwd_workspace_floats sizes for when H or W is odd
+    if (int e = b2h::check_launch("bn_relu_bwd_reduce")) return e;
+    const int sb = bwd_blocks_for(strip, C);
+    bn_bwd_reduce_kernel<false, true><<<sb, EW_THREADS, 0, st>>>(s, scale, shift, mean, rstd,
+                                                                 partial + static_cast<size_t>(blocks) * 2 * C, N, H, W, C,
+                                                                 ew_rev(1));
+    *rows_out = blocks + sb;
+  }
+  return b2h::check_launch("bn_relu_bwd_reduce");
+}
+
+int bn_relu_bwd_apply_impl(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y, int y_cs,
+                           const float* gamma, const float* scale, const float* shift, const float* mean, const float* rstd,
+                           const double* sums, double count, const double* sums_local, void* dy, int dy_cs, float* dgamma,
+                           float* dbeta, int N, int H, int W, int C, bool floor_mode, b200_stream_t stream) {
+  B2_REQUIRE(ok_channels(C), "bn_relu_bwd_apply: C=%d must be a power of two in [64, 2048]", C);
+  B2_REQUIRE(g1 != nullptr || g_pool != nullptr, "bn_relu_bwd_apply: no gradient source");
+  B2_REQUIRE(y && gamma && scale && shift && mean && rstd && sums && dy,
+             "bn_relu_bwd_apply: null argument (eval-mode forwards must save mean/rstd: b200unet_bn_eval_stats)");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  BwdSrc s{static_cast<const __nv_bfloat16*>(g1), g1_cs, static_cast<const __nv_bfloat16*>(g_pool), pool_idx,
+           static_cast<const __nv_bfloat16*>(y), y_cs};
+  const bool pool = g_pool != nullptr;
+  if (pool) B2_REQUIRE((floor_mode || (H % 2 == 0 && W % 2 == 0)) && pool_idx != nullptr, "bn_relu_bwd_apply(pool): bad arguments");
+  const int blocks = bwd_blocks(N, H, W, C, pool);
+  if (pool)
+    bn_bwd_apply_kernel<true><<<blocks, EW_THREADS, 0, st>>>(s, gamma, scale, shift, mean, rstd, sums, count, sums_local,
+                                                             static_cast<__nv_bfloat16*>(dy), dy_cs, dgamma, dbeta, N, H,
+                                                             W, C, ew_rev(2));
+  else
+    bn_bwd_apply_kernel<false><<<blocks, EW_THREADS, 0, st>>>(s, gamma, scale, shift, mean, rstd, sums, count, sums_local,
+                                                              static_cast<__nv_bfloat16*>(dy), dy_cs, dgamma, dbeta, N,
+                                                              H, W, C, ew_rev(2));
+  if (const long long strip = floor_strip_pixels(floor_mode, pool, N, H, W)) {
+    if (int e = b2h::check_launch("bn_relu_bwd_apply")) return e;
+    bn_bwd_apply_kernel<false, true><<<bwd_blocks_for(strip, C), EW_THREADS, 0, st>>>(
+        s, gamma, scale, shift, mean, rstd, sums, count, sums_local, static_cast<__nv_bfloat16*>(dy), dy_cs, nullptr, nullptr,
+        N, H, W, C, ew_rev(2));
+  }
+  return b2h::check_launch("bn_relu_bwd_apply");
+}
+
+int maxpool2x2_fwd_impl(const void* a, int a_cs, void* pooled, int p_cs, uint8_t* pool_idx, int N, int H, int W, int C,
+                        bool floor_mode, b200_stream_t stream) {
+  B2_REQUIRE(C > 0 && C % 8 == 0 && a_cs % 8 == 0 && p_cs % 8 == 0 && a_cs >= C && p_cs >= C,
+             "maxpool2x2_fwd: C=%d and the pitches (%d, %d) must be multiples of 8 with pitch >= C", C, a_cs, p_cs);
+  if (floor_mode)
+    B2_REQUIRE(N > 0 && H >= 2 && W >= 2, "maxpool2x2_fwd: N=%d H=%d W=%d: the map must be at least 2x2", N, H, W);
+  else
+    B2_REQUIRE(N > 0 && H >= 2 && W >= 2 && H % 2 == 0 && W % 2 == 0, "maxpool2x2_fwd: H=%d W=%d must be even and >= 2", H, W);
+  const int blocks = ew_blocks(static_cast<long long>(N) * (H / 2) * (W / 2) * (C / 8));
+  maxpool_fwd_kernel<<<blocks, EW_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const __nv_bfloat16*>(a), a_cs, static_cast<__nv_bfloat16*>(pooled), p_cs, pool_idx, N, H, W, C);
+  return b2h::check_launch("maxpool2x2_fwd");
+}
+
+// what the floor-mode entry points check on top of the shared implementations: the map is at least 2x2 when pooled, and
+// every pitch holds the channels (a pooled call reads 2x2 windows and writes [N][H/2][W/2][C] unchecked)
+int floor_pool_args(const char* what, bool pooled, int N, int H, int W, int C, int y_cs, const void* g1, int g1_cs, int out_cs) {
+  B2_REQUIRE(N > 0 && H > 0 && W > 0, "%s: empty map N=%d H=%d W=%d", what, N, H, W);
+  B2_REQUIRE(N * strip_pixels_per_image(H, W) * (C / 8) <= STRIP_MAX_ITEMS, "%s: pad strip too large", what);
+  B2_REQUIRE(!pooled || (H >= 2 && W >= 2), "%s(pool): H=%d W=%d: the map must be at least 2x2", what, H, W);
+  B2_REQUIRE(y_cs >= C && y_cs % 8 == 0 && out_cs >= C && out_cs % 8 == 0 && (g1 == nullptr || (g1_cs >= C && g1_cs % 8 == 0)),
+             "%s: pixel pitches (%d, %d, %d) must be multiples of 8 and >= C=%d", what, y_cs, g1 == nullptr ? 0 : g1_cs, out_cs, C);
+  return 0;
+}
+
+int strip_args(const char* what, const void* x, int x_cs, int N, int H, int W, int C) {
+  B2_REQUIRE(x != nullptr, "%s: null tensor", what);
+  B2_REQUIRE(N > 0 && H > 0 && W > 0, "%s: empty map N=%d H=%d W=%d", what, N, H, W);
+  B2_REQUIRE(C > 0 && C % 8 == 0 && x_cs % 8 == 0 && x_cs >= C,
+             "%s: C=%d and the pixel pitch %d must be multiples of 8 with pitch >= C", what, C, x_cs);
+  B2_REQUIRE(reinterpret_cast<uintptr_t>(x) % 16 == 0, "%s: the slice must start on a 16-byte boundary", what);
+  B2_REQUIRE(N * strip_pixels_per_image(H, W) * (C / 8) <= STRIP_MAX_ITEMS, "%s: pad strip too large", what);
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b200unet_bn_relu_fwd(const void* y, int y_cs, const float* scale, const float* shift, void* a, int a_cs, void* pooled,
+                         uint8_t* pool_idx, int N, int H, int W, int C, b200_stream_t stream) {
+  return bn_relu_fwd_impl(y, y_cs, scale, shift, a, a_cs, pooled, pool_idx, N, H, W, C, false, stream);
+}
+
+int b200unet_bn_relu_fwd_floor(const void* y, int y_cs, const float* scale, const float* shift, void* a, int a_cs,
+                               void* pooled, uint8_t* pool_idx, int N, int H, int W, int C, b200_stream_t stream) {
+  B2_REQUIRE(y && scale && shift && a, "bn_relu_fwd_floor: null argument");
+  B2_REQUIRE(pooled != nullptr || pool_idx == nullptr, "bn_relu_fwd_floor: pool_idx without pooled");
+  if (int e = floor_pool_args("bn_relu_fwd_floor", pooled != nullptr, N, H, W, C, y_cs, nullptr, 0, a_cs)) return e;
+  return bn_relu_fwd_impl(y, y_cs, scale, shift, a, a_cs, pooled, pool_idx, N, H, W, C, true, stream);
+}
+
 int64_t b200unet_bn_bwd_workspace_floats(int N, int H, int W, int C) {
-  (void)N; (void)H; (void)W;
-  return static_cast<int64_t>(EW_MAX_BLOCKS) * 2 * C;
+  (void)N;
+  // odd H or W: a floor-mode pooled reduce writes the pad strip's partial rows after the windows' (two launches)
+  const int launches = strip_pixels_per_image(H, W) > 0 ? 2 : 1;
+  return static_cast<int64_t>(launches) * EW_MAX_BLOCKS * 2 * C;
 }
 
 int b200unet_bn_relu_bwd_reduce(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
@@ -705,47 +914,48 @@ int b200unet_bn_relu_bwd_reduce(const void* g1, int g1_cs, const void* g_pool, c
 int b200unet_bn_relu_bwd_reduce_rows(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
                                      int y_cs, const float* scale, const float* shift, const float* mean, const float* rstd,
                                      float* partial, int* rows_out, int N, int H, int W, int C, b200_stream_t stream) {
-  B2_REQUIRE(ok_channels(C), "bn_relu_bwd_reduce: C=%d must be a power of two in [64, 2048]", C);
-  B2_REQUIRE(g1 != nullptr || g_pool != nullptr, "bn_relu_bwd_reduce: no gradient source");
-  B2_REQUIRE(y && scale && shift && mean && rstd && partial && rows_out,
-             "bn_relu_bwd_reduce: null argument (eval-mode forwards must save mean/rstd: b200unet_bn_eval_stats)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  BwdSrc s{static_cast<const __nv_bfloat16*>(g1), g1_cs, static_cast<const __nv_bfloat16*>(g_pool), pool_idx,
-           static_cast<const __nv_bfloat16*>(y), y_cs};
-  const bool pool = g_pool != nullptr;
-  if (pool) B2_REQUIRE(H % 2 == 0 && W % 2 == 0 && pool_idx != nullptr, "bn_relu_bwd_reduce(pool): bad arguments");
-  const int blocks = bwd_blocks(N, H, W, C, pool);
-  if (pool)
-    bn_bwd_reduce_kernel<true><<<blocks, EW_THREADS, 0, st>>>(s, scale, shift, mean, rstd, partial, N, H, W, C, ew_rev(1));
-  else
-    bn_bwd_reduce_kernel<false><<<blocks, EW_THREADS, 0, st>>>(s, scale, shift, mean, rstd, partial, N, H, W, C, ew_rev(1));
-  *rows_out = blocks;
-  return b2h::check_launch("bn_relu_bwd_reduce");
+  return bn_relu_bwd_reduce_rows_impl(g1, g1_cs, g_pool, pool_idx, y, y_cs, scale, shift, mean, rstd, partial, rows_out, N, H,
+                                      W, C, false, stream);
 }
 
 int b200unet_bn_relu_bwd_apply(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
                                int y_cs, const float* gamma, const float* scale, const float* shift, const float* mean,
                                const float* rstd, const double* sums, double count, const double* sums_local, void* dy,
                                int dy_cs, float* dgamma, float* dbeta, int N, int H, int W, int C, b200_stream_t stream) {
-  B2_REQUIRE(ok_channels(C), "bn_relu_bwd_apply: C=%d must be a power of two in [64, 2048]", C);
-  B2_REQUIRE(g1 != nullptr || g_pool != nullptr, "bn_relu_bwd_apply: no gradient source");
-  B2_REQUIRE(y && gamma && scale && shift && mean && rstd && sums && dy,
-             "bn_relu_bwd_apply: null argument (eval-mode forwards must save mean/rstd: b200unet_bn_eval_stats)");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  BwdSrc s{static_cast<const __nv_bfloat16*>(g1), g1_cs, static_cast<const __nv_bfloat16*>(g_pool), pool_idx,
-           static_cast<const __nv_bfloat16*>(y), y_cs};
-  const bool pool = g_pool != nullptr;
-  if (pool) B2_REQUIRE(H % 2 == 0 && W % 2 == 0 && pool_idx != nullptr, "bn_relu_bwd_apply(pool): bad arguments");
-  const int blocks = bwd_blocks(N, H, W, C, pool);
-  if (pool)
-    bn_bwd_apply_kernel<true><<<blocks, EW_THREADS, 0, st>>>(s, gamma, scale, shift, mean, rstd, sums, count, sums_local,
-                                                             static_cast<__nv_bfloat16*>(dy), dy_cs, dgamma, dbeta, N, H,
-                                                             W, C, ew_rev(2));
-  else
-    bn_bwd_apply_kernel<false><<<blocks, EW_THREADS, 0, st>>>(s, gamma, scale, shift, mean, rstd, sums, count, sums_local,
-                                                              static_cast<__nv_bfloat16*>(dy), dy_cs, dgamma, dbeta, N,
-                                                              H, W, C, ew_rev(2));
-  return b2h::check_launch("bn_relu_bwd_apply");
+  return bn_relu_bwd_apply_impl(g1, g1_cs, g_pool, pool_idx, y, y_cs, gamma, scale, shift, mean, rstd, sums, count, sums_local,
+                                dy, dy_cs, dgamma, dbeta, N, H, W, C, false, stream);
+}
+
+int b200unet_bn_relu_bwd_reduce_rows_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx,
+                                           const void* y, int y_cs, const float* scale, const float* shift, const float* mean,
+                                           const float* rstd, float* partial, int* rows_out, int N, int H, int W, int C,
+                                           b200_stream_t stream) {
+  B2_REQUIRE(g_pool == nullptr || pool_idx != nullptr, "bn_relu_bwd_reduce_floor(pool): a pooled gradient needs pool_idx");
+  if (int e = floor_pool_args("bn_relu_bwd_reduce_floor", g_pool != nullptr, N, H, W, C, y_cs, g1, g1_cs, y_cs)) return e;
+  return bn_relu_bwd_reduce_rows_impl(g1, g1_cs, g_pool, pool_idx, y, y_cs, scale, shift, mean, rstd, partial, rows_out, N, H,
+                                      W, C, true, stream);
+}
+
+int b200unet_bn_relu_bwd_reduce_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
+                                      int y_cs, const float* scale, const float* shift, const float* mean, const float* rstd,
+                                      float* partial, double* sums, int N, int H, int W, int C, b200_stream_t stream) {
+  B2_REQUIRE(sums != nullptr, "bn_relu_bwd_reduce_floor: null sums");
+  int rows = 0;
+  if (int e = b200unet_bn_relu_bwd_reduce_rows_floor(g1, g1_cs, g_pool, pool_idx, y, y_cs, scale, shift, mean, rstd, partial,
+                                                     &rows, N, H, W, C, stream))
+    return e;
+  return launch_reduce_partials(partial, rows, 2 * C, sums, static_cast<cudaStream_t>(stream));
+}
+
+int b200unet_bn_relu_bwd_apply_floor(const void* g1, int g1_cs, const void* g_pool, const uint8_t* pool_idx, const void* y,
+                                     int y_cs, const float* gamma, const float* scale, const float* shift, const float* mean,
+                                     const float* rstd, const double* sums, double count, const double* sums_local, void* dy,
+                                     int dy_cs, float* dgamma, float* dbeta, int N, int H, int W, int C,
+                                     b200_stream_t stream) {
+  B2_REQUIRE(g_pool == nullptr || pool_idx != nullptr, "bn_relu_bwd_apply_floor(pool): a pooled gradient needs pool_idx");
+  if (int e = floor_pool_args("bn_relu_bwd_apply_floor", g_pool != nullptr, N, H, W, C, y_cs, g1, g1_cs, dy_cs)) return e;
+  return bn_relu_bwd_apply_impl(g1, g1_cs, g_pool, pool_idx, y, y_cs, gamma, scale, shift, mean, rstd, sums, count, sums_local,
+                                dy, dy_cs, dgamma, dbeta, N, H, W, C, true, stream);
 }
 
 int b200unet_partial_colsum(const float* partial, int64_t rows, int row_pitch, int col_lo, int n, float* out,
@@ -773,13 +983,31 @@ int b200unet_channel_sum(const void* x, int x_cs, float* workspace, float* out, 
 
 int b200unet_maxpool2x2_fwd(const void* a, int a_cs, void* pooled, int p_cs, uint8_t* pool_idx, int N, int H, int W, int C,
                             b200_stream_t stream) {
-  B2_REQUIRE(C > 0 && C % 8 == 0 && a_cs % 8 == 0 && p_cs % 8 == 0 && a_cs >= C && p_cs >= C,
-             "maxpool2x2_fwd: C=%d and the pitches (%d, %d) must be multiples of 8 with pitch >= C", C, a_cs, p_cs);
-  B2_REQUIRE(N > 0 && H >= 2 && W >= 2 && H % 2 == 0 && W % 2 == 0, "maxpool2x2_fwd: H=%d W=%d must be even and >= 2", H, W);
-  const int blocks = ew_blocks(static_cast<long long>(N) * (H / 2) * (W / 2) * (C / 8));
-  maxpool_fwd_kernel<<<blocks, EW_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const __nv_bfloat16*>(a), a_cs, static_cast<__nv_bfloat16*>(pooled), p_cs, pool_idx, N, H, W, C);
-  return b2h::check_launch("maxpool2x2_fwd");
+  return maxpool2x2_fwd_impl(a, a_cs, pooled, p_cs, pool_idx, N, H, W, C, false, stream);
+}
+
+int b200unet_maxpool2x2_fwd_floor(const void* a, int a_cs, void* pooled, int p_cs, uint8_t* pool_idx, int N, int H, int W,
+                                  int C, b200_stream_t stream) {
+  B2_REQUIRE(a && pooled, "maxpool2x2_fwd_floor: null argument");
+  return maxpool2x2_fwd_impl(a, a_cs, pooled, p_cs, pool_idx, N, H, W, C, true, stream);
+}
+
+int b200unet_pad_strip_zero(void* x, int x_cs, int N, int H, int W, int C, b200_stream_t stream) {
+  if (int e = strip_args("pad_strip_zero", x, x_cs, N, H, W, C)) return e;
+  const long long items = N * strip_pixels_per_image(H, W) * (C / 8);
+  if (items == 0) return 0;
+  pad_strip_zero_kernel<<<ew_blocks(items), EW_THREADS, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<__nv_bfloat16*>(x), x_cs, N, H, W, C);
+  return b2h::check_launch("pad_strip_zero");
+}
+
+int b200unet_pad_strip_sub_colsum(const void* x, int x_cs, int N, int H, int W, int C, float* out, b200_stream_t stream) {
+  if (int e = strip_args("pad_strip_sub_colsum", x, x_cs, N, H, W, C)) return e;
+  B2_REQUIRE(out != nullptr, "pad_strip_sub_colsum: null out");
+  if (strip_pixels_per_image(H, W) == 0) return 0;
+  pad_strip_sub_colsum_kernel<<<(C + 31) / 32, 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      static_cast<const __nv_bfloat16*>(x), x_cs, N, H, W, C, out);
+  return b2h::check_launch("pad_strip_sub_colsum");
 }
 
 int b200unet_nhwc_copy(const void* src, int src_cs, void* dst, int dst_cs, int64_t pixels, int C, b200_stream_t stream) {

@@ -476,9 +476,8 @@ class UNetEngine:
         if not x.is_cuda:
             raise RuntimeError("the B200 UNet runs on CUDA (sm_100a) only; there is no CPU fallback")
         n, _, h, w = x.shape
-        if h % 16 or w % 16:
-            raise ValueError(f"tensor-core engine: H and W must be multiples of 16 (got {h}x{w}); the generic engine "
-                             "takes other sizes")
+        if h < 16 or w < 16:
+            raise ValueError(f"UNet needs H and W >= 16 (got {h}x{w}): its fifth level would be empty")
         x = x.contiguous().float()
         dev = x.device
         dp = DataParallelContext.current() if training else None
@@ -486,7 +485,8 @@ class UNetEngine:
         ch = [f * (1 << l) for l in range(5)]
         hs = [h >> l for l in range(5)]
         wsz = [w >> l for l in range(5)]
-        # concat buffers of decoder levels 0..3: [skip | upsampled]
+        # concat buffers of decoder levels 0..3: [skip | upsampled]. At an odd level the upsampled map is one row / column
+        # short of the skip (floor-mode pooling): the pad strip of the upsampled half is zeroed after every ConvTranspose2d
         cat = [torch.empty((n, hs[l], wsz[l], 2 * ch[l]), dtype=BF16, device=dev) for l in range(4)]
         saved = _Saved() if save else None
         enc_rec, dec_rec = [], []
@@ -576,6 +576,8 @@ class UNetEngine:
                     grec = self._gate_forward(self.gates[j], d_in, enc_rec[l][2], catk[l][..., : ch[l]], training, dp, save)
                 wf, _ = upo.operands()
                 ops.convt2x2(d_in, wf, upo.up.bias.detach(), catk[l][..., ch[l]:])
+                if hs[l] % 2 or wsz[l] % 2:  # F.pad (Model.py:69-73): zeros below / right of the upsampled map
+                    ops.pad_strip_zero(catk[l][..., ch[l]:])
                 self._tr("convt", up=upo, x=d_in, out=catk[l][..., ch[l]:], cat=catk[l], skip=enc_rec[l][2])
                 if drop_ps[4 + j] > 0:  # Up: cat -> Dropout over both halves; nothing reads the skip half after this
                     self._dropout(catk[l], 4 + j, seed, drop_ps[4 + j])
@@ -729,6 +731,8 @@ class UNetEngine:
                                    pre=pre)
                 if p_up > 0:  # the concat's mask on both halves; the bias gradient sums the masked upsampled half
                     self._dropout(dcat, 4 + j, seed, p_up, sums=(ch[l], db), backward=True)
+                if hs[l] % 2 or wsz[l] % 2:  # those sums cover the pad strip too, which F.pad's backward discards
+                    ops.pad_strip_sub_colsum(dcat[..., ch[l]:], db)
                 dq_gate = None
                 # the side stream reads dcat's upsampled half (ConvTranspose2d weight gradient below). A plain single-decoder
                 # network keeps the storage referenced through skip_grads; behind a gate, or for a second decoder, nothing else
@@ -908,6 +912,7 @@ class UNet(nn.Module):
         self._check_fp32 = os.environ.get("B200UNET_CHECK_FP32", "0") not in ("", "0")
         self._cuda_graphs = os.environ.get("B200UNET_CUDA_GRAPHS", "0") not in ("", "0")
         self._share_grads = False
+        self._unaligned = False
 
     def _topology(self):
         """(inc, [down1..4], [([up1..4], outc)]) - what the engines execute."""
@@ -949,6 +954,26 @@ class UNet(nn.Module):
         self._check_fp32 = bool(flag)
         return self
 
+    def allow_unaligned_sizes(self, flag: bool = True):
+        """Run inputs whose H or W is not a multiple of 16 (any H, W >= 16) on the tensor-core engine, as the reference's
+        floor-mode pooling and F.pad do (Model.py:36,42,69-73), instead of on the generic fp32 engine (UNet) or not at all
+        (UNet_multitask, the fused predict heads, predict_tiled). Off by default: it moves those inputs from fp32 to bf16
+        precision. Check mode still selects the generic engine; UNet_attention rejects these sizes either way."""
+        self._unaligned = bool(flag)
+        return self
+
+    def _size_fits_engine(self, x) -> bool:
+        """Does this input's H x W run on the tensor-core engine? Multiples of 16 always; any H, W >= 16 with
+        allow_unaligned_sizes (smaller ones raise: the reference's fifth level would be empty)."""
+        h, w = x.shape[2], x.shape[3]
+        if h % 16 == 0 and w % 16 == 0:
+            return True
+        if not self._unaligned:
+            return False
+        if h < 16 or w < 16:
+            raise ValueError(f"UNet needs H and W >= 16 (got {h}x{w}): its fifth level would be empty")
+        return True
+
     def _fast_supported(self) -> bool:
         """Can the tensor-core engine run this architecture at all (input size is checked per call)?"""
         # widths: the BN / head kernels take power-of-two channel counts in [64, 2048] -> base width 64 or 128
@@ -967,8 +992,7 @@ class UNet(nn.Module):
     def _engine_for(self, x):
         """Tensor-core engine when the architecture and this input fit it, otherwise (or in check mode) the generic
         fp32 engine. Both are CUDA kernels of this library; there is no PyTorch / CPU fallback."""
-        fast = (not self._check_fp32 and self._fast_supported() and x.dim() == 4 and x.shape[2] % 16 == 0
-                and x.shape[3] % 16 == 0)
+        fast = not self._check_fp32 and self._fast_supported() and x.dim() == 4 and self._size_fits_engine(x)
         if fast:
             return self._get_engine()
         if self._generic is None:
@@ -1001,8 +1025,8 @@ class UNet(nn.Module):
     def _fused_head(self, x, head, head_arg=0.0):
         eng = self._engine_for(x)
         if not isinstance(eng, UNetEngine):
-            raise ValueError("fused inference heads run on the tensor-core engine (H, W multiples of 16, default widths); "
-                             "use predict_mask(net(x)) for other variants")
+            raise ValueError("fused inference heads run on the tensor-core engine (H, W multiples of 16 - or any H, W >= 16 "
+                             "after allow_unaligned_sizes() -, default widths); use predict_mask(net(x)) for other variants")
         with torch.no_grad(), _device_guard(x):
             out, _ = eng.forward(x, training=self.training, save=False, head=head, head_arg=head_arg)
         return out
@@ -1054,6 +1078,7 @@ class UNet_multitask(UNet):
         self._check_fp32 = False
         self._cuda_graphs = False
         self._share_grads = False
+        self._unaligned = False
 
     def _topology(self):
         return self.inc, [self.down1, self.down2, self.down3, self.down4], [
@@ -1063,9 +1088,10 @@ class UNet_multitask(UNet):
         return self.initial_feature_map in (64, 128) and self.n_channels <= 7 and 1 <= self.n_classes <= ops.HEAD_MAX_CLASSES
 
     def _engine_for(self, x):
-        if x.dim() != 4 or x.shape[2] % 16 or x.shape[3] % 16 or not self._fast_supported():
-            raise ValueError("UNet_multitask runs on the tensor-core engine only: H and W multiples of 16, "
-                             "initial_feature_map in (64, 128), n_channels <= 7, n_classes <= 256")
+        if x.dim() != 4 or not self._fast_supported() or not self._size_fits_engine(x):
+            raise ValueError("UNet_multitask runs on the tensor-core engine only: H and W multiples of 16 (any H, W >= 16 "
+                             "after allow_unaligned_sizes()), initial_feature_map in (64, 128), n_channels <= 7, "
+                             "n_classes <= 256")
         return self._get_engine()
 
     def set_check_mode(self, flag: bool = True):
@@ -1128,6 +1154,7 @@ class UNet_attention(UNet):
         self._check_fp32 = os.environ.get("B200UNET_CHECK_FP32", "0") not in ("", "0")
         self._cuda_graphs = False
         self._share_grads = False
+        self._unaligned = False
 
     def _attention_gates(self):
         """Gate of decoder block j = 0..3 (up1..up4)."""
@@ -1193,8 +1220,9 @@ def predict_tiled(net, img_org, crop_size, head="sigmoid", threshold=0.5, max_ba
     crop through the network in eval mode and stitch the per-crop masks -> uint8 [Hp,Wp]. The reference loops over the
     crops one forward at a time; here they form batches (eval-mode BatchNorm makes crops independent of each other) and the
     mask comes from the fused head: head="sigmoid" (channel 0 >= threshold, test.py:436-440) or "mask" (softmax/argmax)."""
-    if crop_size % 16:
-        raise ValueError("predict_tiled: crop_size must be a multiple of 16")
+    if crop_size % 16 and not (getattr(net, "_unaligned", False) and crop_size >= 16):
+        raise ValueError("predict_tiled: crop_size must be a multiple of 16 (any crop_size >= 16 after "
+                         "net.allow_unaligned_sizes())")
     if net.training:
         raise RuntimeError("predict_tiled is an inference path: call net.eval() first (test.py:430)")
     x = preprocess_crop(img_org, crop_size, device=next(net.parameters()).device)

@@ -400,7 +400,8 @@ def _pool_operand(t, n, h, w, c, dtype, what):
 
 
 def bn_relu_fwd(y, scale, shift, a, pooled=None, pool_idx=None):
-    """a = bf16(relu(scale * y + shift)); with `pooled`, also the 2x2 max pool of a (+ window positions into pool_idx).
+    """a = bf16(relu(scale * y + shift)); with `pooled`, also the 2x2 max pool of a (+ window positions into pool_idx),
+    in floor mode: at an odd H or W the last row / column is activated but enters no window.
     y and a may be channel slices; pooled and pool_idx are contiguous."""
     yp, ycs, n, h, w, c = _nhwc(y)
     ap, acs, *sa = _nhwc(a)
@@ -411,7 +412,7 @@ def bn_relu_fwd(y, scale, shift, a, pooled=None, pool_idx=None):
     if pooled is not None:
         pooled = _pool_operand(pooled, n, h, w, c, BF16, "bn_relu_fwd: pooled")
         pool_idx = None if pool_idx is None else _pool_operand(pool_idx, n, h, w, c, torch.uint8, "bn_relu_fwd: pool_idx")
-    _lib.call("b200unet_bn_relu_fwd", yp, ycs, _f32(scale), _f32(shift), ap, acs, pooled, pool_idx, n, h, w, c, _stream())
+    _lib.call("b200unet_bn_relu_fwd_floor", yp, ycs, _f32(scale), _f32(shift), ap, acs, pooled, pool_idx, n, h, w, c, _stream())
 
 
 def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dgamma, dbeta, count=None,
@@ -457,7 +458,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
             ws, nrows = pre
         else:
             rows = ctypes.c_int(0)
-            _lib.call("b200unet_bn_relu_bwd_reduce_rows", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale),
+            _lib.call("b200unet_bn_relu_bwd_reduce_rows_floor", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale),
                       _f32(shift), _f32(mean), _f32(rstd), ws.data_ptr(), ctypes.byref(rows), n, h, w, c, _stream())
             nrows = rows.value
         if use_rows:
@@ -472,7 +473,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
                 sums_local = sums.clone()
                 allreduce.all_reduce_sum(sums)
     else:
-        _lib.call("b200unet_bn_relu_bwd_reduce", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale), _f32(shift),
+        _lib.call("b200unet_bn_relu_bwd_reduce_floor", g1p, g1cs, gpp, idxp, yp, ycs, _f32(scale), _f32(shift),
                   _f32(mean), _f32(rstd), ws.data_ptr(), sums.data_ptr(), n, h, w, c, _stream())
         if frozen:
             sums_local = sums
@@ -480,7 +481,7 @@ def bn_relu_bwd(g1, g_pool, pool_idx, y, gamma, scale, shift, mean, rstd, dy, dg
         elif allreduce is not None:
             sums_local = sums.clone()
             allreduce.all_reduce_sum(sums)
-    _lib.call("b200unet_bn_relu_bwd_apply", g1p, g1cs, gpp, idxp, yp, ycs, _f32(gamma), _f32(scale),
+    _lib.call("b200unet_bn_relu_bwd_apply_floor", g1p, g1cs, gpp, idxp, yp, ycs, _f32(gamma), _f32(scale),
               _f32(shift), _f32(mean), _f32(rstd), sums.data_ptr(), float(count), _ptr(sums_local), dp, dcs,
               _f32(dgamma), _f32(dbeta), n, h, w, c, _stream())
 
@@ -492,14 +493,32 @@ def partial_colsum(stats_partial, rows, row_pitch, col_lo, n, out):
 
 
 def maxpool2x2(a, pooled, pool_idx=None):
-    """pooled = MaxPool2d(2)(a) over NHWC bf16 (a may be a channel slice); optional 1-byte window positions."""
+    """pooled = MaxPool2d(2)(a) over NHWC bf16 (a may be a channel slice; floor mode at odd H or W); optional 1-byte window
+    positions."""
     ap, acs, n, h, w, c = _nhwc(a)
     pp, pcs, n2, h2, w2, c2 = _nhwc(pooled)
     if (n2, h2, w2, c2) != (n, h // 2, w // 2, c):
         raise ValueError(f"maxpool2x2: shapes {tuple(a.shape)} -> {tuple(pooled.shape)}")
     idxp = None if pool_idx is None else _pool_operand(pool_idx, n, h, w, c, torch.uint8, "maxpool2x2: pool_idx")
-    _lib.call("b200unet_maxpool2x2_fwd", ap, acs, pp, pcs, idxp, n, h, w, c, _stream())
+    _lib.call("b200unet_maxpool2x2_fwd_floor", ap, acs, pp, pcs, idxp, n, h, w, c, _stream())
     return pooled
+
+
+def pad_strip_zero(x):
+    """Zero the pad strip of x (NHWC bf16, possibly a channel slice): the last row if H is odd and the last column if W is
+    odd - where F.pad leaves zeros around the upsampled map in the reference's Up (Model.py:69-73). No launch at even H, W."""
+    xp, xcs, n, h, w, c = _nhwc(x)
+    _lib.call("b200unet_pad_strip_zero", xp, xcs, n, h, w, c, _stream())
+    return x
+
+
+def pad_strip_sub_colsum(x, out):
+    """out[c] -= sum over the pad strip of x[..., c] (fp64, fixed order; out fp32 [C]). No launch at even H, W."""
+    xp, xcs, n, h, w, c = _nhwc(x)
+    if out.numel() != c:
+        raise ValueError(f"pad_strip_sub_colsum: out has {out.numel()} elements for {c} channels")
+    _lib.call("b200unet_pad_strip_sub_colsum", xp, xcs, n, h, w, c, _f32(out), _stream())
+    return out
 
 
 def nhwc_copy(src, dst):
